@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — post-backbone detection images/s @1024^2 on B200 (BASELINE.json metric), one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--check] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--check] [--no-extras] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -36,6 +36,12 @@ Reported on ONE JSON line (rank 0):
 `--impl reference` times the CPU restatement alone on the same global batch (the reference itself is TF-1.x graph code;
 TensorFlow is not installable in this image, see DESIGN.md) and prints the same line with "impl": "reference".
 `--check` compares the gathered detections of every shard (headline and batch-64 runs) with the CPU oracle.
+`--dump-outputs DIR` (rank 0) writes what the last timed step returned to its caller as float32 .npy files: detections
+[B,100,6], proposals [B,1000,4] and pooled_7x7_sample / pooled_14x14_sample, the same DUMP_ROIS rows (a seeded choice)
+of the two [1,B*1000,P,P,256] pooled tensors. With N > 1 the detections are the gathered batch of all ranks, while the
+proposals and pooled samples are rank 0's own images. The inputs are seeded, so two builds run with the same arguments
+can be compared file by file.
+The bench writes nothing into the source tree (no bytecode either), so it also runs from a read-only checkout.
 """
 from __future__ import annotations
 
@@ -52,6 +58,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # no __pycache__ in the tree for the project modules imported below
 
 IMAGE = 1024
 B_PER_GPU = 2
@@ -59,6 +66,7 @@ GLOBAL_B64 = int(os.environ.get("OD_BENCH_GLOBAL_B", "64"))   # BASELINE configs
 N_ROIS = 1000
 N_CLASSES = 81
 DEPTH = 256
+DUMP_ROIS = 128                          # --dump-outputs: pooled ROIs kept of B*N_ROIS (32 MB for 7x7 + 14x14)
 WINDOW_PX = [131, 0, 893, 1024]          # test_detection.ipynb window
 WORKLOAD = ("maskrcnn-coco-heads-1024: 261888 anchors, 6000->1000 proposals, ROIAlign 7x7+14x14 over P2-P5 (D=256), "
             "81 classes, batch 2 per GPU")
@@ -600,6 +608,11 @@ def run_ours(args):
     ev1.record()
     torch.cuda.synchronize(); barrier()
     wall1 = time.time()
+    # read before the passes below reuse the output buffers of the input sets
+    dump = None
+    if args.dump_outputs and rank == 0:
+        last = (args.steps - 1) % NSETS
+        dump = last_step_outputs(torch, det, proposals, pooled7s[last], pooled14s[last])
     launches = L.od_launch_count() - launches0     # eager launches ...
     launches += sum(graph_launches[i % NSETS] for i in range(args.steps)) if graphs_a[0] is not None else 0   # + replayed ones
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
@@ -803,9 +816,23 @@ def run_ours(args):
             "check": check, "lib_source_hash": lib_hash,
             "detections_per_image": float((det[:, :, 4] > 0).sum().item()) / det.shape[0],
         }
+        if dump is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dump.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def last_step_outputs(torch, det, proposals, pooled7, pooled14) -> dict:
+    """Host copies of what one step hands its caller (--dump-outputs). The pooled tensors (0.5 GB at 14x14) are cut to
+    DUMP_ROIS rows drawn with a fixed seed, the same rows at both pool sizes."""
+    rows = np.sort(np.random.RandomState(0).choice(pooled7.shape[1], DUMP_ROIS, replace=False))
+    rows = torch.from_numpy(rows).to(pooled7.device)
+    return {"detections": det.cpu().numpy(), "proposals": proposals.cpu().numpy(),
+            "pooled_7x7_sample": pooled7[0].index_select(0, rows).cpu().numpy(),
+            "pooled_14x14_sample": pooled14[0].index_select(0, rows).cpu().numpy()}
 
 
 def kernel_times(torch, step, NSETS):
@@ -1126,7 +1153,12 @@ def main():
     ap.add_argument("--roi-concurrent", action="store_true", help="experiment: 7x7 ROIAlign on its own stream next to the 14x14 launch")
     ap.add_argument("--lanes", type=int, default=4, help="steps in flight (1: strictly one step after the other)")
     ap.add_argument("--kernel-times", action="store_true", help="print per-kernel device times (CUPTI) to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

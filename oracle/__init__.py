@@ -15,8 +15,10 @@ no outputs for those layers).
 from __future__ import annotations
 
 import ctypes
+import hashlib
 import os
 import subprocess
+import tempfile
 from ctypes import POINTER, c_double, c_float, c_int32, c_int64, c_void_p
 
 import numpy as np
@@ -27,21 +29,61 @@ _LIB = os.path.join(_HERE, "liboracle.so")
 _lib = None
 
 
+def _built_from(lib: str, digest: str) -> bool:
+    try:
+        with open(lib + ".sha1") as f:
+            return f.read().strip() == digest and os.path.exists(lib)
+    except OSError:
+        return False
+
+
+def _private_dir(digest: str) -> str:
+    """One directory per user and source under the system's temporary directory, shared by every process that
+    needs the library while the tree is read-only."""
+    d = os.path.join(tempfile.gettempdir(), f"oracle-{os.getuid()}-{digest[:16]}")
+    os.makedirs(d, mode=0o700, exist_ok=True)
+    st = os.stat(d)
+    if st.st_uid != os.getuid() or st.st_mode & 0o022:
+        raise RuntimeError(f"{d} exists and is not a private directory of this user")
+    return d
+
+
 def build(force: bool = False) -> str:
-    """Compile ``liboracle.so`` next to its source (gcc, no FMA contraction)."""
-    if (not force and os.path.exists(_LIB)
-            and (not os.path.exists(_SRC) or os.path.getmtime(_LIB) >= os.path.getmtime(_SRC))):
+    """Compile ``liboracle.so`` next to its source (gcc, no FMA contraction).
+
+    A library is up to date when its stamp (``liboracle.so.sha1``) holds the sha1 of the source it was built from;
+    file times are not used, a copy of the tree does not keep them. In a read-only tree a missing or stale library is
+    built once per source in a directory under the system's temporary directory, which ``_LIB`` then names."""
+    global _LIB
+    if not os.path.exists(_SRC):
         return _LIB
+    with open(_SRC, "rb") as f:
+        digest = hashlib.sha1(f.read()).hexdigest()
+    out = os.path.join(_HERE, "liboracle.so")
+    if not force and _built_from(out, digest):
+        _LIB = out
+        return out
+    if not os.access(_HERE, os.W_OK):
+        out = os.path.join(_private_dir(digest), "liboracle.so")
+        if not force and _built_from(out, digest):
+            _LIB = out
+            return out
+    part = f"{out}.{os.getpid()}.part"       # renamed into place: a concurrent process never loads half a library
     base = ["-O2", "-std=c11", "-fPIC", "-shared", "-ffp-contract=off", "-fno-fast-math",
-            "-fvisibility=hidden", "-o", _LIB, _SRC, "-lm"]
+            "-fvisibility=hidden", "-o", part, _SRC, "-lm"]
     errors = []
     for cc in ("/usr/bin/gcc", "gcc", "cc"):
         for omp in (["-fopenmp"], []):
             try:
                 subprocess.run([cc] + omp + base, check=True, capture_output=True, text=True)
-                return _LIB
             except (subprocess.CalledProcessError, FileNotFoundError) as e:  # try next
                 errors.append(f"{cc} {' '.join(omp)}: {getattr(e, 'stderr', e)}")
+                continue
+            os.replace(part, out)
+            with open(out + ".sha1", "w") as f:
+                f.write(digest)
+            _LIB = out
+            return out
     raise RuntimeError("could not build the oracle:\n" + "\n".join(errors))
 
 

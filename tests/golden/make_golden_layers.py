@@ -6,7 +6,8 @@ of the three TF C++ kernels).  Every `DEBUG=True` intermediate the classes expos
 
 Build container only (needs /root/reference):   python tests/golden/make_golden_layers.py
 The inputs come from tests/golden/layer_recipes.py (seeded; the tests regenerate them), so the .npz holds outputs
-only: full arrays where they are small, sha256 digests + strided samples where they are not.
+only: full arrays where they are small, sha256 digests + strided samples where they are not, and every member above
+golden_sample.MAX_WHOLE elements as its shape, digest and a seeded row sample (golden_sample.shrink).
 """
 import hashlib
 import os
@@ -23,6 +24,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.dirname(HERE))
 sys.path.insert(0, HERE)
 
+import golden_sample  # noqa: E402
 import layer_recipes as R  # noqa: E402
 import tf_shim  # noqa: E402
 
@@ -165,7 +167,7 @@ def main():
                      [0.44881889, 0.23622048, 0.76377952, 0.55118108]])
     assert np.allclose(g["normtf/0"][:3], want, rtol=0, atol=1e-7), g["normtf/0"][:3]
 
-    np.savez_compressed(OUT, **g)
+    np.savez_compressed(OUT, **golden_sample.shrink(g))
     print(f"wrote {OUT}: {len(g)} arrays, {os.path.getsize(OUT) / 1e6:.2f} MB")
 
 

@@ -14,6 +14,7 @@ import pytest
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 sys.path.insert(0, os.path.join(HERE, "golden"))
+import golden_sample  # noqa: E402
 import layer_recipes as R  # noqa: E402
 from test_reference_layer_goldens import (DET_CASES, PROPOSAL_CASES, ROI_CASES, TARGET_CASES, bits, sha)  # noqa: E402
 
@@ -30,7 +31,7 @@ def _need_cuda():
 
 @pytest.fixture(scope="module")
 def G():
-    return np.load(os.path.join(HERE, "golden", "reference_layers.npz"))
+    return golden_sample.Golden(os.path.join(HERE, "golden", "reference_layers.npz"))
 
 
 def cu(a):

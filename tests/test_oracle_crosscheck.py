@@ -365,3 +365,48 @@ def test_head_losses_oracle_vs_torch():
     want = F.binary_cross_entropy(torch.from_numpy(pb2[m, ids[m]]).double(), torch.from_numpy(tb2[m]).double())
     assert np.isclose(bl2, float(want), rtol=1e-5)
     assert oracle.mrcnn_losses(np.zeros_like(ids), lg2, act, tb2, pb2)[2] == 0.0
+
+
+# ------------------------------------------------------------------ the oracle's own build
+def test_oracle_build_follows_the_source_bytes_not_file_times(tmp_path):
+    """liboracle.so is rebuilt when the source changes, not when only its file time does (a copied tree keeps none);
+    in a tree it cannot write, a stale library is built once in a temporary directory that later processes reuse."""
+    import importlib.util
+    import os
+    import shutil
+    d = tmp_path / "oracle"
+    d.mkdir()
+    for f in ("__init__.py", "odhead_oracle.c"):
+        shutil.copy(os.path.join(os.path.dirname(oracle.__file__), f), d / f)
+
+    def load():                     # a fresh import of the copy, as a new process would see it
+        spec = importlib.util.spec_from_file_location("oracle_copy", d / "__init__.py")
+        m = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(m)
+        return m
+
+    copy = load()
+    lib = copy.build()
+    assert lib == str(d / "liboracle.so")
+    t = os.path.getmtime(lib)
+    os.utime(d / "odhead_oracle.c", (t + 60, t + 60))
+    assert copy.build() == lib and os.path.getmtime(lib) == t
+    with open(d / "odhead_oracle.c", "a") as f:
+        f.write("\n")
+    assert copy.build() == lib and os.path.getmtime(lib) != t
+    if os.geteuid() == 0:
+        return                      # root writes into a read-only directory anyway
+    with open(d / "odhead_oracle.c", "a") as f:
+        f.write("\n")
+    t = os.path.getmtime(lib)
+    d.chmod(0o555)
+    try:
+        out = copy.build()
+        built = os.path.getmtime(out)
+        again = load()
+        assert again.build() == out and again._LIB == out and os.path.getmtime(out) == built
+    finally:
+        d.chmod(0o755)
+    assert os.path.dirname(out) != str(d) and copy._LIB == out
+    assert os.path.getmtime(lib) == t
+    shutil.rmtree(os.path.dirname(out))

@@ -5,7 +5,9 @@ proposals_tf.py / maskrcnn.py / data_processor.py / detection.py / utils.py unmo
 them through the numpy-eager TensorFlow stand-in tests/tf_shim (the three TF C++ kernels delegate to the oracle's
 restatements; everything the reference itself wrote executes as written). Here — CPU only, no reference tree needed —
 the C oracle (oracle/odhead_oracle.c) and the independent numpy oracle (oracle/np_layers.py) are required to equal those
-files bit for bit; tests/test_gpu_parity_goldens.py asks the same of the CUDA path.
+files bit for bit; tests/test_gpu_parity_goldens.py asks the same of the CUDA path. A large member is stored as its
+shape, a digest of all of its bits and a seeded sample of its rows (tests/golden/golden_sample.py); `bits` compares
+a result with all three.
 """
 import hashlib
 import os
@@ -17,6 +19,7 @@ import pytest
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 sys.path.insert(0, os.path.join(HERE, "golden"))
+import golden_sample  # noqa: E402
 import layer_recipes as R  # noqa: E402
 
 import oracle  # noqa: E402
@@ -27,10 +30,12 @@ f32 = np.float32
 
 @pytest.fixture(scope="module")
 def G():
-    return np.load(os.path.join(HERE, "golden", "reference_layers.npz"))
+    return golden_sample.Golden(os.path.join(HERE, "golden", "reference_layers.npz"))
 
 
 def bits(a, b, what=""):
+    if isinstance(b, golden_sample.Sampled):
+        return b.check(a, what, bits)
     a, b = np.asarray(a), np.asarray(b)
     assert a.shape == b.shape, (what, a.shape, b.shape)
     if a.dtype.kind == "f" or b.dtype.kind == "f":

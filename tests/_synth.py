@@ -23,6 +23,28 @@ def rois_log_uniform(rs, B, N, image=1024, lo=16, hi=512):
     return boxes.astype(f32)
 
 
+def rois_with_edge_cases(rs, B, N, lo=4, hi=900):
+    """rois_log_uniform boxes with the last 10 of image 1 zero padded and rows 0..12 of image 0 set to the cases where
+    ROIAlign kernels go wrong: whole image, zero area, far edge, partly / entirely outside, flipped, NaN, thin,
+    sub-pixel and integer-aligned taps."""
+    props = rois_log_uniform(rs, B, N, lo=lo, hi=hi)
+    props[1, N - 10:] = 0                                                     # zero padded proposals -> level 2
+    props[0, 0] = [0, 0, 1, 1]                                                # last tap exactly on the far edge
+    props[0, 1] = [0.3, 0.3, 0.3, 0.3]                                        # zero area: every bin on one pixel
+    props[0, 2] = [0.25, 0.5, 1.0, 1.0]
+    props[0, 3] = [-0.1, -0.2, 0.4, 0.5]                                      # partly outside -> extrapolated bins
+    props[0, 4] = [0.5, 0.5, 1.2, 1.3]
+    props[0, 5] = [0.9, 0.1, 0.2, 0.8]                                        # flipped in y -> per-bin path
+    props[0, 6] = [0.1, 0.9, 0.8, 0.2]                                        # flipped in x
+    props[0, 7] = [np.nan, 0.1, 0.5, 0.6]
+    props[0, 8] = [0.0, 0.40, 1.0, 0.41]                                      # tall and thin: sparse rows, one column pair
+    props[0, 9] = [0.40, 0.0, 0.41, 1.0]                                      # wide and flat: many column runs
+    props[0, 10] = [1.5, 1.5, 2.0, 2.0]                                       # entirely outside
+    props[0, 11] = [0.5, 0.5, 0.5 + 1e-4, 0.5 + 1e-4]                         # sub-pixel ROI
+    props[0, 12] = [0.2, 0.2, 0.2 + 3 / 63.0, 0.2 + 3 / 63.0]                 # integer-aligned taps on P2 (lerp 0)
+    return props
+
+
 def pyramid(rs, B, sizes=(256, 128, 64, 32), D=256):
     return [rs.random_sample((B, s, s, D)).astype(f32) for s in sizes]
 

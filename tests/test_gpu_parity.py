@@ -375,21 +375,7 @@ def test_roi_pooling_d256_rows_kernel_edge_cases(pool):
     NaN, zero-area, out-of-image and whole-image ROIs on a small pyramid, every pooled value bit-identical."""
     rs = np.random.RandomState(4321 + pool[0])
     fmaps = [rs.random_sample((2, s, s, 256)).astype(f32) for s in (64, 32, 16, 8)]
-    props = _synth.rois_log_uniform(rs, 2, 160, lo=4, hi=900)
-    props[1, 150:] = 0                                                        # zero padded proposals -> level 2
-    props[0, 0] = [0, 0, 1, 1]                                                # last tap exactly on the far edge
-    props[0, 1] = [0.3, 0.3, 0.3, 0.3]                                        # zero area: every bin on one pixel
-    props[0, 2] = [0.25, 0.5, 1.0, 1.0]
-    props[0, 3] = [-0.1, -0.2, 0.4, 0.5]                                      # partly outside -> extrapolated bins
-    props[0, 4] = [0.5, 0.5, 1.2, 1.3]
-    props[0, 5] = [0.9, 0.1, 0.2, 0.8]                                        # flipped in y -> per-bin path
-    props[0, 6] = [0.1, 0.9, 0.8, 0.2]                                        # flipped in x
-    props[0, 7] = [np.nan, 0.1, 0.5, 0.6]
-    props[0, 8] = [0.0, 0.40, 1.0, 0.41]                                      # tall and thin: sparse rows, one column pair
-    props[0, 9] = [0.40, 0.0, 0.41, 1.0]                                      # wide and flat: many column runs
-    props[0, 10] = [1.5, 1.5, 2.0, 2.0]                                       # entirely outside
-    props[0, 11] = [0.5, 0.5, 0.5 + 1e-4, 0.5 + 1e-4]                         # sub-pixel ROI
-    props[0, 12] = [0.2, 0.2, 0.2 + 3 / 63.0, 0.2 + 3 / 63.0]                 # integer-aligned taps on P2 (lerp 0)
+    props = _synth.rois_with_edge_cases(rs, 2, 160)
     _roi_align_check(fmaps, props, 1024, pool)
     _roi_align_check(fmaps, props, 1024, pool)                                # again: the ticket counter was left zeroed
     from objectdetection_b200 import _lib

@@ -177,8 +177,10 @@ __device__ __forceinline__ int32_t f_to_i32_x86(float r) {
   return (int32_t)r;
 }
 
-// Order-preserving float -> uint32 (larger float = larger key); -0 == +0.
+// Order-preserving float -> uint32 (larger float = larger key); -0 == +0. Every NaN, of either sign and any payload,
+// is one value above +inf (numpy's sort order), so NaN ties go to the lower index like any other tie.
 __device__ __forceinline__ uint32_t score_key(float s) {
+  if (s != s) return 0xFFFFFFFFu;
   s = s + 0.0f;
   uint32_t b = __float_as_uint(s);
   return (b & 0x80000000u) ? ~b : (b | 0x80000000u);

@@ -42,12 +42,18 @@ det_prepare_kernel(const float4* __restrict__ proposals, const float* __restrict
   const int n = (int)slot;
   const int64_t r = (int64_t)b * N + n;
   const float* p = probs + r * C;
-  // argmax, first maximum (detection.py:115)
+  // argmax, first maximum (detection.py:115), as the sequential `best = p[0]; if (p[c] > best)` scan decides it: a NaN
+  // in p[0] wins (nothing compares greater), a NaN anywhere else is never taken. A lane's own first value is the only
+  // one it takes without a compare, so lanes other than 0 drop a NaN there.
   float best = -INFINITY;
   int arg = 0x7fffffff;
   if (lane < C) {
     best = p[lane];
     arg = lane;
+    if (lane > 0 && best != best) {
+      best = -INFINITY;
+      arg = 0x7fffffff;
+    }
     for (int c = lane + 32; c < C; c += 32) {
       const float v = p[c];
       if (v > best) {

@@ -17,7 +17,8 @@ struct __align__(16) Key128 {
 __device__ __forceinline__ bool key_less(const Key128& a, const Key128& b) {
   return (a.hi < b.hi) || (a.hi == b.hi && a.lo < b.lo);
 }
-__device__ __forceinline__ unsigned long long d_key(double s) {
+__device__ __forceinline__ unsigned long long d_key(double s) {   // score_key's order: -0 == +0, every NaN above +inf
+  if (s != s) return 0xFFFFFFFFFFFFFFFFull;
   s = s + 0.0;
   const unsigned long long b = (unsigned long long)__double_as_longlong(s);
   return (b & 0x8000000000000000ull) ? ~b : (b | 0x8000000000000000ull);
@@ -138,10 +139,14 @@ __device__ __forceinline__ PBox load_pbox(const double* b) {
   return p;
 }
 
+// The fp32 screen of frcnn_mask_kernel is exact only while every clipped coordinate is below this bound (see there);
+// larger images send every pair to the fp64 path.
+constexpr int kFrcnnScreenMaxSide = 8192;
+
 // proposals.py:141-164 as 64x64 tiles (i = kept/earlier box, j = later box).
 __global__ void __launch_bounds__(64)
 frcnn_mask_kernel(const double* __restrict__ boxes, const int32_t* __restrict__ counters, int K, int W, int Ws, double thr,
-                  unsigned long long* __restrict__ mask, unsigned long long* __restrict__ diagT) {
+                  int screen, unsigned long long* __restrict__ mask, unsigned long long* __restrict__ diagT) {
   const int cb = blockIdx.x, rb = blockIdx.y;
   if (cb < rb) return;
   const int n = min(counters[1], K);
@@ -163,9 +168,12 @@ frcnn_mask_kernel(const double* __restrict__ boxes, const int32_t* __restrict__ 
   unsigned long long bits = 0ull;
   // Screening in fp32: with pixel coordinates below 2^13 (rounding <= 5e-4 px per corner) and sides >= 1 px (the +1
   // convention) the fp32 overlap is within ~2.5e-3 of the fp64 one for the smallest boxes and ~1e-5 for typical ones, so
-  // only pairs within kMargin of the threshold (and NaNs) take the exact fp64 path of the reference.
+  // only pairs within kMargin of the threshold (and NaNs) take the exact fp64 path of the reference. The error grows
+  // with the coordinates (~1e-2 at 1.2e5 px), so `screen` is 0 for images with a side above kFrcnnScreenMaxSide (the
+  // clip keeps coordinates <= side - 1): the bounds become -inf / +inf and every pair takes the fp64 path.
+  // tests/test_filter_replays.py replays this screen in numpy over the whole screened domain.
   constexpr float kMargin = 4e-3f;
-  const float thr_hi = (float)thr + kMargin, thr_lo = (float)thr - kMargin;
+  const float thr_hi = screen ? (float)thr + kMargin : INFINITY, thr_lo = screen ? (float)thr - kMargin : -INFINITY;
   if (i < n) {
     const PBox my = load_pbox(boxes + 4 * (int64_t)i);
     const float mx1 = (float)my.x1, my1 = (float)my.y1, mx2 = (float)(my.x2 + 1), my2 = (float)(my.y2 + 1), ma = (float)my.area;
@@ -287,6 +295,7 @@ int od_frcnn_proposal_forward(const DLTensor* rpn_box_class_prob, const DLTensor
   OD_CHECK(check_tensor(num_out, "num_out", I32, 1, true, &dev));
   const int na = params->num_anchors;
   if (na < 1 || na > 16) OD_FAIL(OD_ERR_PARAM, "num_anchors must be in [1,16]");
+  if (params->image_h < 1 || params->image_w < 1) OD_FAIL(OD_ERR_PARAM, "image_h and image_w must be >= 1");
   const int64_t fh = rpn_box_class_prob->shape[1], fw = rpn_box_class_prob->shape[2];
   if (rpn_box_class_prob->shape[0] != 1 || rpn_box_class_prob->shape[3] != 2 * na) OD_FAIL(OD_ERR_SHAPE, "rpn_box_class_prob must be [1,h,w,2*na]");
   if (rpn_bbox->shape[0] != 1 || rpn_bbox->shape[1] != fh || rpn_bbox->shape[2] != fw || rpn_bbox->shape[3] != 4 * na)
@@ -326,8 +335,9 @@ int od_frcnn_proposal_forward(const DLTensor* rpn_box_class_prob, const DLTensor
       OD_LAUNCH_CHECK("frcnn_gather_kernel");
     }
     const dim3 grid((unsigned)W, (unsigned)W, 1);
-    frcnn_mask_kernel<<<grid, 64, 0, st>>>(f.sorted, f.counters, (int)K, W, (int)nms_mask_stride(K), params->nms_threshold, f.mask,
-                                           f.diagT);
+    const int screen = params->image_h <= kFrcnnScreenMaxSide && params->image_w <= kFrcnnScreenMaxSide;
+    frcnn_mask_kernel<<<grid, 64, 0, st>>>(f.sorted, f.counters, (int)K, W, (int)nms_mask_stride(K), params->nms_threshold, screen,
+                                           f.mask, f.diagT);
     OD_LAUNCH_CHECK("frcnn_mask_kernel");
   }
   OD_CHECK(nms_scan_launch(f.mask, f.diagT, f.counters + 1, 1, K, nms_mask_stride(K), post_n, f.keep_pos, f.counters + 2, nullptr, st));

@@ -62,9 +62,12 @@ static inline int32_t i32_add_wrap(int32_t a, int32_t b) {
   return (int32_t)((uint32_t)a + (uint32_t)b);
 }
 
-/* Order-preserving map float -> uint32 (larger float = larger key); -0 == +0. */
+/* Order-preserving map float -> uint32 (larger float = larger key); -0 == +0. Every NaN, of either sign and any
+ * payload, is one value above +inf (numpy's sort order; TF's comparator leaves NaNs unordered), so NaN ties go to
+ * the lower index like any other tie. */
 static inline uint32_t score_key(float s) {
   uint32_t b;
+  if (s != s) return 0xFFFFFFFFu;
   s = s + 0.0f;
   memcpy(&b, &s, 4);
   return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
@@ -608,8 +611,10 @@ ORC_API int32_t orc_frcnn_nms_sorted(const double* boxes, int32_t n, double thr,
   return (cnt < max_out) ? cnt : max_out;
 }
 
-static inline uint64_t d_key(double s) {
-  uint64_t b; s = s + 0.0; memcpy(&b, &s, 8);
+static inline uint64_t d_key(double s) {   /* score_key's order: -0 == +0, every NaN above +inf */
+  uint64_t b;
+  if (s != s) return 0xFFFFFFFFFFFFFFFFull;
+  s = s + 0.0; memcpy(&b, &s, 8);
   return (b & 0x8000000000000000ull) ? ~b : (b | 0x8000000000000000ull);
 }
 typedef struct { uint64_t key; int32_t idx; } dk_t;

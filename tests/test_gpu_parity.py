@@ -239,7 +239,8 @@ def _check_proposals(P, probs, bbox, anchors, conf, training=False):
     assert_bits(host(P.get_anchors_delta_clipped()), dbg["anchor_delta_clipped"], "clipped")
     assert np.array_equal(host(P.num_kept), dbg["num_kept"])
     assert np.array_equal(host(P.keep_idx), dbg["keep_idx"])
-    assert_bits(host(P.get_proposals()), want, "proposals")
+    # the DEBUG layer zeroes NaN rows like the reference does in DEBUG mode (proposals_tf.py:202-209)
+    assert_bits(host(P.get_proposals()), np.where(np.isnan(want), f32(0), want), "proposals")
     return want
 
 

@@ -135,19 +135,8 @@ struct Workspace {
 // the launch latency of every link overlaps its predecessor. Every kernel on the chain calls pdl_prologue() first, on
 // every path (a kernel that finished without waiting would release its own dependents too early). Without the launch
 // attribute both instructions are no-ops.
-#ifndef OD_PDL
-#define OD_PDL 1
-#endif
-__device__ __forceinline__ void pdl_launch_dependents() {
-#if OD_PDL
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
-__device__ __forceinline__ void pdl_wait() {
-#if OD_PDL
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
-}
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_prologue() {
   pdl_launch_dependents();
   pdl_wait();
@@ -161,7 +150,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = OD_PDL;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
@@ -239,32 +228,8 @@ __device__ __forceinline__ float tf_iou(const CBox& i, const CBox& j) {
 }
 
 // 16-byte global accesses with cache hints.
-#ifndef OD_LOAD_MODE
-#define OD_LOAD_MODE 0
-#endif
-#ifndef OD_STORE_MODE
-#define OD_STORE_MODE 0
-#endif
-__device__ __forceinline__ float4 ldg_f4(const float4* p) {
-#if OD_LOAD_MODE == 0
-  return __ldg(p);
-#elif OD_LOAD_MODE == 1
-  return __ldcg(p);    // L2 only
-#else
-  float4 v;
-  asm("ld.global.nc.L1::evict_last.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
-  return v;
-#endif
-}
-__device__ __forceinline__ void stg_cs_f4(float4* p, float4 v) {   // streaming store (evict first)
-#if OD_STORE_MODE == 0
-  __stcs(p, v);
-#elif OD_STORE_MODE == 1
-  *p = v;
-#else
-  __stcg(p, v);
-#endif
-}
+__device__ __forceinline__ float4 ldg_f4(const float4* p) { return __ldg(p); }
+__device__ __forceinline__ void stg_cs_f4(float4* p, float4 v) { __stcs(p, v); }   // streaming store (evict first)
 
 constexpr int kNumSMsB200 = 148;
 

@@ -22,14 +22,8 @@
 
 namespace od {
 
-#ifndef OD_MASK_COL_TILES
-#define OD_MASK_COL_TILES 4
-#endif
-constexpr int kMaskColTiles = OD_MASK_COL_TILES;   // column tiles (of 64 boxes) per CTA (A/B builds may override)
-#ifndef OD_MASK_THREADS
-#define OD_MASK_THREADS 256
-#endif
-constexpr int kMaskThreads = OD_MASK_THREADS;            // 64 rows x kMaskGroups thread groups
+constexpr int kMaskColTiles = 4;                         // column tiles (of 64 boxes) per CTA
+constexpr int kMaskThreads = 256;                        // 64 rows x kMaskGroups thread groups
 constexpr int kMaskGroups = kMaskThreads / 64;           // group h owns column tiles h, h + kMaskGroups, ... of the span
 
 template <bool FAST>  // FAST: thr >= 0, division skipped when the intersection is not positive
@@ -139,9 +133,7 @@ nms_mask_kernel(const float4* __restrict__ boxes, const int32_t* __restrict__ nu
 
 constexpr int kScanThreads = 256;
 constexpr int kScanMaxSlots = 8;
-#ifndef OD_SCAN_COPY_PARTS
-#define OD_SCAN_COPY_PARTS 4   // bulk copies per chunk of 64 mask rows (issued by different lanes of the producer warp)
-#endif
+constexpr int kScanCopyParts = 4;   // bulk copies per chunk of 64 mask rows (issued by different lanes of the producer warp)
 // named barriers (ids 1..4; 0 is __syncthreads): bar.arrive does not block, bar.sync does; both order shared memory
 __device__ __forceinline__ void nb_sync(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "n"(kScanThreads) : "memory"); }
 __device__ __forceinline__ void nb_sync_n(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
@@ -309,15 +301,15 @@ nms_scan_kernel(const unsigned long long* __restrict__ mask, const unsigned long
       for (int c = c_first; c < c_last; ++c) {
         nb_sync(1 + (c & 1));
         const int cn = c + nslots - 1;
-        if (cn < c_last && lane <= OD_SCAN_COPY_PARTS) {
+        if (cn < c_last && lane <= kScanCopyParts) {
           unsigned long long* bar = &full_bar[slot];
           unsigned long long* dst = stage + (size_t)slot * slot_words;
           const int rows = min(64, n - cn * 64);
           if (lane == 0) {
             mbar_expect_tx(bar, (uint32_t)rows * (uint32_t)Ws * 8u + 512u);
             bulk_g2s(dst + (size_t)64 * Ws, dimg + (size_t)cn * 64, 512u, bar);
-          } else {   // the rows in OD_SCAN_COPY_PARTS pieces, one lane each
-            constexpr int kPart = 64 / OD_SCAN_COPY_PARTS;
+          } else {   // the rows in kScanCopyParts pieces, one lane each
+            constexpr int kPart = 64 / kScanCopyParts;
             const int r0 = (lane - 1) * kPart, nr = min(kPart, rows - r0);
             if (nr > 0) bulk_g2s(dst + (size_t)r0 * Ws, mrow + ((size_t)cn * 64 + r0) * Ws, (uint32_t)nr * (uint32_t)Ws * 8u, bar);
           }

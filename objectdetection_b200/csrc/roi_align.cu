@@ -8,8 +8,9 @@
 // warp reads/writes 512 contiguous bytes. The reference's per-level where/gather, concat and
 // re-sort (maskrcnn.py:127-173) are not reproduced: each ROI writes straight to out[b*N+n].
 //
-//   crop_rows_kernel : D = 256 and pool widths 10..14 (the 14x14 mask-branch pooling): one persistent CTA per SM, planner /
-//      issuer / consumer warps around a TMA-fed shared-memory ring of feature rows, separable blend (described below).
+//   crop_rows_kernel : D = 256, pool height <= 16, width <= 14 and the larger side >= 10 (the 14x14 mask-branch pooling):
+//      one persistent CTA per SM, planner / issuer / consumer warps around a TMA-fed shared-memory ring of feature rows,
+//      separable blend (described below).
 //   roi_order_kernel : pre-pass of both kernels, the order in which the ROIs are walked (level by level, top to bottom).
 //   crop_bins_kernel : every other shape. The output is one flat array of bins (roi, y, x), each D*4 contiguous bytes. A CTA owns
 //      32 consecutive bins (every CTA does the same amount of work, ROI boundaries are irrelevant). Its
@@ -21,8 +22,6 @@
 //   crop_pool_bins_kernel : FasterRCNN roi_pool = crop 14x14 fused with 2x2 max-pool, same scheme over pooled bins.
 #include "common.cuh"
 #include "tma.cuh"
-
-#include <stdlib.h>
 
 namespace od {
 
@@ -103,21 +102,11 @@ struct __align__(16) BinInfo {  // base pointer (16-byte aligned) | flag in the 
   float xl, yl;
 };
 constexpr uintptr_t kBinSample = 0, kBinExtrapolate = 1, kBinSkip = 2;
-// CTA shape of the flat-bin kernels; the -D overrides exist for A/B builds (build.build_variant, tools/ab_libs.sh).
-// 128 threads x 32 bins measured best (profiles/r1_crop_variants.md).
-#ifndef OD_BIN_THREADS
-#define OD_BIN_THREADS 128
-#endif
-#ifndef OD_BIN_MINB
-#define OD_BIN_MINB 1
-#endif
-#ifndef OD_BIN_BINS
-#define OD_BIN_BINS 32
-#endif
-#ifndef OD_BIN_UNROLL
-#define OD_BIN_UNROLL 2
-#endif
-constexpr int kBinThreads = OD_BIN_THREADS;
+// CTA shape of the flat-bin kernels: 32 bins per 128-thread CTA, 2 quads in flight per thread, the best of the sweeps in
+// profiles/r1_crop_variants.md.
+constexpr int kBinThreads = 128;
+constexpr int kBinBins = 32;
+constexpr int kBinUnroll = 2;
 
 // packed fp32 pairs (sm_100 FADD2): IEEE add/sub on both halves, so results equal two scalar ops
 __device__ __forceinline__ void add2(float& d0, float& d1, float a0, float a1, float b0, float b1) {
@@ -231,7 +220,7 @@ __device__ __forceinline__ void bin_table_entry(const RoiSource& src, int64_t ro
 }
 
 template <int BINS, int UNROLL, bool POW2, bool ORDERED>
-__global__ void __launch_bounds__(kBinThreads, OD_BIN_MINB)
+__global__ void __launch_bounds__(kBinThreads, 1)
 crop_bins_kernel(RoiSource src, int64_t total_bins, int32_t bins_per_roi, int32_t ph, int32_t pw, int32_t D4,
                  int32_t lgD4, float extrap, float4* __restrict__ out, int32_t* __restrict__ level_out) {
   pdl_prologue();
@@ -391,22 +380,30 @@ roi_order_kernel(const float4* __restrict__ boxes, int32_t N, int32_t image_h, i
 //             left/right straight from the ring (4 LDS.128) into registers and the entry released; every output row is then
 //             one lerp between the two cached rows and two streaming 16-byte stores. Every feature pixel is read once from
 //             L2 per ROI and each x-blend is computed once per (row, x) instead of once per bin.
-//   ROIs the plan cannot serve (flipped / NaN / partly outside boxes, rows wider than half the ring) take a per-bin path
-//   with direct loads on the consumer warps.
+//   ROIs the plan cannot serve (flipped / NaN / partly outside boxes) take a per-bin path with direct loads on the
+//   consumer warps.
 // Arithmetic per output value is the reference's (crop_and_resize_op.cc): top = tl + (tr - tl) * xl, bot likewise,
 // out = top + (bot - top) * yl, so the results are bit-identical to crop_bins_kernel and to the oracle.
-// Template parameters select measured alternatives kept for A/B runs (env OD_ROI_*): TMAST = output rows staged in shared
-// memory and written by bulk shared->global copies (2-8 % slower), QPL = channel quads per lane (1: two warps per x bin),
-// MAXT/MINB = launch bounds (two 64-register CTAs per SM with half the ring each: 10 % slower).
-constexpr int kRowsMaxPool = 16;
+// Measured and slower (profiles/r2_roialign.md): output rows written by bulk shared->global copies (2-8 %), one channel
+// quad per lane with two warps per x bin, two 64-register CTAs per SM with half the ring each (10 %), L2 evict_last
+// hints on the ring copies and an L2 prefetch of the planned rows.
+constexpr int kRowsThreads = 512;
+constexpr int kRowsMaxPool = 16;                // plan tables: pool height <= 16 (the width is capped by kRowsMaxWidth)
+constexpr int kRowsMaxWidth = kRowsThreads / 32 - 2;   // one consumer warp per x bin next to the issuer and the planner
+constexpr int kRowsMinPool = 10;                // smaller pools leave too few consumer warps per SM: 7x7 takes 0.063 ms
+                                                // here against 0.043 ms in crop_bins_kernel (profiles/r2_roialign.md)
 constexpr int kRowsEntries = 32;                // outstanding ring entries (one feature row each)
-#ifndef OD_ROWS_PLANS
-#define OD_ROWS_PLANS 3
-#endif
-constexpr int kRowsPlans = OD_ROWS_PLANS;       // plans in flight
-constexpr int kRowsStages = 2;                  // output staging slots (1 KiB each) per consumer warp, TMA-store variant
+constexpr int kRowsPlans = 3;                   // plans in flight
 constexpr int kRowsD4 = 64;                     // D = 256 floats = 64 quads = 1 KiB per pixel
 constexpr uint32_t kRowsPixelBytes = 1024;
+// Ring size: 176 KiB. The kernel alone is ~1 % faster with everything an SM has (221 KiB), but leaving ~45 KiB lets the
+// small CTAs of concurrently running kernels (the other steps' proposal front and 7x7 ROIAlign) become resident next to
+// it, which is worth 8 % of whole-step throughput (profiles/r2_roialign.md).
+constexpr uint32_t kRowsRingBytes = 176 * 1024;
+// A row may have to skip the tail of the ring (it never straddles the end): row + skipped tail must fit an EMPTY ring,
+// which holds for every head position only if a row is at most half the ring. A row holds the distinct columns of one
+// ROI, at most two per x sample.
+static_assert(2u * (2 * kRowsMaxWidth) * kRowsPixelBytes <= kRowsRingBytes, "a ring row can exceed half the ring");
 
 struct RowsPlan {
   int2 ytab[kRowsMaxPool + 2];                  // ring mode, per y: {y_lerp bits, top row == bottom row}; two pad entries
@@ -419,13 +416,12 @@ struct RowsPlan {
   int32_t run_col[kRowsMaxPool], run_rank[kRowsMaxPool], run_len[kRowsMaxPool];
   int32_t nr, ncols, nruns, mode;
   int32_t W;
-  int32_t keep;                                 // issuer: copy this ROI's rows with the L2 evict_last policy
   uint32_t row_bytes;                           // ncols KiB: one ring entry
   int64_t roi;
   const float* base;
 };
 // ring: every bin of the ROI has four valid taps and the grid steps are non-negative (the streaming fast path);
-// flat: anything else (extrapolated bins, flipped / NaN boxes, rows wider than the ring) - per-bin direct loads;
+// flat: anything else (extrapolated bins, flipped / NaN boxes) - per-bin direct loads;
 // skip: box_ind out of range, the crop is left untouched; done: no ROI left for this CTA.
 constexpr int kRowsRing = 0, kRowsFlat = 1, kRowsSkip = 2, kRowsDone = 3;
 
@@ -465,8 +461,7 @@ __device__ __forceinline__ uintptr_t roi_geometry(const RoiSource& src, int64_t 
 // sample; first-use order is ascending order, the rank of a new tap is the number of new taps before it (two
 // ballots and a popcount) and a repeated tap is the largest or second largest value seen so far.
 __device__ __forceinline__ void rows_make_plan(const RoiSource& src, int64_t roi, float4 box, int32_t bidx, int32_t ph,
-                                               int32_t pw, uint32_t ring_bytes, int32_t l2_keep, int32_t lane, RowsPlan& P,
-                                               RowsShared& S, int32_t* level_out) {
+                                               int32_t pw, int32_t lane, RowsPlan& P, RowsShared& S, int32_t* level_out) {
   RoiMeta m;
   int32_t level = 0;
   const uintptr_t flag = roi_geometry(src, roi, box, bidx, ph, pw, m, &level);
@@ -495,7 +490,7 @@ __device__ __forceinline__ void rows_make_plan(const RoiSource& src, int64_t roi
     }
   }
   const bool all_ok = __all_sync(0xffffffffu, ok);  // every bin has four valid taps
-  int32_t mode = (flag == kBinSkip) ? kRowsSkip : ((all_ok && mono) ? kRowsRing : kRowsFlat);
+  const int32_t mode = (flag == kBinSkip) ? kRowsSkip : ((all_ok && mono) ? kRowsRing : kRowsFlat);
   if (mode == kRowsRing) {
     const int32_t plo = __shfl_up_sync(0xffffffffu, lo, 1), phi = __shfl_up_sync(0xffffffffu, hi, 1);
     const bool new_lo = valid && (i == 0 || (lo != plo && lo != phi));
@@ -542,9 +537,6 @@ __device__ __forceinline__ void rows_make_plan(const RoiSource& src, int64_t roi
       P.run_rank[j] = lane;
       P.run_len[j] = (rest ? __ffs(rest) - 1 : nc) - lane;
     }
-    // A row may have to skip the tail of the ring (it never straddles the end): row + skipped tail must fit an EMPTY
-    // ring, which holds for every head position only if a row is at most half the ring. Wider rows take the flat path.
-    if (2u * (uint32_t)nc * kRowsPixelBytes > ring_bytes) mode = kRowsFlat;
     if (lane == 0) {
       P.nr = nr;
       P.ncols = nc;
@@ -557,7 +549,6 @@ __device__ __forceinline__ void rows_make_plan(const RoiSource& src, int64_t roi
     P.base = m.base;
     P.W = m.W;
     P.mode = mode;
-    P.keep = l2_keep == 1 || (l2_keep == 2 && src.mode == 0 && level > src.min_level);
     if (level_out && src.mode == 0) level_out[roi] = level;
   }
   __syncwarp();
@@ -565,18 +556,16 @@ __device__ __forceinline__ void rows_make_plan(const RoiSource& src, int64_t roi
 
 // counter[0]: next ROI ticket, counter[1]: CTAs that have drawn their last ticket. Both are zero between launches: the
 // last CTA to finish resets them (the workspace is zero-initialised once by its owner).
-template <bool TMAST, int QPL, int MAXT, int MINB>
-__global__ void __launch_bounds__(MAXT, MINB)
-crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t ring_bytes, float extrap,
-                 float4* __restrict__ out, int32_t* __restrict__ level_out, unsigned int* __restrict__ counter,
-                 int32_t l2_prefetch, int32_t l2_keep, int32_t dbg) {
+// Warps 0 .. pw-1 are the consumers (warp = x bin), warp pw the issuer, warp pw+1 the planner.
+__global__ void __launch_bounds__(kRowsThreads, 1)
+crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, float extrap, float4* __restrict__ out,
+                 int32_t* __restrict__ level_out, unsigned int* __restrict__ counter) {
   pdl_prologue();
   extern __shared__ __align__(128) unsigned char s_ring[];
   __shared__ RowsShared S;
   const int32_t t = threadIdx.x;
   const int32_t lane = t & 31, warp = t >> 5;
-  constexpr int kWarpsPerBin = 2 / QPL;            // QPL channel quads per lane: 2 -> one consumer warp per x bin, 1 -> two
-  const int32_t n_cwarps = pw * kWarpsPerBin, n_cons = 32 * n_cwarps;
+  const int32_t n_cwarps = pw, n_cons = 32 * n_cwarps;
   if (t == 0) {
     for (int32_t e = 0; e < kRowsEntries; ++e) {
       mbar_init(&S.full[e], 1);
@@ -649,22 +638,9 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t
         }
         __syncwarp();
       } else {
-        rows_make_plan(src, roi, box, bi, ph, pw, ring_bytes, l2_keep, lane, P, S, level_out);
+        rows_make_plan(src, roi, box, bi, ph, pw, lane, P, S, level_out);
       }
       if (lane == 0) mbar_arrive(&S.plan_full[ps]);
-      if (l2_prefetch && P.mode == kRowsRing) {
-        // The planner runs a few ROIs ahead of the ring: pull this ROI's rows into L2 now, so that the ring copies issued
-        // later pay an L2 hit instead of a DRAM access queued behind the output stream.
-        const char* __restrict__ gbase = reinterpret_cast<const char*>(P.base);
-        const size_t row_pitch = (size_t)P.W * kRowsPixelBytes;
-        const int32_t nruns = P.nruns, total = P.nr * nruns;
-        for (int32_t i = lane; i < total; i += 32) {
-          const int32_t kk = i / nruns, j = i - kk * nruns;
-          const char* a = gbase + (size_t)P.rows[kk] * row_pitch + (size_t)P.run_col[j] * kRowsPixelBytes;
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a), "r"((uint32_t)P.run_len[j] * kRowsPixelBytes)
-                       : "memory");
-        }
-      }
       if (++ps == kRowsPlans) {
         ps = 0;
         pphase ^= 1u;
@@ -683,18 +659,17 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t
     uint32_t head = 0, used = 0;
     int32_t e_idx = 0, old_idx = 0, outstanding = 0;
     uint32_t old_phase = 0;
-    const uint64_t pol_keep = l2_policy_evict_last(), pol_normal = l2_policy_evict_normal();
+    const uint64_t pol = l2_policy_evict_normal();
     for (;;) {
       mbar_wait(&S.plan_full[ps], pphase);
       const RowsPlan& P = S.plan[ps];
       const int32_t mode = P.mode;
       if (mode == kRowsDone) return;
-      if (mode == kRowsRing && !(dbg & 2)) {
+      if (mode == kRowsRing) {
         const int32_t nr = P.nr, nruns = P.nruns;
         const uint32_t bytes = P.row_bytes;
         const char* __restrict__ gbase = reinterpret_cast<const char*>(P.base);
         const size_t row_pitch = (size_t)P.W * kRowsPixelBytes;
-        const uint64_t pol = P.keep ? pol_keep : pol_normal;
         // this lane's column run (nruns <= 16): smem offset inside the row, global offset inside the feature row, bytes
         const int32_t jr = lane < nruns ? lane : 0;
         const uint32_t run_dst = (uint32_t)P.run_rank[jr] * kRowsPixelBytes;
@@ -702,10 +677,10 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t
         const uint32_t run_bytes = (uint32_t)P.run_len[jr] * kRowsPixelBytes;
         int32_t my_row = lane < nr ? P.rows[lane] : 0;           // rank k's feature row lives on lane k (nr <= 32)
         for (int32_t k = 0; k < nr; ++k) {
-          const bool wrap = head + bytes > ring_bytes;            // the tail a wrapped row skips counts as part of it
-          const uint32_t need = bytes + (wrap ? ring_bytes - head : 0u);
-          OD_DBG_ASSERT(need <= ring_bytes, "a row and the ring tail it skips exceed the ring");
-          while (used + need > ring_bytes || outstanding == kRowsEntries) {
+          const bool wrap = head + bytes > kRowsRingBytes;        // the tail a wrapped row skips counts as part of it
+          const uint32_t need = bytes + (wrap ? kRowsRingBytes - head : 0u);
+          OD_DBG_ASSERT(need <= kRowsRingBytes, "a row and the ring tail it skips exceed the ring");
+          while (used + need > kRowsRingBytes || outstanding == kRowsEntries) {
             mbar_wait(&S.empty[old_idx], old_phase);              // reclaim the oldest entry (FIFO)
             used -= S.entry_fp[old_idx];
             --outstanding;
@@ -715,7 +690,7 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t
             }
           }
           const uint32_t off = wrap ? 0u : head;
-          OD_DBG_ASSERT(off + bytes <= ring_bytes && run_dst + run_bytes <= bytes && bytes > 0, "row outside the ring");
+          OD_DBG_ASSERT(off + bytes <= kRowsRingBytes && run_dst + run_bytes <= bytes && bytes > 0, "row outside the ring");
           OD_DBG_IDX(e_idx, kRowsEntries);
           head = off + bytes;
           used += need;
@@ -740,16 +715,10 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t
   }
 
   // -------------------------------------------------------------------- consumers
-  // QPL = 2: warp = x bin, lane = channel quads `lane` and `lane + 32`: one output pixel (1 KiB) per warp and output row.
-  // QPL = 1: two warps per x bin, one quad per lane (twice the warps for the same registers per thread).
-  // TMAST: the pixel is staged in a per-warp shared-memory slot and leaves through the bulk-copy engine (lane 0 issues
-  // one 1 KiB shared->global copy per output row and only ever waits for the slot it is about to overwrite), so the
-  // number of stores in flight does not depend on registers or on LSU back-pressure.
-  const int32_t x = warp / kWarpsPerBin, qoff = (warp % kWarpsPerBin) * 32 + lane;
+  // warp = x bin, lane = channel quads `lane` and `lane + 32`: one output pixel (1 KiB) per warp and output row.
+  const int32_t x = warp;
   const float4 ext4 = make_float4(extrap, extrap, extrap, extrap);
-  float4* const stage = reinterpret_cast<float4*>(s_ring + ring_bytes) + warp * (kRowsStages * kRowsD4);   // (TMAST: QPL = 2)
-  const uint64_t pol_out = l2_policy_evict_first();
-  int32_t e_idx = 0, st = 0;
+  int32_t e_idx = 0;
   uint32_t e_phase = 0, c_head = 0;              // ring entry, its phase, and the issuer's head replayed locally
   for (;;) {
     mbar_wait(&S.plan_full[ps], pphase);
@@ -759,25 +728,23 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t
     float4* __restrict__ o = out + P.roi * ((int64_t)ph * pw * kRowsD4);
     if (mode == kRowsRing) {
       // Column ranks -> float4 index inside a ring row (+ the channel quad).
-      const int32_t xcl = P.x_cl[x] * kRowsD4 + qoff, xcr = P.x_cr[x] * kRowsD4 + qoff;
+      const int32_t xcl = P.x_cl[x] * kRowsD4 + lane, xcr = P.x_cr[x] * kRowsD4 + lane;
       const float xl = P.x_lerp[x];
       const int32_t nr = P.nr;
       const uint32_t row_bytes = P.row_bytes;
       // Rank-major walk: the y's whose top row has rank k are contiguous (P.yfirst), their bottom row is rank k or k+1.
       // Rows alternate between RA (even ranks) and RB (odd ranks). bottom - top is recomputed per y: a group holds 1.2 y's
       // on average, caching the difference would only cost registers.
-      float4 RA[QPL], RB[QPL];
-#pragma unroll
-      for (int i = 0; i < QPL; ++i) RA[i] = RB[i] = ext4;
+      float4 RA[2], RB[2];
+      RA[0] = RA[1] = RB[0] = RB[1] = ext4;
 #define OD_ROWS_LOAD(V)                                                                              \
   do {                                                                                               \
-    if (dbg & 2) break;               /* timing experiment: no input stream at all */                \
-    const uint32_t off_ = (c_head + row_bytes > ring_bytes) ? 0u : c_head;                           \
+    const uint32_t off_ = (c_head + row_bytes > kRowsRingBytes) ? 0u : c_head;                       \
     c_head = off_ + row_bytes;                                                                       \
-    OD_DBG_ASSERT(c_head <= ring_bytes && (uint32_t)(xcr + 32 * (QPL - 1)) * 16u < row_bytes && xcl <= xcr, "ring read outside the row"); \
+    OD_DBG_ASSERT(c_head <= kRowsRingBytes && (uint32_t)(xcr + 32) * 16u < row_bytes && xcl <= xcr, "ring read outside the row"); \
     mbar_wait(&S.full[e_idx], e_phase);                                                              \
     const float4* rowp = reinterpret_cast<const float4*>(s_ring + off_);                             \
-    _Pragma("unroll") for (int i = 0; i < QPL; ++i) {                                                \
+    _Pragma("unroll") for (int i = 0; i < 2; ++i) {                                                  \
       const float4 l_ = rowp[xcl + 32 * i], r_ = rowp[xcr + 32 * i];                                 \
       V[i] = axpy4p(l_, sub4p(r_, l_), xl);                                                          \
     }                                                                                                \
@@ -788,22 +755,6 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t
       e_phase ^= 1u;                                                                                 \
     }                                                                                                \
   } while (0)
-#define OD_ROWS_PUT(V)                                                                               \
-  if (TMAST) {                                                                                       \
-    float4* sp_ = stage + st * kRowsD4;                                                              \
-    if (lane == 0) bulk_wait_read<kRowsStages - 1>();   /* the copy that last read this slot is done */ \
-    __syncwarp();                                                                                    \
-    _Pragma("unroll") for (int i = 0; i < QPL; ++i) sp_[lane + 32 * i] = V[i];                       \
-    fence_proxy_async_smem();                                                                        \
-    __syncwarp();                                                                                    \
-    if (lane == 0) {                                                                                 \
-      if (!(dbg & 1)) bulk_s2g_hint(orow, sp_, kRowsPixelBytes, pol_out);                            \
-      bulk_commit();                                                                                 \
-    }                                                                                                \
-    if (++st == kRowsStages) st = 0;                                                                 \
-  } else if (!(dbg & 1)) {                                                                           \
-    _Pragma("unroll") for (int i = 0; i < QPL; ++i) stg_cs_f4(orow + qoff + 32 * i, V[i]);           \
-  }
 #define OD_ROWS_GROUP(CUR, NXT)                                                                      \
   {                                                                                                  \
     OD_DBG_IDX(k + 1, 2 * kRowsMaxPool + 1);                                                         \
@@ -814,13 +765,13 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t
     _Pragma("unroll 1") while (y < yend) {                                                           \
       const int2 nxt_ = P.ytab[y + 2];      /* two rows ahead: the read is off the critical path */    \
       const float yl = __int_as_float(ent.x);                                                        \
-      float4 v_[QPL];                                                                                \
+      float4 v_[2];                                                                                  \
       if (ent.y) {                    /* top row == bottom row: (top - top) * yl, as the reference */ \
-        _Pragma("unroll") for (int i = 0; i < QPL; ++i) v_[i] = axpy4p(CUR[i], sub4p(CUR[i], CUR[i]), yl); \
+        _Pragma("unroll") for (int i = 0; i < 2; ++i) v_[i] = axpy4p(CUR[i], sub4p(CUR[i], CUR[i]), yl); \
       } else {                                                                                       \
-        _Pragma("unroll") for (int i = 0; i < QPL; ++i) v_[i] = axpy4p(CUR[i], sub4p(NXT[i], CUR[i]), yl); \
+        _Pragma("unroll") for (int i = 0; i < 2; ++i) v_[i] = axpy4p(CUR[i], sub4p(NXT[i], CUR[i]), yl); \
       }                                                                                              \
-      OD_ROWS_PUT(v_)                                                                                \
+      _Pragma("unroll") for (int i = 0; i < 2; ++i) stg_cs_f4(orow + lane + 32 * i, v_[i]);          \
       ent = ent1;                                                                                    \
       ent1 = nxt_;                                                                                   \
       ++y;                                                                                           \
@@ -829,7 +780,7 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t
     if (!more) break;                                                                                \
     ++k;                                                                                             \
   }
-      float4* __restrict__ orow = o + x * kRowsD4;    // this warp's pixel of output row 0 (TMAST: the bulk copy's target)
+      float4* __restrict__ orow = o + x * kRowsD4;    // this warp's pixel of output row 0
       int2 ent = P.ytab[0], ent1 = P.ytab[1];
       int32_t y = 0, k = 0;
       OD_ROWS_LOAD(RA);
@@ -838,7 +789,6 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t
         OD_ROWS_GROUP(RB, RA)
       }
 #undef OD_ROWS_LOAD
-#undef OD_ROWS_PUT
 #undef OD_ROWS_GROUP
     } else if (mode == kRowsFlat) {   // per-bin path: 4 direct loads per output quad
       const float4* __restrict__ base = reinterpret_cast<const float4*>(P.base);
@@ -869,7 +819,6 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, uint32_t
       pphase ^= 1u;
     }
   }
-  if (TMAST && lane == 0) bulk_wait_read<0>();        // the staging slots must outlive the copies that read them
 }
 
 // FasterRCNN roi_pool (fastrcnn.py:22-70): crop_and_resize to (2*oh) x (2*ow) fused with max_pool 2x2 / stride 2.
@@ -929,96 +878,33 @@ crop_pool_bins_kernel(RoiSource src, int64_t total_bins, int32_t oh, int32_t ow,
 }
 
 // ----------------------------------------------------------------------------- host side
-// Tunables of the TMA-staged kernel, read once from the environment (A/B runs on one box without rebuilding); the
-// defaults are the measured best (profiles/r2_roialign.md):
-//   OD_ROI_KERNEL=flat   forces crop_bins_kernel;       OD_ROI_MIN_POOL  smallest max(pool_h, pool_w) served (default 10);
-//   OD_ROI_CPS           persistent CTAs per SM: 1 (default, up to 128 registers) or 2 (64 registers, half the ring each);
-//   OD_ROI_RING_KB       shared-memory ring per CTA (default 176 with one CTA per SM, else what two CTAs can share);
-//   OD_ROI_QPL=1         two consumer warps per x bin (one channel quad per lane) instead of one;
-//   OD_ROI_TMA_STORE=1   output rows staged in shared memory and written by bulk shared->global copies;
-//   OD_ROI_DYNAMIC=0     static round robin even with a workspace;   OD_ROI_ORDER=0|1|2  ROI order pre-pass off / for this
-//   kernel only / for the flat kernel too (default);   OD_ROI_L2_KEEP, OD_ROI_L2_PREFETCH  L2 policy experiments.
-struct RowsTuning {
-  bool use_rows, dynamic, tma_store;
-  int ring_kb;
-  int cps, qpl, min_pool, l2_prefetch, l2_keep, dbg;
-};
-static int env_int(const char* name, int dflt, int lo, int hi) {
-  const char* v = getenv(name);
-  int x = v ? atoi(v) : dflt;
-  return x < lo ? lo : (x > hi ? hi : x);
-}
-static const RowsTuning& rows_tuning() {
-  static const RowsTuning t = [] {
-    RowsTuning r;
-    const char* k = getenv("OD_ROI_KERNEL");
-    r.use_rows = !(k && strcmp(k, "flat") == 0);
-    r.ring_kb = env_int("OD_ROI_RING_KB", 0, 0, 222);       // 0: derived from the CTA count per SM
-    r.cps = env_int("OD_ROI_CPS", 1, 1, 2);
-    r.qpl = env_int("OD_ROI_QPL", 2, 1, 2);
-    r.min_pool = env_int("OD_ROI_MIN_POOL", 10, 1, 17);
-    r.dynamic = env_int("OD_ROI_DYNAMIC", 1, 0, 1) != 0;
-    r.tma_store = env_int("OD_ROI_TMA_STORE", 0, 0, 1) != 0;   // measured slower (profiles/r2_roialign.md): opt-in
-    r.l2_prefetch = env_int("OD_ROI_L2_PREFETCH", 0, 0, 1);
-    r.l2_keep = env_int("OD_ROI_L2_KEEP", 0, 0, 2);         // 1: every level evict_last, 2: all but the finest level
-    r.dbg = env_int("OD_ROI_TIMING_EXPERIMENT", 0, 0, 3);   // 1: no output stores, 2: no input stream (WRONG RESULTS; timing only)
-    return r;
-  }();
-  return t;
-}
-
-template <bool TMAST, int QPL, int MAXT, int MINB>
-static int launch_crop_rows_t(const RoiSource& src, int64_t n_rois, int32_t ph, int32_t pw, const RowsTuning& tn,
-                              float extrap, float* out, int32_t* level_out, unsigned int* counter, cudaStream_t st) {
-  auto kern = crop_rows_kernel<TMAST, QPL, MAXT, MINB>;
-  static uint32_t configured[64] = {0};    // dynamic shared memory opted in, per device
-  static int sms[64] = {0};
-  int dev = 0;
-  OD_CUDA(cudaGetDevice(&dev));
-  if (dev < 0 || dev >= 64) OD_FAIL(OD_ERR_DEVICE, "device index %d not supported", dev);
-  // Ring size. One CTA per SM (default): 176 KiB - the kernel alone is ~1 % faster with everything an SM has (221 KiB),
-  // but leaving ~45 KiB lets the small CTAs of concurrently running kernels (the other steps' proposal front and 7x7
-  // ROIAlign) become resident next to it, which is worth 8 % of whole-step throughput (profiles/r2_roialign.md).
-  // Two CTAs per SM: what is left of 227 KiB after the static part and the staging slots of the TMA-store variant.
-  const uint32_t stage_bytes = TMAST ? (uint32_t)pw * kRowsStages * kRowsPixelBytes : 0u;
-  uint32_t ring_bytes = tn.ring_kb ? (uint32_t)tn.ring_kb * 1024u
-                        : (tn.cps == 1) ? 176u * 1024u - stage_bytes
-                                                  : ((227u * 1024u) / (uint32_t)tn.cps - 6u * 1024u - stage_bytes) & ~1023u;
-  const uint32_t dyn = ring_bytes + stage_bytes;
-  if (dyn > 222u * 1024u) OD_FAIL(OD_ERR_PARAM, "OD_ROI_RING_KB too large: %u bytes of dynamic shared memory", dyn);
-  if (configured[dev] < dyn) {
-    OD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-    configured[dev] = dyn;
-  }
-  if (!sms[dev]) OD_CUDA(cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev));
-  const int64_t grid = n_rois < (int64_t)sms[dev] * tn.cps ? n_rois : (int64_t)sms[dev] * tn.cps;
-  OD_CUDA(launch_pdl(kern, dim3((unsigned)grid), dim3((unsigned)(32 * pw * (2 / QPL) + 64)), (size_t)dyn, st, src, n_rois, ph, pw,
-                     ring_bytes, extrap, reinterpret_cast<float4*>(out), level_out, counter, tn.l2_prefetch, tn.l2_keep, tn.dbg));
-  OD_LAUNCH_CHECK("crop_rows_kernel");
-  return OD_OK;
+// Shapes crop_rows_kernel serves; every other shape goes to crop_bins_kernel.
+static bool crop_rows_serves(const RoiSource& src, int64_t n_rois, int32_t ph, int32_t pw, int32_t D) {
+  const int32_t pmax = ph > pw ? ph : pw;
+  if (D != 4 * kRowsD4 || ph > kRowsMaxPool || pw > kRowsMaxWidth || pmax < kRowsMinPool || src.mode > 1) return false;
+  return n_rois + 4096 <= 0x7FFFFFFFll;
 }
 
 // returns OD_OK after launching, or 1 when the shape is not served by this kernel (caller falls back to crop_bins).
 // `counter`: two zeroed uint32 in the caller's workspace (dynamic ROI scheduling) or NULL (static round robin).
-// one consumer warp per x bin + issuer + planner in a 512-thread CTA: pool widths up to 14
-static bool crop_rows_serves(const RoiSource& src, int64_t n_rois, int32_t ph, int32_t pw, int32_t D) {
-  const RowsTuning& tn = rows_tuning();
-  const int32_t pmax = ph > pw ? ph : pw;
-  if (!tn.use_rows || D != 4 * kRowsD4 || ph > kRowsMaxPool || pw > 14 || pmax < tn.min_pool || src.mode > 1) return false;
-  return n_rois + 4096 <= 0x7FFFFFFFll;
-}
 static int launch_crop_rows(const RoiSource& src, int64_t n_rois, int32_t ph, int32_t pw, int32_t D, float extrap, float* out,
                             int32_t* level_out, unsigned int* counter, cudaStream_t st) {
-  const RowsTuning& tn = rows_tuning();
   if (!crop_rows_serves(src, n_rois, ph, pw, D)) return 1;
-  if (!tn.dynamic) counter = nullptr;
-#define OD_ROWS_GO(T, Q, M, B) return launch_crop_rows_t<T, Q, M, B>(src, n_rois, ph, pw, tn, extrap, out, level_out, counter, st)
-  if (tn.tma_store && tn.cps == 1) OD_ROWS_GO(true, 2, 512, 1);
-  if (tn.tma_store) OD_ROWS_GO(true, 2, 512, 2);
-  if (tn.qpl == 1 && tn.cps == 1) OD_ROWS_GO(false, 1, 1024, 1);    // 2 warps per x bin, one CTA per SM
-  if (tn.cps == 1) OD_ROWS_GO(false, 2, 512, 1);                    // one CTA per SM: up to 128 registers per thread
-  OD_ROWS_GO(false, 2, 512, 2);
-#undef OD_ROWS_GO
+  static bool configured[64] = {false};    // dynamic shared memory opted in, per device
+  static int sms[64] = {0};
+  int dev = 0;
+  OD_CUDA(cudaGetDevice(&dev));
+  if (dev < 0 || dev >= 64) OD_FAIL(OD_ERR_DEVICE, "device index %d not supported", dev);
+  if (!configured[dev]) {
+    OD_CUDA(cudaFuncSetAttribute(crop_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRowsRingBytes));
+    configured[dev] = true;
+  }
+  if (!sms[dev]) OD_CUDA(cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev));
+  const int64_t grid = n_rois < (int64_t)sms[dev] ? n_rois : (int64_t)sms[dev];
+  OD_CUDA(launch_pdl(crop_rows_kernel, dim3((unsigned)grid), dim3((unsigned)(32 * pw + 64)), (size_t)kRowsRingBytes, st, src,
+                     n_rois, ph, pw, extrap, reinterpret_cast<float4*>(out), level_out, counter));
+  OD_LAUNCH_CHECK("crop_rows_kernel");
+  return OD_OK;
 }
 
 static int launch_roi_order(const RoiSource& src, int32_t* order_buf, cudaStream_t st) {
@@ -1039,10 +925,8 @@ static int launch_crop_bins(RoiSource src, int64_t n_rois, int32_t ph, int32_t p
   // persistent 14x14 kernel. For the flat 7x7 kernel the launch itself gets ~2 us faster but its pre-pass adds more than
   // that to a stand-alone call; with several steps in flight (the throughput case) that latency is hidden and the order is
   // worth +2.5 % images/s, so it is on for both (profiles/r2_roialign.md).
-  static const int use_order = env_int("OD_ROI_ORDER", 2, 0, 2);   // 1: crop_rows_kernel only, 2: the flat kernel too
   src.order = nullptr;
-  const bool order_ok = use_order && src.mode == 0 && D == 4 * kRowsD4 && n_rois <= 0x7FFFFFFFll &&
-                        (use_order == 2 || crop_rows_serves(src, n_rois, ph, pw, D));
+  const bool order_ok = src.mode == 0 && D == 4 * kRowsD4 && n_rois <= 0x7FFFFFFFll;
   if (order_ok && order_in) {
     src.order = order_in;
   } else if (order_ok && order_buf && n_rois >= 512 && src.rois_per_image <= kOrderThreads * kOrderPerThread) {
@@ -1066,15 +950,13 @@ static int launch_crop_bins(RoiSource src, int64_t n_rois, int32_t ph, int32_t p
   }
   if (lg >= 0 && D4 >= 16) {
     if ((int64_t)64 * D4 > 0x7FFFFFFFll) OD_FAIL(OD_ERR_PARAM, "depth %d too large", D);
-    constexpr int BINS = OD_BIN_BINS;
-    const int64_t grid = (total_bins + BINS - 1) / BINS;
+    const int64_t grid = (total_bins + kBinBins - 1) / kBinBins;
     if (grid > 0x7FFFFFFFll) OD_FAIL(OD_ERR_PARAM, "too many bins: %lld", (long long)total_bins);
-    // 32 bins per 128-thread CTA, 2 quads in flight per thread: best of the sweeps in profiles/r1_crop_variants.md
     if (src.order)
-      OD_CUDA(launch_pdl(crop_bins_kernel<BINS, OD_BIN_UNROLL, true, true>, dim3((unsigned)grid), dim3(kBinThreads), 0, st,
+      OD_CUDA(launch_pdl(crop_bins_kernel<kBinBins, kBinUnroll, true, true>, dim3((unsigned)grid), dim3(kBinThreads), 0, st,
           src, total_bins, (int32_t)bins_per_roi, ph, pw, D4, lg, extrap, reinterpret_cast<float4*>(out), level_out));
     else
-      OD_CUDA(launch_pdl(crop_bins_kernel<BINS, OD_BIN_UNROLL, true, false>, dim3((unsigned)grid), dim3(kBinThreads), 0, st,
+      OD_CUDA(launch_pdl(crop_bins_kernel<kBinBins, kBinUnroll, true, false>, dim3((unsigned)grid), dim3(kBinThreads), 0, st,
           src, total_bins, (int32_t)bins_per_roi, ph, pw, D4, lg, extrap, reinterpret_cast<float4*>(out), level_out));
   } else {
     // thin or non-power-of-two depth: more bins per CTA so that the table build is amortised

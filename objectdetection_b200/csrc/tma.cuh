@@ -44,12 +44,7 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, u
                : "memory");
 }
 
-// L2 eviction policies for the bulk copies (createpolicy; a 64-bit opaque operand of the .L2::cache_hint forms)
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
+// L2 eviction policy for the bulk copies (createpolicy; a 64-bit opaque operand of the .L2::cache_hint forms)
 __device__ __forceinline__ uint64_t l2_policy_evict_normal() {
   uint64_t pol;
   asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol));
@@ -62,25 +57,6 @@ __device__ __forceinline__ void bulk_g2s_hint(void* smem_dst, const void* gmem_s
                "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
                : "memory");
 }
-
-// shared -> global bulk copies (TMA store engine; SASS UBLKCP.G.S / UBLKRED-class): completion is tracked per issuing
-// THREAD in bulk groups; wait_read<N> returns when all but the N most recent groups have finished READING shared memory.
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ void bulk_s2g_hint(void* gmem_dst, const void* smem_src, uint32_t bytes, uint64_t policy) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(gmem_dst),
-               "r"(smem_u32(smem_src)), "r"(bytes), "l"(policy)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_read() {
-  asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // plain arrive (count 1) on a CTA-local mbarrier: consumers release a ring slot with it
 __device__ __forceinline__ void mbar_arrive(unsigned long long* bar) {

@@ -4,8 +4,8 @@ against the CPU oracle as strictly as test_gpu_parity.py does, and read from a C
 kernel ran and its sibling did not, so that a retuned threshold cannot silently turn a test into a test of another
 branch. Non-power-of-two depths are also compared with a float64 numpy crop_and_resize written here.
 
-KERNEL_PATHS names, for every __global__ kernel in objectdetection_b200/csrc, the test that launches it or the reason
-no default configuration does; test_kernel_paths_cover_every_kernel (no GPU) fails when a kernel is missing from it."""
+KERNEL_PATHS names, for every __global__ kernel in objectdetection_b200/csrc, the test that launches it;
+test_kernel_paths_cover_every_kernel (no GPU) fails when a kernel is missing from it."""
 import ctypes
 import glob
 import os
@@ -28,7 +28,6 @@ f32 = np.float32
 CSRC = os.path.join(os.path.dirname(HERE), "objectdetection_b200", "csrc")
 
 P, D_ = "test_gpu_parity.py::", "test_gpu_dispatch.py::"
-ENV_ONLY = "not run: chosen only by the OD_ROI_* developer environment switches of roi_align.cu"
 KERNEL_PATHS = {
     # topk.cu
     "topk_collect_kernel": P + "test_topk",
@@ -59,15 +58,11 @@ KERNEL_PATHS = {
     "rpn_emit_kernel": P + "test_rpn_targets_golden_and_coco_shape",
     # roi_align.cu
     "crop_bins_kernel<32, 2, true, true>": P + "test_roi_pooling_processing_order",
-    "crop_bins_kernel<32, 2, true, false>": D_ + "test_roi_align_d256_rows_kernel_bounds",
+    "crop_bins_kernel<32, 2, true, false>": D_ + "test_roi_align_d256_crop_rows_serves_bounds",
     "crop_bins_kernel<512, 2, true, false>": P + "test_crop_and_resize_generic",
     "crop_bins_kernel<512, 2, false, false>": D_ + "test_roi_align_non_power_of_two_depth",
     "roi_order_kernel": P + "test_roi_pooling_processing_order",
-    "crop_rows_kernel<false, 2, 512, 1>": D_ + "test_roi_align_d256_rows_kernel_bounds",
-    "crop_rows_kernel<false, 2, 512, 2>": ENV_ONLY + " (OD_ROI_CPS=2: two CTAs per SM)",
-    "crop_rows_kernel<false, 1, 1024, 1>": ENV_ONLY + " (OD_ROI_QPL=1: two consumer warps per x bin)",
-    "crop_rows_kernel<true, 2, 512, 1>": ENV_ONLY + " (OD_ROI_TMA_STORE=1: bulk-store variant)",
-    "crop_rows_kernel<true, 2, 512, 2>": ENV_ONLY + " (OD_ROI_TMA_STORE=1 with OD_ROI_CPS=2)",
+    "crop_rows_kernel": D_ + "test_roi_align_d256_crop_rows_serves_bounds",
     "crop_pool_bins_kernel": D_ + "test_roi_pool_non_power_of_two_depth",
     # nms.cu
     "nms_mask_kernel<true>": D_ + "test_nms_thresholds_zero_one_and_padded_rows",
@@ -116,8 +111,7 @@ def _kernels_in_sources():
 
 
 def test_kernel_paths_cover_every_kernel():
-    """Every __global__ kernel has a KERNEL_PATHS entry; every entry names a kernel that exists and either a test that
-    exists or the reason no default configuration launches it."""
+    """Every __global__ kernel has a KERNEL_PATHS entry; every entry names a kernel that exists and a test that exists."""
     kernels = _kernels_in_sources()
     assert len(kernels) > 40, kernels
     covered = {k.split("<")[0] for k in KERNEL_PATHS}
@@ -126,8 +120,6 @@ def test_kernel_paths_cover_every_kernel():
     stale = sorted(covered - kernels)
     assert not stale, f"KERNEL_PATHS entries for kernels that no longer exist: {stale}"
     for kernel, where in KERNEL_PATHS.items():
-        if where.startswith("not run: "):
-            continue
         fname, test = where.split("::")
         src = open(os.path.join(HERE, fname)).read()
         assert re.search(rf"^def {re.escape(test)}\(", src, re.M), f"{kernel}: {where} does not exist"
@@ -415,7 +407,7 @@ def test_roi_align_non_power_of_two_depth(_cuda, kernel_trace, D):
     kernel = "od::crop_bins_kernel<512, 2, false, false>("
     for pool in ([7, 7], [14, 14]):
         got, names = kernel_trace(lambda: _roi_align_check(fmaps, props, 1024, pool))
-        assert_launched(names, must=[kernel], must_not=["od::crop_rows_kernel<", "od::crop_bins_kernel<32,"])
+        assert_launched(names, must=[kernel], must_not=["od::crop_rows_kernel(", "od::crop_bins_kernel<32,"])
         want, ok = _pyramid_f64(fmaps, props, pool)
         _assert_close_f64(got[0], want, ok, f"pyramid D={D} {pool}")
     img = rs.random_sample((3, 19, 23, D)).astype(f32)
@@ -459,7 +451,7 @@ def test_roi_pool_non_power_of_two_depth(_cuda, kernel_trace):
 @pytest.mark.gpu
 @pytest.mark.parametrize("pool,rows", [([1, 14], True), ([14, 1], True), ([16, 14], True), ([10, 10], True),
                                        ([9, 9], False), ([17, 14], False)])
-def test_roi_align_d256_rows_kernel_bounds(_cuda, kernel_trace, pool, rows):
+def test_roi_align_d256_crop_rows_serves_bounds(_cuda, kernel_trace, pool, rows):
     """The bounds of crop_rows_serves at D = 256: pool height <= 16, width <= 14 and max(height, width) >= 10 take the
     TMA-staged row kernel; just outside them the flat per-bin kernel runs. Same edge-case ROIs, bit-exact either way."""
     rs = np.random.RandomState(4321 + 100 * pool[0] + pool[1])
@@ -467,9 +459,9 @@ def test_roi_align_d256_rows_kernel_bounds(_cuda, kernel_trace, pool, rows):
     props = _synth.rois_with_edge_cases(rs, 2, 160)
     _, names = kernel_trace(lambda: _roi_align_check(fmaps, props, 1024, pool))
     if rows:
-        assert_launched(names, must=["od::crop_rows_kernel<false, 2, 512, 1>("], must_not=["od::crop_bins_kernel<"])
+        assert_launched(names, must=["od::crop_rows_kernel("], must_not=["od::crop_bins_kernel<"])
     else:
-        assert_launched(names, must=["od::crop_bins_kernel<32, 2, true, false>("], must_not=["od::crop_rows_kernel<"])
+        assert_launched(names, must=["od::crop_bins_kernel<32, 2, true, false>("], must_not=["od::crop_rows_kernel("])
 
 
 # ------------------------------------------------------------------ DetectionTargetLayer

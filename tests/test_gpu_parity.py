@@ -441,9 +441,6 @@ def test_roi_pooling_caller_supplied_order(pool):
     assert sorted(host(order).tolist()) == list(range(1200))
     got = host(pyramid_roi_align(fm, pr, [1024, 1024, 3], pool, order=order))
     assert_bits(got, want, "pooled with a caller-supplied order")
-    mode = int(os.environ.get("OD_ROI_ORDER", "2"))      # developer switch of the library: 0 = orders are ignored,
-    if mode == 0 or (mode == 1 and pool[0] < 10):        # 1 = only the row-ring kernel (pool >= 10) walks an order
-        return
     bad = host(order).copy()
     skipped = [int(bad[3]), int(bad[700])]
     bad[3], bad[700] = -1, 5000                       # two ROIs are never visited ...

@@ -1,6 +1,7 @@
 #!/bin/bash
-# Developer aid: A/B several builds of libodhead (objectdetection_b200/libodhead_<name>.so, see build.build_variant) in ONE
-# GPU session, since box-to-box variance is ~8 %. Usage: bash tools/ab_libs.sh name1 name2 ...   ("base" = libodhead.so)
+# Developer aid: A/B several builds of libodhead in ONE GPU session, since box-to-box variance is ~8 %. Each build is an
+# objectdetection_b200/libodhead_<name>.so, e.g. the library of another commit or a build.build_variant build.
+# Usage: bash tools/ab_libs.sh name1 name2 ...   ("base" = libodhead.so)
 for rep in 1 2; do
 for name in "$@"; do
   lib=$PWD/objectdetection_b200/libodhead_$name.so

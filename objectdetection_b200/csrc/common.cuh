@@ -13,6 +13,7 @@
 #include <stdio.h>
 #include <stdarg.h>
 #include <string.h>
+#include <initializer_list>
 
 #include "../../include/odhead.h"
 
@@ -56,23 +57,40 @@ void count_launches(int n);
   } while (0)
 
 // ----------------------------------------------------------------------------- device selection
-// Every entry point declares one DeviceScope before it validates its tensors. check_tensor() activates it with the
-// device id of the first tensor it sees: if that is not the calling thread's current device, the scope switches to it
-// (kernel launches, cudaFuncSetAttribute and cooperative-launch queries then address the tensors' GPU) and the
-// destructor restores the caller's device.
+// Every entry point declares one DeviceScope and passes it to check_tensor() for each of its tensors. The first tensor
+// checked selects the device: if that is not the calling thread's current device, the scope switches to it (kernel
+// launches, cudaFuncSetAttribute and cooperative-launch queries then address the tensors' GPU), every later tensor
+// must be on it, and the destructor restores the caller's device.
 struct DeviceScope {
+  int device = -1;
   int prev = -1;
-  bool active = false, switched = false;
-  DeviceScope* outer;
-  DeviceScope();
-  ~DeviceScope();
-  static void activate(int device_id);
+  bool switched = false;
+  ~DeviceScope() {
+    if (switched) cudaSetDevice(prev);
+  }
 };
 
 // ----------------------------------------------------------------------------- DLPack checks
 enum DType { F32, F64, I32 };
-int check_tensor(const DLTensor* t, const char* name, DType dt, int ndim, bool need_contig, int* device);
-bool is_contiguous(const DLTensor* t);
+// An extent check_tensor accepts at any value. A caller's int64 parameter is checked for a negative value before it is
+// used as an extent, so that it cannot pass as kAny.
+constexpr int64_t kAny = INT64_MIN;
+// Validates one tensor argument, in this order: not NULL, a kDLCUDA tensor on the call's device (see DeviceScope), dtype
+// `dt`, rank ndim, no negative extent, C-contiguous (any_strides: any strides), a data pointer unless it is empty,
+// extent i == extents[i] (kAny: any value), and, unless it is empty, a data pointer aligned to align_bytes: the size of
+// the type the kernels read it as (16 for float4, 8 for float2 and double, else 4). ndim < 0 checks neither rank nor
+// extents.
+int check_tensor(const DLTensor* t, const char* name, DType dt, const int64_t* extents, int ndim, int align_bytes,
+                 DeviceScope& scope, bool any_strides = false);
+inline int check_tensor(const DLTensor* t, const char* name, DType dt, std::initializer_list<int64_t> extents,
+                        int align_bytes, DeviceScope& scope, bool any_strides = false) {
+  return check_tensor(t, name, dt, extents.begin(), (int)extents.size(), align_bytes, scope, any_strides);
+}
+// The same for an optional argument: NULL is accepted.
+inline int check_opt_tensor(const DLTensor* t, const char* name, DType dt, std::initializer_list<int64_t> extents,
+                            int align_bytes, DeviceScope& scope) {
+  return t ? check_tensor(t, name, dt, extents, align_bytes, scope) : OD_OK;
+}
 inline int64_t numel(const DLTensor* t) {
   int64_t n = 1;
   for (int i = 0; i < t->ndim; ++i) n *= t->shape[i];

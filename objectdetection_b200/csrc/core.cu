@@ -6,20 +6,6 @@ namespace od {
 static thread_local char g_detail[512] = "";
 static unsigned long long g_launches = 0;
 
-static thread_local DeviceScope* g_scope = nullptr;
-DeviceScope::DeviceScope() : outer(g_scope) { g_scope = this; }
-DeviceScope::~DeviceScope() {
-  if (switched) cudaSetDevice(prev);
-  g_scope = outer;
-}
-void DeviceScope::activate(int device_id) {
-  DeviceScope* s = g_scope;
-  if (!s || s->active) return;
-  s->active = true;
-  if (cudaGetDevice(&s->prev) != cudaSuccess) return;
-  if (s->prev != device_id && cudaSetDevice(device_id) == cudaSuccess) s->switched = true;
-}
-
 void count_launches(int n) { __atomic_fetch_add(&g_launches, (unsigned long long)n, __ATOMIC_RELAXED); }
 
 void set_error_detail(const char* fmt, ...) {
@@ -29,7 +15,7 @@ void set_error_detail(const char* fmt, ...) {
   va_end(ap);
 }
 
-bool is_contiguous(const DLTensor* t) {
+static bool is_contiguous(const DLTensor* t) {
   if (!t->strides) return true;
   int64_t expect = 1;
   for (int i = t->ndim - 1; i >= 0; --i) {
@@ -39,16 +25,17 @@ bool is_contiguous(const DLTensor* t) {
   return true;
 }
 
-int check_tensor(const DLTensor* t, const char* name, DType dt, int ndim, bool need_contig, int* device) {
+int check_tensor(const DLTensor* t, const char* name, DType dt, const int64_t* extents, int ndim, int align_bytes,
+                 DeviceScope& scope, bool any_strides) {
   if (!t) OD_FAIL(OD_ERR_NULL, "%s is NULL", name);
   if (t->device.device_type != kDLCUDA)
     OD_FAIL(OD_ERR_DEVICE, "%s: device_type %d is not kDLCUDA (there is no CPU path)", name, (int)t->device.device_type);
-  if (device) {
-    if (*device < 0) {
-      *device = t->device.device_id;
-      DeviceScope::activate(*device);
-    } else if (*device != t->device.device_id)
-      OD_FAIL(OD_ERR_DEVICE, "%s is on cuda:%d, expected cuda:%d", name, t->device.device_id, *device);
+  if (scope.device < 0) {
+    scope.device = t->device.device_id;
+    if (cudaGetDevice(&scope.prev) == cudaSuccess && scope.prev != scope.device && cudaSetDevice(scope.device) == cudaSuccess)
+      scope.switched = true;
+  } else if (scope.device != t->device.device_id) {
+    OD_FAIL(OD_ERR_DEVICE, "%s is on cuda:%d, expected cuda:%d", name, t->device.device_id, scope.device);
   }
   const uint8_t code = (dt == I32) ? (uint8_t)kDLInt : (uint8_t)kDLFloat;
   const uint8_t bits = (dt == F64) ? 64 : 32;
@@ -58,8 +45,14 @@ int check_tensor(const DLTensor* t, const char* name, DType dt, int ndim, bool n
   if (ndim >= 0 && t->ndim != ndim) OD_FAIL(OD_ERR_SHAPE, "%s: rank %d != %d", name, t->ndim, ndim);
   for (int i = 0; i < t->ndim; ++i)
     if (t->shape[i] < 0) OD_FAIL(OD_ERR_SHAPE, "%s: negative extent", name);
-  if (need_contig && !is_contiguous(t)) OD_FAIL(OD_ERR_LAYOUT, "%s must be C-contiguous", name);
-  if (numel(t) > 0 && dptr<char>(t) == nullptr) OD_FAIL(OD_ERR_NULL, "%s: data pointer is NULL", name);
+  if (!any_strides && !is_contiguous(t)) OD_FAIL(OD_ERR_LAYOUT, "%s must be C-contiguous", name);
+  const bool empty = numel(t) == 0;
+  if (!empty && dptr<char>(t) == nullptr) OD_FAIL(OD_ERR_NULL, "%s: data pointer is NULL", name);
+  for (int i = 0; i < ndim; ++i)
+    if (extents[i] != kAny && t->shape[i] != extents[i])
+      OD_FAIL(OD_ERR_SHAPE, "%s: extent %d is %lld, expected %lld", name, i, (long long)t->shape[i], (long long)extents[i]);
+  if (!empty && reinterpret_cast<uintptr_t>(dptr<char>(t)) % align_bytes)
+    OD_FAIL(OD_ERR_LAYOUT, "%s is not %d-byte aligned", name, align_bytes);
   return OD_OK;
 }
 

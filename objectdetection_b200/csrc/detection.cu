@@ -358,13 +358,6 @@ static size_t carve_det_ws(Workspace& w, int64_t B, int64_t N, DetWs* out) {
   return w.off + 256;
 }
 
-static int check_opt3(const DLTensor* t, const char* name, DType dt, int* dev, int64_t a, int64_t b, int64_t c) {
-  if (!t) return OD_OK;
-  OD_CHECK(check_tensor(t, name, dt, c < 0 ? 2 : 3, true, dev));
-  if (t->shape[0] != a || t->shape[1] != b || (c >= 0 && t->shape[2] != c)) OD_FAIL(OD_ERR_SHAPE, "%s has the wrong shape", name);
-  return OD_OK;
-}
-
 }  // namespace od
 
 using namespace od;
@@ -381,36 +374,26 @@ int od_detection_forward(const DLTensor* proposals, const DLTensor* mrcnn_class_
                          const od_detection_debug* debug, void* ws, size_t ws_bytes, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (!params) OD_FAIL(OD_ERR_NULL, "params is NULL");
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(proposals, "proposals", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(mrcnn_class_probs, "mrcnn_class_probs", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(mrcnn_bbox, "mrcnn_bbox", F32, 4, true, &dev));
-  OD_CHECK(check_tensor(window_norm, "window_norm", F32, 2, true, &dev));
-  OD_CHECK(check_tensor(detections, "detections", F32, 3, true, &dev));
+  DeviceScope scope;
+  OD_CHECK(check_tensor(proposals, "proposals", F32, {kAny, kAny, 4}, 16, scope));
+  OD_CHECK(check_tensor(mrcnn_class_probs, "mrcnn_class_probs", F32, {proposals->shape[0], proposals->shape[1], kAny}, 4, scope));
   const int64_t B = mrcnn_class_probs->shape[0], N = mrcnn_class_probs->shape[1], C = mrcnn_class_probs->shape[2];
   const int64_t M = params->max_instances;
-  if (proposals->shape[0] != B || proposals->shape[1] != N || proposals->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "proposals must be [B,N,4]");
-  if (mrcnn_bbox->shape[0] != B || mrcnn_bbox->shape[1] != N || mrcnn_bbox->shape[2] != C || mrcnn_bbox->shape[3] != 4)
-    OD_FAIL(OD_ERR_SHAPE, "mrcnn_bbox must be [B,N,C,4]");
-  if (window_norm->shape[0] != B || window_norm->shape[1] != 4) OD_FAIL(OD_ERR_SHAPE, "window_norm must be [B,4]");
-  if (M < 0 || detections->shape[0] != B || detections->shape[1] != M || detections->shape[2] != 6)
-    OD_FAIL(OD_ERR_SHAPE, "detections must be [B,max_instances,6]");
+  OD_CHECK(check_tensor(mrcnn_bbox, "mrcnn_bbox", F32, {B, N, C, 4}, 16, scope));
+  OD_CHECK(check_tensor(window_norm, "window_norm", F32, {B, 4}, 16, scope));
+  OD_CHECK(check_tensor(detections, "detections", F32, {B, M, 6}, 4, scope));
   if (N > 16384 || C > 65535 || C < 1) OD_FAIL(OD_ERR_PARAM, "DetectionLayer supports N <= 16384 ROIs and 1 <= C <= 65535 classes");
   if (B > 65535) OD_FAIL(OD_ERR_PARAM, "batch > 65535");
-  if (reinterpret_cast<uintptr_t>(dptr<float>(proposals)) % 16 || reinterpret_cast<uintptr_t>(dptr<float>(mrcnn_bbox)) % 16 ||
-      reinterpret_cast<uintptr_t>(dptr<float>(window_norm)) % 16)
-    OD_FAIL(OD_ERR_LAYOUT, "proposals / mrcnn_bbox / window_norm must be 16-byte aligned");
   od_detection_debug dbg;
   memset(&dbg, 0, sizeof(dbg));
   if (debug) dbg = *debug;
-  OD_CHECK(check_opt3(dbg.class_ids, "debug.class_ids", I32, &dev, B, N, -1));
-  OD_CHECK(check_opt3(dbg.class_scores, "debug.class_scores", F32, &dev, B, N, -1));
-  OD_CHECK(check_opt3(dbg.bbox_delta, "debug.bbox_delta", F32, &dev, B, N, 4));
-  OD_CHECK(check_opt3(dbg.refined_proposals, "debug.refined_proposals", F32, &dev, B, N, 4));
-  OD_CHECK(check_opt3(dbg.clipped_proposals, "debug.clipped_proposals", F32, &dev, B, N, 4));
-  OD_CHECK(check_opt3(dbg.keep_mask, "debug.keep_mask", I32, &dev, B, N, -1));
-  OD_CHECK(check_opt3(dbg.nms_keep_mask, "debug.nms_keep_mask", I32, &dev, B, N, -1));
+  OD_CHECK(check_opt_tensor(dbg.class_ids, "debug.class_ids", I32, {B, N}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.class_scores, "debug.class_scores", F32, {B, N}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.bbox_delta, "debug.bbox_delta", F32, {B, N, 4}, 16, scope));
+  OD_CHECK(check_opt_tensor(dbg.refined_proposals, "debug.refined_proposals", F32, {B, N, 4}, 16, scope));
+  OD_CHECK(check_opt_tensor(dbg.clipped_proposals, "debug.clipped_proposals", F32, {B, N, 4}, 16, scope));
+  OD_CHECK(check_opt_tensor(dbg.keep_mask, "debug.keep_mask", I32, {B, N}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.nms_keep_mask, "debug.nms_keep_mask", I32, {B, N}, 4, scope));
   if (B == 0 || M == 0) return OD_OK;
   if (N == 0) {
     OD_CUDA(cudaMemsetAsync(dptr<float>(detections), 0, sizeof(float) * (size_t)(B * M * 6), st));
@@ -465,23 +448,15 @@ int od_detection_forward(const DLTensor* proposals, const DLTensor* mrcnn_class_
 
 int od_unmold_detections(const DLTensor* detections, const DLTensor* window_norm, const DLTensor* original_shape,
                          DLTensor* boxes, DLTensor* class_ids, DLTensor* scores, DLTensor* counts, void* stream) {
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(detections, "detections", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(window_norm, "window_norm", F32, 2, true, &dev));
-  OD_CHECK(check_tensor(original_shape, "original_shape", I32, 2, true, &dev));
-  OD_CHECK(check_tensor(boxes, "boxes", I32, 3, true, &dev));
-  OD_CHECK(check_tensor(class_ids, "class_ids", I32, 2, true, &dev));
-  OD_CHECK(check_tensor(scores, "scores", F32, 2, true, &dev));
-  OD_CHECK(check_tensor(counts, "counts", I32, 1, true, &dev));
+  DeviceScope scope;
+  OD_CHECK(check_tensor(detections, "detections", F32, {kAny, kAny, 6}, 4, scope));
   const int64_t B = detections->shape[0], M = detections->shape[1];
-  if (detections->shape[2] != 6) OD_FAIL(OD_ERR_SHAPE, "detections must be [B,M,6]");
-  if (window_norm->shape[0] != B || window_norm->shape[1] != 4) OD_FAIL(OD_ERR_SHAPE, "window_norm must be [B,4]");
-  if (original_shape->shape[0] != B || original_shape->shape[1] != 2) OD_FAIL(OD_ERR_SHAPE, "original_shape must be [B,2] (h,w)");
-  if (boxes->shape[0] != B || boxes->shape[1] != M || boxes->shape[2] != 4 || class_ids->shape[0] != B ||
-      class_ids->shape[1] != M || scores->shape[0] != B || scores->shape[1] != M || counts->shape[0] != B)
-    OD_FAIL(OD_ERR_SHAPE, "outputs must be boxes [B,M,4], class_ids [B,M], scores [B,M], counts [B]");
-  if (reinterpret_cast<uintptr_t>(dptr<float>(window_norm)) % 16) OD_FAIL(OD_ERR_LAYOUT, "window_norm must be 16-byte aligned");
+  OD_CHECK(check_tensor(window_norm, "window_norm", F32, {B, 4}, 16, scope));
+  OD_CHECK(check_tensor(original_shape, "original_shape", I32, {B, 2}, 4, scope));
+  OD_CHECK(check_tensor(boxes, "boxes", I32, {B, M, 4}, 4, scope));
+  OD_CHECK(check_tensor(class_ids, "class_ids", I32, {B, M}, 4, scope));
+  OD_CHECK(check_tensor(scores, "scores", F32, {B, M}, 4, scope));
+  OD_CHECK(check_tensor(counts, "counts", I32, {B}, 4, scope));
   if (B > 0x7FFFFFFFll || M > (1 << 24)) OD_FAIL(OD_ERR_PARAM, "batch / rows out of range");
   if (B == 0) return OD_OK;
   unmold_kernel<<<(unsigned)B, kUnmoldThreads, 0, static_cast<cudaStream_t>(stream)>>>(

@@ -285,24 +285,19 @@ int od_frcnn_proposal_forward(const DLTensor* rpn_box_class_prob, const DLTensor
                               DLTensor* proposals, DLTensor* num_out, void* ws, size_t ws_bytes, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (!params) OD_FAIL(OD_ERR_NULL, "params is NULL");
-  if (!rpn_box_class_prob || !rpn_bbox) OD_FAIL(OD_ERR_NULL, "inputs are NULL");
+  if (!rpn_box_class_prob) OD_FAIL(OD_ERR_NULL, "rpn_box_class_prob is NULL");   // its dtype selects that of rpn_bbox
   const bool f64 = rpn_box_class_prob->dtype.bits == 64;
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(rpn_box_class_prob, "rpn_box_class_prob", f64 ? F64 : F32, 4, true, &dev));
-  OD_CHECK(check_tensor(rpn_bbox, "rpn_bbox", f64 ? F64 : F32, 4, true, &dev));
-  OD_CHECK(check_tensor(proposals, "proposals", F32, 2, true, &dev));
-  OD_CHECK(check_tensor(num_out, "num_out", I32, 1, true, &dev));
   const int na = params->num_anchors;
   if (na < 1 || na > 16) OD_FAIL(OD_ERR_PARAM, "num_anchors must be in [1,16]");
   if (params->image_h < 1 || params->image_w < 1) OD_FAIL(OD_ERR_PARAM, "image_h and image_w must be >= 1");
-  const int64_t fh = rpn_box_class_prob->shape[1], fw = rpn_box_class_prob->shape[2];
-  if (rpn_box_class_prob->shape[0] != 1 || rpn_box_class_prob->shape[3] != 2 * na) OD_FAIL(OD_ERR_SHAPE, "rpn_box_class_prob must be [1,h,w,2*na]");
-  if (rpn_bbox->shape[0] != 1 || rpn_bbox->shape[1] != fh || rpn_bbox->shape[2] != fw || rpn_bbox->shape[3] != 4 * na)
-    OD_FAIL(OD_ERR_SHAPE, "rpn_bbox must be [1,h,w,4*na]");
   const int64_t post_n = params->post_nms_top_n;
   if (post_n < 0 || params->pre_nms_top_n < 0) OD_FAIL(OD_ERR_PARAM, "negative top-n");
-  if (proposals->shape[0] != post_n || proposals->shape[1] != 5 || num_out->shape[0] != 1) OD_FAIL(OD_ERR_SHAPE, "proposals must be [post_nms_top_n,5], num_out [1]");
+  DeviceScope scope;
+  OD_CHECK(check_tensor(rpn_box_class_prob, "rpn_box_class_prob", f64 ? F64 : F32, {1, kAny, kAny, 2 * na}, f64 ? 8 : 4, scope));
+  const int64_t fh = rpn_box_class_prob->shape[1], fw = rpn_box_class_prob->shape[2];
+  OD_CHECK(check_tensor(rpn_bbox, "rpn_bbox", f64 ? F64 : F32, {1, fh, fw, 4 * na}, f64 ? 8 : 4, scope));
+  OD_CHECK(check_tensor(proposals, "proposals", F32, {post_n, 5}, 4, scope));
+  OD_CHECK(check_tensor(num_out, "num_out", I32, {1}, 4, scope));
   const int64_t total = fh * fw * na;
   const int64_t K = total < params->pre_nms_top_n ? total : params->pre_nms_top_n;
   if (post_n == 0) return OD_OK;

@@ -245,42 +245,26 @@ int od_rpn_loss_forward(const DLTensor* rpn_target_class, const DLTensor* rpn_cl
                         const DLTensor* rpn_pred_box, DLTensor* losses, DLTensor* pred_box_pos, DLTensor* num_pos, void* ws,
                         size_t ws_bytes, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(rpn_target_class, "rpn_target_class", I32, -1, true, &dev));
-  OD_CHECK(check_tensor(rpn_class_logits, "rpn_class_logits", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(losses, "losses", F32, 1, true, &dev));
-  const int64_t B = rpn_class_logits->shape[0], A = rpn_class_logits->shape[1];
-  const bool tc_ok = (rpn_target_class->ndim == 2 || (rpn_target_class->ndim == 3 && rpn_target_class->shape[2] == 1)) &&
-                     rpn_target_class->shape[0] == B && rpn_target_class->shape[1] == A;
-  if (!tc_ok) OD_FAIL(OD_ERR_SHAPE, "rpn_target_class must be [B,A] or [B,A,1]");
-  if (rpn_class_logits->shape[2] != 2) OD_FAIL(OD_ERR_SHAPE, "rpn_class_logits must be [B,A,2]");
+  DeviceScope scope;
+  if (rpn_target_class && rpn_target_class->ndim == 3)
+    OD_CHECK(check_tensor(rpn_target_class, "rpn_target_class", I32, {kAny, kAny, 1}, 4, scope));
+  else
+    OD_CHECK(check_tensor(rpn_target_class, "rpn_target_class", I32, {kAny, kAny}, 4, scope));
+  const int64_t B = rpn_target_class->shape[0], A = rpn_target_class->shape[1];
+  OD_CHECK(check_tensor(rpn_class_logits, "rpn_class_logits", F32, {B, A, 2}, 8, scope));
+  OD_CHECK(check_tensor(losses, "losses", F32, {2}, 4, scope));
   const bool with_box = rpn_target_bbox && rpn_pred_box;   // both NULL: class loss only (losses[1] = 0)
   if (!with_box && (rpn_target_bbox || rpn_pred_box || pred_box_pos)) OD_FAIL(OD_ERR_NULL, "rpn_target_bbox and rpn_pred_box go together");
   int64_t T = 0;
   if (with_box) {
-    OD_CHECK(check_tensor(rpn_target_bbox, "rpn_target_bbox", F32, 3, true, &dev));
-    OD_CHECK(check_tensor(rpn_pred_box, "rpn_pred_box", F32, 3, true, &dev));
+    OD_CHECK(check_tensor(rpn_target_bbox, "rpn_target_bbox", F32, {B, kAny, 4}, 16, scope));
+    OD_CHECK(check_tensor(rpn_pred_box, "rpn_pred_box", F32, {B, A, 4}, 16, scope));
     T = rpn_target_bbox->shape[1];
-    if (rpn_pred_box->shape[0] != B || rpn_pred_box->shape[1] != A || rpn_pred_box->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "rpn_pred_box must be [B,A,4]");
-    if (rpn_target_bbox->shape[0] != B || rpn_target_bbox->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "rpn_target_bbox must be [B,T,4]");
-    if (reinterpret_cast<uintptr_t>(dptr<float>(rpn_pred_box)) % 16 || reinterpret_cast<uintptr_t>(dptr<float>(rpn_target_bbox)) % 16)
-      OD_FAIL(OD_ERR_LAYOUT, "box tensors must be 16-byte aligned");
   }
-  if (losses->shape[0] != 2) OD_FAIL(OD_ERR_SHAPE, "losses must be [2]");
   if (A >= (1ll << 31) || B > 65535) OD_FAIL(OD_ERR_PARAM, "supports A < 2^31, B <= 65535");
-  int64_t pos_rows = 0;
-  if (pred_box_pos) {
-    OD_CHECK(check_tensor(pred_box_pos, "pred_box_pos", F32, 2, true, &dev));
-    if (pred_box_pos->shape[1] != 4) OD_FAIL(OD_ERR_SHAPE, "pred_box_pos must be [P,4]");
-    pos_rows = pred_box_pos->shape[0];
-  }
-  if (num_pos) {
-    OD_CHECK(check_tensor(num_pos, "num_pos", I32, 1, true, &dev));
-    if (num_pos->shape[0] != 1) OD_FAIL(OD_ERR_SHAPE, "num_pos must be [1]");
-  }
-  if (reinterpret_cast<uintptr_t>(dptr<float>(rpn_class_logits)) % 8 || (pred_box_pos && reinterpret_cast<uintptr_t>(dptr<float>(pred_box_pos)) % 16))
-    OD_FAIL(OD_ERR_LAYOUT, "rpn_class_logits / pred_box_pos must be 8 / 16-byte aligned");
+  OD_CHECK(check_opt_tensor(pred_box_pos, "pred_box_pos", F32, {kAny, 4}, 16, scope));
+  const int64_t pos_rows = pred_box_pos ? pred_box_pos->shape[0] : 0;
+  OD_CHECK(check_opt_tensor(num_pos, "num_pos", I32, {1}, 4, scope));
   if (!ws) OD_FAIL(OD_ERR_WORKSPACE, "workspace is NULL");
   Workspace w(ws, ws_bytes);
   const int64_t nchunk = (A + kLossChunk - 1) / kLossChunk;
@@ -306,38 +290,27 @@ int od_mrcnn_loss_forward(const DLTensor* target_class_ids, const DLTensor* pred
                           const DLTensor* target_box, const DLTensor* pred_box, DLTensor* losses, DLTensor* pred_active,
                           void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(target_class_ids, "mrcnn_target_class_ids", I32, 2, true, &dev));
-  OD_CHECK(check_tensor(losses, "losses", F32, 1, true, &dev));
+  DeviceScope scope;
+  OD_CHECK(check_tensor(target_class_ids, "mrcnn_target_class_ids", I32, {kAny, kAny}, 4, scope));
+  OD_CHECK(check_tensor(losses, "losses", F32, {2}, 4, scope));
   const bool with_cls = pred_logits && active_class_ids, with_box = target_box && pred_box;   // either pair may be NULL
   if ((!with_cls && (pred_logits || active_class_ids || pred_active)) || (!with_box && (target_box || pred_box)) || (!with_cls && !with_box))
-    OD_FAIL(OD_ERR_NULL, "pass (pred_logits, active_class_ids) and / or (target_box, pred_box)");
+    OD_FAIL(OD_ERR_NULL, "pass (mrcnn_pred_logits, batch_active_class_ids) and / or (mrcnn_target_box, mrcnn_pred_box)");
   const int64_t B = target_class_ids->shape[0], R = target_class_ids->shape[1];
   int64_t C = 0;
   if (with_cls) {
-    OD_CHECK(check_tensor(pred_logits, "mrcnn_pred_logits", F32, 3, true, &dev));
-    OD_CHECK(check_tensor(active_class_ids, "batch_active_class_ids", F32, 2, true, &dev));
+    OD_CHECK(check_tensor(pred_logits, "mrcnn_pred_logits", F32, {B, R, kAny}, 4, scope));
     C = pred_logits->shape[2];
-    if (pred_logits->shape[0] != B || pred_logits->shape[1] != R) OD_FAIL(OD_ERR_SHAPE, "mrcnn_pred_logits must be [B,R,C]");
-    if (active_class_ids->shape[0] < 1 || active_class_ids->shape[1] != C) OD_FAIL(OD_ERR_SHAPE, "batch_active_class_ids must be [B,C]");
+    OD_CHECK(check_tensor(active_class_ids, "batch_active_class_ids", F32, {kAny, C}, 4, scope));
+    if (active_class_ids->shape[0] < 1) OD_FAIL(OD_ERR_SHAPE, "batch_active_class_ids must be [B,C]");
   }
   if (with_box) {
-    OD_CHECK(check_tensor(target_box, "mrcnn_target_box", F32, 3, true, &dev));
-    OD_CHECK(check_tensor(pred_box, "mrcnn_pred_box", F32, 4, true, &dev));
+    OD_CHECK(check_tensor(target_box, "mrcnn_target_box", F32, {B, R, 4}, 16, scope));
+    OD_CHECK(check_tensor(pred_box, "mrcnn_pred_box", F32, {B, R, with_cls ? C : kAny, 4}, 16, scope));
     if (!with_cls) C = pred_box->shape[2];
-    if (target_box->shape[0] != B || target_box->shape[1] != R || target_box->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "mrcnn_target_box must be [B,R,4]");
-    if (pred_box->shape[0] != B || pred_box->shape[1] != R || pred_box->shape[2] != C || pred_box->shape[3] != 4)
-      OD_FAIL(OD_ERR_SHAPE, "mrcnn_pred_box must be [B,R,C,4]");
-    if (reinterpret_cast<uintptr_t>(dptr<float>(target_box)) % 16 || reinterpret_cast<uintptr_t>(dptr<float>(pred_box)) % 16)
-      OD_FAIL(OD_ERR_LAYOUT, "box tensors must be 16-byte aligned");
   }
-  if (losses->shape[0] != 2) OD_FAIL(OD_ERR_SHAPE, "losses must be [2]");
   if (C < 1 || C > (1 << 20)) OD_FAIL(OD_ERR_PARAM, "class count out of range");
-  if (pred_active) {
-    OD_CHECK(check_tensor(pred_active, "pred_active", F32, 2, true, &dev));
-    if (pred_active->shape[0] != B || pred_active->shape[1] != R) OD_FAIL(OD_ERR_SHAPE, "pred_active must be [B,R]");
-  }
+  OD_CHECK(check_opt_tensor(pred_active, "pred_active", F32, {B, R}, 4, scope));
   mrcnn_loss_kernel<<<1, 1024, 0, st>>>(dptr<int32_t>(target_class_ids), dptr<float>(pred_logits), dptr<float>(active_class_ids),
                                         dptr<float4>(target_box), dptr<float4>(pred_box), B * R, (int)C, dptr<float>(losses),
                                         dptr<float>(pred_active));

@@ -912,23 +912,14 @@ size_t od_nms_workspace_bytes(int64_t batch, int64_t num_boxes) {
 int od_nms(const DLTensor* boxes, const DLTensor* scores, const DLTensor* num_valid, float iou_threshold,
            int64_t max_out, DLTensor* keep_idx, DLTensor* num_kept, void* ws, size_t ws_bytes, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(boxes, "boxes", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(scores, "scores", F32, 2, true, &dev));
-  OD_CHECK(check_tensor(keep_idx, "keep_idx", I32, 2, true, &dev));
+  DeviceScope scope;
+  OD_CHECK(check_tensor(boxes, "boxes", F32, {kAny, kAny, 4}, 16, scope));
   const int64_t B = boxes->shape[0], K = boxes->shape[1];
-  if (boxes->shape[2] != 4 || scores->shape[0] != B || scores->shape[1] != K) OD_FAIL(OD_ERR_SHAPE, "boxes [B,K,4] / scores [B,K] mismatch");
-  if (keep_idx->shape[0] != B || keep_idx->shape[1] != max_out) OD_FAIL(OD_ERR_SHAPE, "keep_idx must be [B,max_out]");
-  if (num_valid) {
-    OD_CHECK(check_tensor(num_valid, "num_valid", I32, 1, true, &dev));
-    if (num_valid->shape[0] != B) OD_FAIL(OD_ERR_SHAPE, "num_valid must be [B]");
-  }
-  if (num_kept) {
-    OD_CHECK(check_tensor(num_kept, "num_kept", I32, 1, true, &dev));
-    if (num_kept->shape[0] != B) OD_FAIL(OD_ERR_SHAPE, "num_kept must be [B]");
-  }
-  if (reinterpret_cast<uintptr_t>(dptr<float>(boxes)) % 16) OD_FAIL(OD_ERR_LAYOUT, "boxes not 16-byte aligned");
+  OD_CHECK(check_tensor(scores, "scores", F32, {B, K}, 4, scope));
+  if (max_out < 0) OD_FAIL(OD_ERR_SHAPE, "keep_idx: max_out = %lld is negative", (long long)max_out);
+  OD_CHECK(check_tensor(keep_idx, "keep_idx", I32, {B, max_out}, 4, scope));
+  OD_CHECK(check_opt_tensor(num_valid, "num_valid", I32, {B}, 4, scope));
+  OD_CHECK(check_opt_tensor(num_kept, "num_kept", I32, {B}, 4, scope));
   if (B == 0 || max_out == 0) return OD_OK;
   if (!ws) OD_FAIL(OD_ERR_WORKSPACE, "NMS workspace is NULL");
   const int64_t n_pow2 = next_pow2(K > 0 ? K : 1);

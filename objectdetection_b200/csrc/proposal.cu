@@ -154,17 +154,6 @@ static size_t carve_proposal_ws(Workspace& w, int64_t B, int64_t A, int64_t K, i
   return w.off + 256;
 }
 
-static int check_opt(const DLTensor* t, const char* name, DType dt, int ndim, int* dev, std::initializer_list<int64_t> shape) {
-  if (!t) return OD_OK;
-  OD_CHECK(check_tensor(t, name, dt, ndim, true, dev));
-  int d = 0;
-  for (int64_t s : shape) {
-    if (t->shape[d] != s) OD_FAIL(OD_ERR_SHAPE, "%s: extent %d is %lld, expected %lld", name, d, (long long)t->shape[d], (long long)s);
-    ++d;
-  }
-  return OD_OK;
-}
-
 }  // namespace od
 
 using namespace od;
@@ -182,16 +171,13 @@ int od_gen_anchors(const od_anchor_spec* spec, int normalized, DLTensor* anchors
   DevAnchorSpec d;
   OD_CHECK(make_dev_anchor_spec(spec, &d));
   const int64_t A = d.offset[d.num_levels];
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
+  DeviceScope scope;
   if (normalized) {
-    OD_CHECK(check_tensor(anchors, "anchors", F32, 3, true, &dev));
-    if (anchors->shape[1] != A || anchors->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "anchors must be [B,%lld,4]", (long long)A);
+    OD_CHECK(check_tensor(anchors, "anchors", F32, {kAny, A, 4}, 16, scope));
     if (A == 0 || anchors->shape[0] == 0) return OD_OK;
     gen_anchors_norm_kernel<<<(unsigned)((A + 255) / 256), 256, 0, st>>>(d, A, anchors->shape[0], dptr<float4>(anchors));
   } else {
-    OD_CHECK(check_tensor(anchors, "anchors", F64, 2, true, &dev));
-    if (anchors->shape[0] != A || anchors->shape[1] != 4) OD_FAIL(OD_ERR_SHAPE, "anchors must be [%lld,4]", (long long)A);
+    OD_CHECK(check_tensor(anchors, "anchors", F64, {A, 4}, 8, scope));
     if (A == 0) return OD_OK;
     gen_anchors_pixel_kernel<<<(unsigned)((A + 255) / 256), 256, 0, st>>>(d, A, dptr<double>(anchors));
   }
@@ -200,14 +186,10 @@ int od_gen_anchors(const od_anchor_spec* spec, int normalized, DLTensor* anchors
 }
 
 int od_apply_box_deltas(const DLTensor* boxes, const DLTensor* deltas, DLTensor* out, void* stream) {
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(boxes, "boxes", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(deltas, "deltas", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(out, "out", F32, 3, true, &dev));
-  for (int i = 0; i < 3; ++i)
-    if (boxes->shape[i] != deltas->shape[i] || boxes->shape[i] != out->shape[i]) OD_FAIL(OD_ERR_SHAPE, "boxes/deltas/out shapes differ");
-  if (boxes->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "last extent must be 4");
+  DeviceScope scope;
+  OD_CHECK(check_tensor(boxes, "boxes", F32, {kAny, kAny, 4}, 16, scope));
+  OD_CHECK(check_tensor(deltas, "deltas", F32, {boxes->shape[0], boxes->shape[1], 4}, 16, scope));
+  OD_CHECK(check_tensor(out, "out", F32, {boxes->shape[0], boxes->shape[1], 4}, 16, scope));
   const int64_t total = boxes->shape[0] * boxes->shape[1];
   if (total == 0) return OD_OK;
   apply_box_deltas_kernel<<<(unsigned)((total + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
@@ -217,18 +199,12 @@ int od_apply_box_deltas(const DLTensor* boxes, const DLTensor* deltas, DLTensor*
 }
 
 int od_clip_boxes(const DLTensor* boxes, const DLTensor* window, DLTensor* out, void* stream) {
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(boxes, "boxes", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(window, "window", F32, -1, true, &dev));
-  OD_CHECK(check_tensor(out, "out", F32, 3, true, &dev));
-  for (int i = 0; i < 3; ++i)
-    if (boxes->shape[i] != out->shape[i]) OD_FAIL(OD_ERR_SHAPE, "boxes/out shapes differ");
-  if (boxes->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "last extent must be 4");
-  int per_image = 0;
-  if (window->ndim == 1 && window->shape[0] == 4) per_image = 0;
-  else if (window->ndim == 2 && window->shape[0] == boxes->shape[0] && window->shape[1] == 4) per_image = 1;
-  else OD_FAIL(OD_ERR_SHAPE, "window must be [4] or [B,4]");
+  DeviceScope scope;
+  OD_CHECK(check_tensor(boxes, "boxes", F32, {kAny, kAny, 4}, 16, scope));
+  const int per_image = window && window->ndim == 2;   // window [B,4], else [4]
+  if (per_image) OD_CHECK(check_tensor(window, "window", F32, {boxes->shape[0], 4}, 16, scope));
+  else OD_CHECK(check_tensor(window, "window", F32, {4}, 16, scope));
+  OD_CHECK(check_tensor(out, "out", F32, {boxes->shape[0], boxes->shape[1], 4}, 16, scope));
   const int64_t total = boxes->shape[0] * boxes->shape[1];
   if (total == 0) return OD_OK;
   clip_boxes_kernel<<<(unsigned)((total + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
@@ -238,18 +214,16 @@ int od_clip_boxes(const DLTensor* boxes, const DLTensor* window, DLTensor* out, 
 }
 
 int od_norm_boxes(const DLTensor* boxes, int32_t image_h, int32_t image_w, int32_t tf_float32, DLTensor* out, void* stream) {
-  int dev = -1;
-  DeviceScope dev_scope;
+  DeviceScope scope;
   if (!boxes) OD_FAIL(OD_ERR_NULL, "boxes is NULL");
   const bool is_i32 = boxes->dtype.code == kDLInt && boxes->dtype.bits == 32;
   const bool is_f64 = boxes->dtype.code == kDLFloat && boxes->dtype.bits == 64;
-  OD_CHECK(check_tensor(boxes, "boxes", is_i32 ? I32 : (is_f64 ? F64 : F32), -1, true, &dev));
-  OD_CHECK(check_tensor(out, "out", F32, boxes->ndim, true, &dev));
-  if (boxes->ndim < 1 || boxes->shape[boxes->ndim - 1] != 4) OD_FAIL(OD_ERR_SHAPE, "boxes must be [...,4]");
-  for (int i = 0; i < boxes->ndim; ++i)
-    if (boxes->shape[i] != out->shape[i]) OD_FAIL(OD_ERR_SHAPE, "boxes/out shapes differ");
+  OD_CHECK(check_tensor(boxes, "boxes", is_i32 ? I32 : (is_f64 ? F64 : F32), nullptr, -1, is_f64 ? 8 : 4, scope));
+  if (boxes->ndim < 1) OD_FAIL(OD_ERR_SHAPE, "boxes must be [...,4]");
+  if (boxes->shape[boxes->ndim - 1] != 4)
+    OD_FAIL(OD_ERR_SHAPE, "boxes: extent %d is %lld, expected 4", boxes->ndim - 1, (long long)boxes->shape[boxes->ndim - 1]);
+  OD_CHECK(check_tensor(out, "out", F32, boxes->shape, boxes->ndim, 16, scope));
   if (tf_float32 && !(!is_i32 && !is_f64)) OD_FAIL(OD_ERR_DTYPE, "norm_boxes_tf takes float32 boxes");
-  if (reinterpret_cast<uintptr_t>(dptr<float>(out)) % 16) OD_FAIL(OD_ERR_LAYOUT, "out not 16-byte aligned");
   const int64_t n = numel(boxes) / 4;
   if (n == 0) return OD_OK;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -273,41 +247,43 @@ size_t od_proposal_workspace_bytes(int64_t batch, int64_t num_anchors, const od_
 
 namespace od {
 // Shared body of od_proposal_forward / od_proposal_forward_levels. `scores` addresses the fg score of anchor i of image b at
-// scores[b * score_sb + i * score_sa]; the deltas come from `rpn_bbox4` ([B,A,4]) or, when it is NULL, from `lv`.
-// `p` is the carved workspace. Shapes B, A are those of the caller's (virtual) [B,A,.] tensors.
-static int proposal_core(const float* scores_src, int64_t score_sb, int64_t score_sa, const float4* rpn_bbox4, const LevelTable& lv,
-                         int64_t B, int64_t A, const DLTensor* anchors, const od_anchor_spec* spec,
+// scores[b * score_sb + i * score_sa]; with `logits` (the per-level class logits), it is a workspace row that is first
+// filled from them. The deltas come from `rpn_bbox4` ([B,A,4]) or, when it is NULL, from `lv`. `p` is the carved
+// workspace. Shapes B, A are those of the caller's (virtual) [B,A,.] tensors.
+static int proposal_core(float* scores_src, int64_t score_sb, int64_t score_sa, const LevelTable* logits, const float4* rpn_bbox4,
+                         const LevelTable& lv, int64_t B, int64_t A, const DLTensor* anchors, const od_anchor_spec* spec,
                          const od_proposal_params* params, DLTensor* proposals, const od_proposal_debug* debug, ProposalWs& p,
-                         int dev, cudaStream_t st) {
+                         DeviceScope& scope, cudaStream_t st) {
   const int64_t K = params->pre_nms_limit < A ? params->pre_nms_limit : A;
   const int64_t N = params->post_nms_count;
-  if (proposals->shape[0] != B || proposals->shape[1] != N || proposals->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "proposals must be [B,%lld,4]", (long long)N);
+  OD_CHECK(check_tensor(proposals, "proposals", F32, {B, N, 4}, 16, scope));
   DevAnchorSpec dspec;
   memset(&dspec, 0, sizeof(dspec));
   int use_spec = 0;
   if (anchors) {
-    OD_CHECK(check_tensor(anchors, "anchors", F32, 3, true, &dev));
-    if (anchors->shape[0] != B || anchors->shape[1] != A || anchors->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "anchors must be [B,A,4]");
-    if (reinterpret_cast<uintptr_t>(dptr<float>(anchors)) % 16) OD_FAIL(OD_ERR_LAYOUT, "anchors not 16-byte aligned");
+    OD_CHECK(check_tensor(anchors, "anchors", F32, {B, A, 4}, 16, scope));
   } else {
     if (!spec) OD_FAIL(OD_ERR_NULL, "either anchors or an anchor spec is required");
     OD_CHECK(make_dev_anchor_spec(spec, &dspec));
     if (dspec.offset[dspec.num_levels] != A) OD_FAIL(OD_ERR_SHAPE, "anchor spec yields %lld anchors, inputs have %lld", (long long)dspec.offset[dspec.num_levels], (long long)A);
     use_spec = 1;
   }
-  if (reinterpret_cast<uintptr_t>(dptr<float>(proposals)) % 16) OD_FAIL(OD_ERR_LAYOUT, "proposals not 16-byte aligned");
   od_proposal_debug dbg;
   memset(&dbg, 0, sizeof(dbg));
   if (debug) dbg = *debug;
-  OD_CHECK(check_opt(dbg.ix, "debug.ix", I32, 2, &dev, {B, K}));
-  OD_CHECK(check_opt(dbg.scores, "debug.scores", F32, 2, &dev, {B, K}));
-  OD_CHECK(check_opt(dbg.bbox_delta, "debug.bbox_delta", F32, 3, &dev, {B, K, 4}));
-  OD_CHECK(check_opt(dbg.anchors, "debug.anchors", F32, 3, &dev, {B, K, 4}));
-  OD_CHECK(check_opt(dbg.anchor_delta, "debug.anchor_delta", F32, 3, &dev, {B, K, 4}));
-  OD_CHECK(check_opt(dbg.anchor_delta_clipped, "debug.anchor_delta_clipped", F32, 3, &dev, {B, K, 4}));
-  OD_CHECK(check_opt(dbg.keep_idx, "debug.keep_idx", I32, 2, &dev, {B, N}));
-  OD_CHECK(check_opt(dbg.num_kept, "debug.num_kept", I32, 1, &dev, {B}));
+  OD_CHECK(check_opt_tensor(dbg.ix, "debug.ix", I32, {B, K}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.scores, "debug.scores", F32, {B, K}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.bbox_delta, "debug.bbox_delta", F32, {B, K, 4}, 16, scope));
+  OD_CHECK(check_opt_tensor(dbg.anchors, "debug.anchors", F32, {B, K, 4}, 16, scope));
+  OD_CHECK(check_opt_tensor(dbg.anchor_delta, "debug.anchor_delta", F32, {B, K, 4}, 16, scope));
+  OD_CHECK(check_opt_tensor(dbg.anchor_delta_clipped, "debug.anchor_delta_clipped", F32, {B, K, 4}, 16, scope));
+  OD_CHECK(check_opt_tensor(dbg.keep_idx, "debug.keep_idx", I32, {B, N}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.num_kept, "debug.num_kept", I32, {B}, 4, scope));
   if (B == 0 || N == 0) return OD_OK;
+  if (logits && B * A > 0) {
+    rpn_level_scores_kernel<<<(unsigned)((B * A + 255) / 256), 256, 0, st>>>(*logits, (int)A, B * A, scores_src);
+    OD_LAUNCH_CHECK("rpn_level_scores_kernel");
+  }
   int32_t* ix = dbg.ix ? dptr<int32_t>(dbg.ix) : p.ix;
   float* scores = dbg.scores ? dptr<float>(dbg.scores) : nullptr;  // only materialised on request
   int32_t* keep_pos = dbg.keep_idx ? dptr<int32_t>(dbg.keep_idx) : p.keep_pos;
@@ -350,16 +326,11 @@ int od_proposal_forward(const DLTensor* rpn_class_probs, const DLTensor* rpn_bbo
                         const od_proposal_debug* debug, void* ws, size_t ws_bytes, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (!params) OD_FAIL(OD_ERR_NULL, "params is NULL");
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(rpn_class_probs, "rpn_class_probs", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(rpn_bbox, "rpn_bbox", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(proposals, "proposals", F32, 3, true, &dev));
+  DeviceScope scope;
+  OD_CHECK(check_tensor(rpn_class_probs, "rpn_class_probs", F32, {kAny, kAny, 2}, 4, scope));
   const int64_t B = rpn_class_probs->shape[0], A = rpn_class_probs->shape[1];
-  if (rpn_class_probs->shape[2] != 2) OD_FAIL(OD_ERR_SHAPE, "rpn_class_probs must be [B,A,2]");
-  if (rpn_bbox->shape[0] != B || rpn_bbox->shape[1] != A || rpn_bbox->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "rpn_bbox must be [B,A,4]");
+  OD_CHECK(check_tensor(rpn_bbox, "rpn_bbox", F32, {B, A, 4}, 16, scope));
   if (params->pre_nms_limit < 0 || params->post_nms_count < 0) OD_FAIL(OD_ERR_PARAM, "negative counts");
-  if (reinterpret_cast<uintptr_t>(dptr<float>(rpn_bbox)) % 16) OD_FAIL(OD_ERR_LAYOUT, "rpn_bbox not 16-byte aligned");
   const int64_t K = params->pre_nms_limit < A ? params->pre_nms_limit : A;
   const int64_t N = params->post_nms_count;
   ProposalWs p;
@@ -373,8 +344,8 @@ int od_proposal_forward(const DLTensor* rpn_class_probs, const DLTensor* rpn_bbo
   LevelTable lv;
   memset(&lv, 0, sizeof(lv));
   // scores = probs[:,:,1]  (:153)
-  return proposal_core(dptr<float>(rpn_class_probs) + 1, 2 * A, 2, dptr<float4>(rpn_bbox), lv, B, A, anchors, spec, params,
-                       proposals, debug, p, dev, st);
+  return proposal_core(dptr<float>(rpn_class_probs) + 1, 2 * A, 2, nullptr, dptr<float4>(rpn_bbox), lv, B, A, anchors, spec,
+                       params, proposals, debug, p, scope, st);
 }
 
 size_t od_proposal_levels_workspace_bytes(int64_t batch, int64_t num_anchors, const od_proposal_params* p) {
@@ -392,25 +363,19 @@ int od_proposal_forward_levels(const DLTensor* const* class_logits, const DLTens
   if (!params || !class_logits || !bbox) OD_FAIL(OD_ERR_NULL, "params / class_logits / bbox is NULL");
   if (num_levels < 1 || num_levels > OD_MAX_LEVELS) OD_FAIL(OD_ERR_PARAM, "num_levels %d out of range", num_levels);
   if (params->pre_nms_limit < 0 || params->post_nms_count < 0) OD_FAIL(OD_ERR_PARAM, "negative counts");
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(proposals, "proposals", F32, 3, true, &dev));
+  DeviceScope scope;
   LevelTable lc, lb;
   memset(&lc, 0, sizeof(lc));
   memset(&lb, 0, sizeof(lb));
   lc.num_levels = lb.num_levels = num_levels;
-  int64_t B = -1, A = 0;
+  int64_t B = kAny, A = 0;   // B: that of the first level
   for (int l = 0; l < num_levels; ++l) {
-    OD_CHECK(check_tensor(class_logits[l], "class_logits[l]", F32, 4, true, &dev));
-    OD_CHECK(check_tensor(bbox[l], "bbox[l]", F32, 4, true, &dev));
     const DLTensor* c = class_logits[l];
     const DLTensor* d = bbox[l];
-    if (B < 0) B = c->shape[0];
-    if (c->shape[0] != B || d->shape[0] != B || c->shape[1] != d->shape[1] || c->shape[2] != d->shape[2] || c->shape[3] % 2 ||
-        d->shape[3] != 2 * c->shape[3])
-      OD_FAIL(OD_ERR_SHAPE, "level %d: class_logits must be [B,H,W,2a] and bbox [B,H,W,4a] with the same B, H, W, a", l);
-    if (reinterpret_cast<uintptr_t>(dptr<float>(d)) % 16 || reinterpret_cast<uintptr_t>(dptr<float>(c)) % 8)
-      OD_FAIL(OD_ERR_LAYOUT, "level %d: class_logits / bbox not 8 / 16-byte aligned", l);
+    OD_CHECK(check_tensor(c, "class_logits[l]", F32, {B, kAny, kAny, kAny}, 8, scope));
+    B = c->shape[0];
+    if (c->shape[3] % 2) OD_FAIL(OD_ERR_SHAPE, "class_logits[l]: extent 3 is %lld, expected an even value (level %d)", (long long)c->shape[3], l);
+    OD_CHECK(check_tensor(d, "bbox[l]", F32, {B, c->shape[1], c->shape[2], 2 * c->shape[3]}, 16, scope));
     const int64_t n_l = c->shape[1] * c->shape[2] * (c->shape[3] / 2);
     lc.base[l] = dptr<float>(c);
     lb.base[l] = dptr<float>(d);
@@ -430,13 +395,8 @@ int od_proposal_forward_levels(const DLTensor* const* class_logits, const DLTens
     scores = w.take<float>((size_t)(B * A));
     carve_proposal_ws(w, B, A, K, N, &p);
     if (!w.ok()) OD_FAIL(OD_ERR_WORKSPACE, "workspace %zu < %zu bytes", ws_bytes, w.off);
-    const int64_t total = B * A;
-    if (total > 0) {
-      rpn_level_scores_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(lc, (int)A, total, scores);
-      OD_LAUNCH_CHECK("rpn_level_scores_kernel");
-    }
   }
-  return proposal_core(scores, A, 1, nullptr, lb, B, A, anchors, spec, params, proposals, debug, p, dev, st);
+  return proposal_core(scores, A, 1, &lc, nullptr, lb, B, A, anchors, spec, params, proposals, debug, p, scope, st);
 }
 
 }  // extern "C"

@@ -989,17 +989,13 @@ size_t od_pyramid_roi_align_workspace_bytes_n(int64_t n_rois) {
 int od_roi_processing_order(const DLTensor* rois, int32_t image_h, int32_t image_w, int32_t min_level, int32_t num_levels,
                             DLTensor* order, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int dev = -1;
-  DeviceScope dev_scope;
-  OD_CHECK(check_tensor(rois, "rois", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(order, "order", I32, 1, true, &dev));
-  if (rois->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "rois must be [B,N,4]");
-  if (num_levels < 1 || num_levels > OD_MAX_LEVELS) OD_FAIL(OD_ERR_PARAM, "num_levels %d not in [1,%d]", num_levels, OD_MAX_LEVELS);
+  DeviceScope scope;
+  OD_CHECK(check_tensor(rois, "rois", F32, {kAny, kAny, 4}, 16, scope));
   const int64_t B = rois->shape[0], N = rois->shape[1];
-  if (order->shape[0] != B * N) OD_FAIL(OD_ERR_SHAPE, "order must be [B*N]");
+  OD_CHECK(check_tensor(order, "order", I32, {B * N}, 4, scope));
+  if (num_levels < 1 || num_levels > OD_MAX_LEVELS) OD_FAIL(OD_ERR_PARAM, "num_levels %d not in [1,%d]", num_levels, OD_MAX_LEVELS);
   if (B * N == 0) return OD_OK;
   if (B * N > 0x7FFFFFFFll || B > 65535) OD_FAIL(OD_ERR_PARAM, "too many ROIs");
-  if (reinterpret_cast<uintptr_t>(dptr<float>(rois)) % 16) OD_FAIL(OD_ERR_LAYOUT, "rois not 16-byte aligned");
   if (N > kOrderThreads * kOrderPerThread) OD_FAIL(OD_ERR_PARAM, "at most %d ROIs per image", kOrderThreads * kOrderPerThread);
   RoiSource src;
   memset(&src, 0, sizeof(src));
@@ -1029,39 +1025,24 @@ int od_pyramid_roi_align_forward_ordered(const DLTensor* const* fmaps, int32_t n
   if (!fmaps) OD_FAIL(OD_ERR_NULL, "fmaps is NULL");
   if (num_levels < 1 || num_levels > OD_MAX_LEVELS) OD_FAIL(OD_ERR_PARAM, "num_levels %d not in [1,%d]", num_levels, OD_MAX_LEVELS);
   if (pool_h < 1 || pool_w < 1) OD_FAIL(OD_ERR_PARAM, "pool shape %dx%d unsupported", pool_h, pool_w);
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(rois, "rois", F32, 3, true, &dev));
-  if (rois->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "rois must be [B,N,4]");
+  DeviceScope scope;
+  OD_CHECK(check_tensor(rois, "rois", F32, {kAny, kAny, 4}, 16, scope));
   const int64_t B = rois->shape[0], N = rois->shape[1];
   LevelTable lt;
-  int64_t D = -1;
+  int64_t D = kAny;   // that of the first level
   for (int l = 0; l < num_levels; ++l) {
-    OD_CHECK(check_tensor(fmaps[l], "fmaps[l]", F32, 4, true, &dev));
-    if (fmaps[l]->shape[0] != B) OD_FAIL(OD_ERR_SHAPE, "fmaps[%d] batch %lld != %lld", l, (long long)fmaps[l]->shape[0], (long long)B);
-    if (D < 0) D = fmaps[l]->shape[3];
-    if (fmaps[l]->shape[3] != D) OD_FAIL(OD_ERR_SHAPE, "fmaps[%d] depth mismatch", l);
+    OD_CHECK(check_tensor(fmaps[l], "fmaps[l]", F32, {B, kAny, kAny, D}, 16, scope));
+    D = fmaps[l]->shape[3];
     lt.ptr[l] = dptr<float>(fmaps[l]);
     lt.H[l] = (int32_t)fmaps[l]->shape[1];
     lt.W[l] = (int32_t)fmaps[l]->shape[2];
-    if (reinterpret_cast<uintptr_t>(lt.ptr[l]) % 16) OD_FAIL(OD_ERR_LAYOUT, "fmaps[%d] not 16-byte aligned", l);
   }
   if (D % 4) OD_FAIL(OD_ERR_SHAPE, "depth %lld must be a multiple of 4", (long long)D);
-  OD_CHECK(check_tensor(pooled, "pooled", F32, -1, true, &dev));
-  const int64_t want = B * N * pool_h * pool_w * D;
-  const bool shape5 = pooled->ndim == 5 && pooled->shape[0] == 1 && pooled->shape[1] == B * N && pooled->shape[2] == pool_h &&
-                      pooled->shape[3] == pool_w && pooled->shape[4] == D;
-  const bool shape4 = pooled->ndim == 4 && pooled->shape[0] == B * N && pooled->shape[1] == pool_h &&
-                      pooled->shape[2] == pool_w && pooled->shape[3] == D;
-  if (!(shape5 || shape4) || numel(pooled) != want) OD_FAIL(OD_ERR_SHAPE, "pooled must be [1,B*N,ph,pw,D] or [B*N,ph,pw,D]");
-  if (reinterpret_cast<uintptr_t>(dptr<float>(pooled)) % 16) OD_FAIL(OD_ERR_LAYOUT, "pooled not 16-byte aligned");
-  if (roi_level) {
-    OD_CHECK(check_tensor(roi_level, "roi_level", I32, 2, true, &dev));
-    if (roi_level->shape[0] != B || roi_level->shape[1] != N) OD_FAIL(OD_ERR_SHAPE, "roi_level must be [B,N]");
-  }
+  if (pooled && pooled->ndim == 5) OD_CHECK(check_tensor(pooled, "pooled", F32, {1, B * N, pool_h, pool_w, D}, 16, scope));
+  else OD_CHECK(check_tensor(pooled, "pooled", F32, {B * N, pool_h, pool_w, D}, 16, scope));
+  OD_CHECK(check_opt_tensor(roi_level, "roi_level", I32, {B, N}, 4, scope));
   const int64_t total = B * N;
   if (total == 0) return OD_OK;
-  if (reinterpret_cast<uintptr_t>(dptr<float>(rois)) % 16) OD_FAIL(OD_ERR_LAYOUT, "rois not 16-byte aligned");
   RoiSource src;
   memset(&src, 0, sizeof(src));
   src.mode = 0;
@@ -1078,10 +1059,7 @@ int od_pyramid_roi_align_forward_ordered(const DLTensor* const* fmaps, int32_t n
   // workspace: [0,256) the ticket counters (stay zeroed), [256, 256 + 4*B*N) the ROI processing order (scratch)
   int32_t* order_buf = (ws && ws_bytes >= od_pyramid_roi_align_workspace_bytes_n(total))
                            ? reinterpret_cast<int32_t*>(static_cast<char*>(ws) + 256) : nullptr;
-  if (order) {
-    OD_CHECK(check_tensor(order, "order", I32, 1, true, &dev));
-    if (order->shape[0] != total) OD_FAIL(OD_ERR_SHAPE, "order must be [B*N]");
-  }
+  OD_CHECK(check_opt_tensor(order, "order", I32, {total}, 4, scope));
   return launch_crop_bins(src, total, pool_h, pool_w, (int32_t)D, 0.0f, dptr<float>(pooled), dptr<int32_t>(roi_level), st,
                           static_cast<unsigned int*>(ws), order_buf, dptr<int32_t>(order));
 }
@@ -1097,21 +1075,14 @@ int od_pyramid_roi_align_forward(const DLTensor* const* fmaps, int32_t num_level
 int od_crop_and_resize(const DLTensor* image, const DLTensor* boxes, const DLTensor* box_ind, int32_t crop_h,
                        int32_t crop_w, float extrapolation_value, DLTensor* out, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(image, "image", F32, 4, true, &dev));
-  OD_CHECK(check_tensor(boxes, "boxes", F32, 2, true, &dev));
-  OD_CHECK(check_tensor(box_ind, "box_ind", I32, 1, true, &dev));
-  OD_CHECK(check_tensor(out, "out", F32, 4, true, &dev));
-  if (crop_h < 1 || crop_w < 1) OD_FAIL(OD_ERR_PARAM, "crop size %dx%d unsupported", crop_h, crop_w);
+  DeviceScope scope;
+  OD_CHECK(check_tensor(image, "image", F32, {kAny, kAny, kAny, kAny}, 16, scope));
+  OD_CHECK(check_tensor(boxes, "boxes", F32, {kAny, 4}, 16, scope));
   const int64_t n = boxes->shape[0], D = image->shape[3];
-  if (boxes->shape[1] != 4 || box_ind->shape[0] != n) OD_FAIL(OD_ERR_SHAPE, "boxes [n,4] / box_ind [n] mismatch");
-  if (out->shape[0] != n || out->shape[1] != crop_h || out->shape[2] != crop_w || out->shape[3] != D)
-    OD_FAIL(OD_ERR_SHAPE, "out must be [n,crop_h,crop_w,D]");
+  OD_CHECK(check_tensor(box_ind, "box_ind", I32, {n}, 4, scope));
+  if (crop_h < 1 || crop_w < 1) OD_FAIL(OD_ERR_PARAM, "crop size %dx%d unsupported", crop_h, crop_w);
+  OD_CHECK(check_tensor(out, "out", F32, {n, crop_h, crop_w, D}, 16, scope));
   if (D % 4) OD_FAIL(OD_ERR_SHAPE, "depth %lld must be a multiple of 4", (long long)D);
-  if (reinterpret_cast<uintptr_t>(dptr<float>(image)) % 16 || reinterpret_cast<uintptr_t>(dptr<float>(out)) % 16 ||
-      reinterpret_cast<uintptr_t>(dptr<float>(boxes)) % 16)
-    OD_FAIL(OD_ERR_LAYOUT, "image/boxes/out must be 16-byte aligned");
   if (n == 0) return OD_OK;
   RoiSource src;
   memset(&src, 0, sizeof(src));
@@ -1128,18 +1099,12 @@ int od_crop_and_resize(const DLTensor* image, const DLTensor* boxes, const DLTen
 int od_roi_pool_forward(const DLTensor* feature_map, const DLTensor* proposals, float image_h, float image_w,
                         DLTensor* out, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(feature_map, "feature_map", F32, 4, true, &dev));
-  OD_CHECK(check_tensor(proposals, "proposals", F32, 2, true, &dev));
-  OD_CHECK(check_tensor(out, "out", F32, 4, true, &dev));
+  DeviceScope scope;
+  OD_CHECK(check_tensor(feature_map, "feature_map", F32, {kAny, kAny, kAny, kAny}, 16, scope));
+  OD_CHECK(check_tensor(proposals, "proposals", F32, {kAny, 5}, 4, scope));
   const int64_t n = proposals->shape[0], D = feature_map->shape[3];
-  if (proposals->shape[1] != 5) OD_FAIL(OD_ERR_SHAPE, "proposals must be [n,5]");
-  if (out->shape[0] != n || out->shape[1] != 7 || out->shape[2] != 7 || out->shape[3] != D)
-    OD_FAIL(OD_ERR_SHAPE, "out must be [n,7,7,D]");
+  OD_CHECK(check_tensor(out, "out", F32, {n, 7, 7, D}, 16, scope));
   if (D % 4) OD_FAIL(OD_ERR_SHAPE, "depth %lld must be a multiple of 4", (long long)D);
-  if (reinterpret_cast<uintptr_t>(dptr<float>(feature_map)) % 16 || reinterpret_cast<uintptr_t>(dptr<float>(out)) % 16)
-    OD_FAIL(OD_ERR_LAYOUT, "feature_map/out must be 16-byte aligned");
   if (n == 0) return OD_OK;
   if ((int64_t)feature_map->shape[1] * feature_map->shape[2] * (D / 4) > 0xFFFFFFFFll)
     OD_FAIL(OD_ERR_PARAM, "feature map exceeds 2^32 16-byte units per image");

@@ -550,27 +550,17 @@ int od_rpn_target_forward(const DLTensor* anchors, const DLTensor* gt_boxes, con
                           DLTensor* counts, void* ws, size_t ws_bytes, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (!params) OD_FAIL(OD_ERR_NULL, "params is NULL");
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(anchors, "anchors", F64, 2, true, &dev));
-  OD_CHECK(check_tensor(gt_boxes, "gt_boxes", F64, 3, true, &dev));
-  OD_CHECK(check_tensor(gt_count, "gt_count", I32, 1, true, &dev));
-  OD_CHECK(check_tensor(perm_pos, "perm_pos", I32, 2, true, &dev));
-  OD_CHECK(check_tensor(perm_neg, "perm_neg", I32, 2, true, &dev));
-  OD_CHECK(check_tensor(rpn_target_class, "rpn_target_class", I32, 2, true, &dev));
-  OD_CHECK(check_tensor(rpn_target_bbox, "rpn_target_bbox", F64, 3, true, &dev));
-  OD_CHECK(check_tensor(positive_anchors, "positive_anchors", F64, 3, true, &dev));
-  OD_CHECK(check_tensor(counts, "counts", I32, 2, true, &dev));
+  DeviceScope scope;
+  OD_CHECK(check_tensor(anchors, "anchors", F64, {kAny, 4}, 8, scope));
+  OD_CHECK(check_tensor(gt_boxes, "gt_boxes", F64, {kAny, kAny, 4}, 8, scope));
   const int64_t A = anchors->shape[0], B = gt_boxes->shape[0], G = gt_boxes->shape[1], T = params->max_rpn_targets;
-  if (anchors->shape[1] != 4 || gt_boxes->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "anchors [A,4] / gt_boxes [B,G,4] expected");
-  if (gt_count->shape[0] != B) OD_FAIL(OD_ERR_SHAPE, "gt_count must be [B]");
-  if (perm_pos->shape[0] != B || perm_pos->shape[1] != A || perm_neg->shape[0] != B || perm_neg->shape[1] != A)
-    OD_FAIL(OD_ERR_SHAPE, "perm_pos / perm_neg must be [B,A]");
-  if (rpn_target_class->shape[0] != B || rpn_target_class->shape[1] != A) OD_FAIL(OD_ERR_SHAPE, "rpn_target_class must be [B,A]");
-  if (T < 0 || rpn_target_bbox->shape[0] != B || rpn_target_bbox->shape[1] != T || rpn_target_bbox->shape[2] != 4 ||
-      positive_anchors->shape[0] != B || positive_anchors->shape[1] != T || positive_anchors->shape[2] != 4)
-    OD_FAIL(OD_ERR_SHAPE, "rpn_target_bbox / positive_anchors must be [B,max_rpn_targets,4]");
-  if (counts->shape[0] != B || counts->shape[1] != 4) OD_FAIL(OD_ERR_SHAPE, "counts must be [B,4]");
+  OD_CHECK(check_tensor(gt_count, "gt_count", I32, {B}, 4, scope));
+  OD_CHECK(check_tensor(perm_pos, "perm_pos", I32, {B, A}, 4, scope));
+  OD_CHECK(check_tensor(perm_neg, "perm_neg", I32, {B, A}, 4, scope));
+  OD_CHECK(check_tensor(rpn_target_class, "rpn_target_class", I32, {B, A}, 4, scope));
+  OD_CHECK(check_tensor(rpn_target_bbox, "rpn_target_bbox", F64, {B, T, 4}, 8, scope));
+  OD_CHECK(check_tensor(positive_anchors, "positive_anchors", F64, {B, T, 4}, 8, scope));
+  OD_CHECK(check_tensor(counts, "counts", I32, {B, 4}, 4, scope));
   if (A >= (1ll << 30) || G > 4096 || B > 65535) OD_FAIL(OD_ERR_PARAM, "supports A < 2^30, G <= 4096, B <= 65535");
   if (B == 0 || A == 0) return OD_OK;
   if (!ws) OD_FAIL(OD_ERR_WORKSPACE, "workspace is NULL");

@@ -318,17 +318,6 @@ mask_target_kernel(const float4* __restrict__ rois, const float4* __restrict__ g
   }
 }
 
-static int check_opt_nd(const DLTensor* t, const char* name, DType dt, int* dev, std::initializer_list<int64_t> shape) {
-  if (!t) return OD_OK;
-  OD_CHECK(check_tensor(t, name, dt, (int)shape.size(), true, dev));
-  int d = 0;
-  for (int64_t s : shape) {
-    if (t->shape[d] != s) OD_FAIL(OD_ERR_SHAPE, "%s: extent %d is %lld, expected %lld", name, d, (long long)t->shape[d], (long long)s);
-    ++d;
-  }
-  return OD_OK;
-}
-
 }  // namespace od
 
 using namespace od;
@@ -351,42 +340,26 @@ int od_detection_target_forward(const DLTensor* proposals, const DLTensor* gt_cl
                                 void* ws, size_t ws_bytes, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (!params) OD_FAIL(OD_ERR_NULL, "params is NULL");
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(proposals, "proposals", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(gt_class_ids, "gt_class_ids", I32, 2, true, &dev));
-  OD_CHECK(check_tensor(gt_boxes, "gt_boxes", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(perm_pos, "perm_pos", I32, 2, true, &dev));
-  OD_CHECK(check_tensor(perm_neg, "perm_neg", I32, 2, true, &dev));
-  OD_CHECK(check_tensor(rois, "rois", F32, 3, true, &dev));
-  OD_CHECK(check_tensor(roi_gt_class_ids, "roi_gt_class_ids", I32, 2, true, &dev));
-  OD_CHECK(check_tensor(roi_gt_box_deltas, "roi_gt_box_deltas", F32, 3, true, &dev));
-  const int64_t B = proposals->shape[0], N = proposals->shape[1], G = gt_class_ids->shape[1], R = params->rois_per_image;
-  if (proposals->shape[2] != 4) OD_FAIL(OD_ERR_SHAPE, "proposals must be [B,N,4]");
-  if (gt_class_ids->shape[0] != B || gt_boxes->shape[0] != B || gt_boxes->shape[1] != G || gt_boxes->shape[2] != 4)
-    OD_FAIL(OD_ERR_SHAPE, "gt_class_ids [B,G] / gt_boxes [B,G,4] mismatch");
-  if (perm_pos->shape[0] != B || perm_pos->shape[1] != N || perm_neg->shape[0] != B || perm_neg->shape[1] != N)
-    OD_FAIL(OD_ERR_SHAPE, "perm_pos / perm_neg must be [B,N]");
-  if (R < 0 || rois->shape[0] != B || rois->shape[1] != R || rois->shape[2] != 4 || roi_gt_class_ids->shape[0] != B ||
-      roi_gt_class_ids->shape[1] != R || roi_gt_box_deltas->shape[0] != B || roi_gt_box_deltas->shape[1] != R ||
-      roi_gt_box_deltas->shape[2] != 4)
-    OD_FAIL(OD_ERR_SHAPE, "outputs must be rois [B,R,4], roi_gt_class_ids [B,R], roi_gt_box_deltas [B,R,4]");
+  DeviceScope scope;
+  OD_CHECK(check_tensor(proposals, "proposals", F32, {kAny, kAny, 4}, 16, scope));
+  const int64_t B = proposals->shape[0], N = proposals->shape[1], R = params->rois_per_image;
+  OD_CHECK(check_tensor(gt_class_ids, "gt_class_ids", I32, {B, kAny}, 4, scope));
+  const int64_t G = gt_class_ids->shape[1];
+  OD_CHECK(check_tensor(gt_boxes, "gt_boxes", F32, {B, G, 4}, 16, scope));
+  OD_CHECK(check_tensor(perm_pos, "perm_pos", I32, {B, N}, 4, scope));
+  OD_CHECK(check_tensor(perm_neg, "perm_neg", I32, {B, N}, 4, scope));
+  OD_CHECK(check_tensor(rois, "rois", F32, {B, R, 4}, 16, scope));
+  OD_CHECK(check_tensor(roi_gt_class_ids, "roi_gt_class_ids", I32, {B, R}, 4, scope));
+  OD_CHECK(check_tensor(roi_gt_box_deltas, "roi_gt_box_deltas", F32, {B, R, 4}, 16, scope));
   if ((gt_masks == nullptr) != (mask_targets == nullptr)) OD_FAIL(OD_ERR_NULL, "gt_masks and mask_targets go together");
   int64_t Mh = 0, Mw = 0;
   if (gt_masks) {
-    OD_CHECK(check_tensor(gt_masks, "gt_masks", F32, 4, true, &dev));
-    OD_CHECK(check_tensor(mask_targets, "mask_targets", F32, 4, true, &dev));
-    if (params->mask_layout_hwg) {
-      Mh = gt_masks->shape[1]; Mw = gt_masks->shape[2];
-      if (gt_masks->shape[0] != B || gt_masks->shape[3] != G) OD_FAIL(OD_ERR_SHAPE, "gt_masks must be [B,Mh,Mw,G]");
-    } else {
-      Mh = gt_masks->shape[2]; Mw = gt_masks->shape[3];
-      if (gt_masks->shape[0] != B || gt_masks->shape[1] != G) OD_FAIL(OD_ERR_SHAPE, "gt_masks must be [B,G,Mh,Mw]");
-    }
+    if (params->mask_layout_hwg) OD_CHECK(check_tensor(gt_masks, "gt_masks", F32, {B, kAny, kAny, G}, 4, scope));
+    else OD_CHECK(check_tensor(gt_masks, "gt_masks", F32, {B, G, kAny, kAny}, 4, scope));
+    Mh = gt_masks->shape[params->mask_layout_hwg ? 1 : 2];
+    Mw = gt_masks->shape[params->mask_layout_hwg ? 2 : 3];
     if (params->mask_h < 1 || params->mask_w < 1 || Mh < 1 || Mw < 1) OD_FAIL(OD_ERR_PARAM, "mask sizes must be positive");
-    if (mask_targets->shape[0] != B || mask_targets->shape[1] != R || mask_targets->shape[2] != params->mask_h ||
-        mask_targets->shape[3] != params->mask_w)
-      OD_FAIL(OD_ERR_SHAPE, "mask_targets must be [B,R,mask_h,mask_w]");
+    OD_CHECK(check_tensor(mask_targets, "mask_targets", F32, {B, R, params->mask_h, params->mask_w}, 4, scope));
     if (R > 4096) OD_FAIL(OD_ERR_PARAM, "mask targets support rois_per_image <= 4096");
   }
   if (G > 8192) OD_FAIL(OD_ERR_PARAM, "at most 8192 GT boxes per image");
@@ -398,19 +371,17 @@ int od_detection_target_forward(const DLTensor* proposals, const DLTensor* gt_cl
     for (int p = 0; p <= num_pos_inst; ++p)
       if ((int)(inv * (float)p) > R) OD_FAIL(OD_ERR_PARAM, "rois_per_image=%lld cannot hold pos+neg samples", (long long)R);
   }
-  for (const DLTensor* t : {proposals, (const DLTensor*)gt_boxes, (const DLTensor*)rois, (const DLTensor*)roi_gt_box_deltas})
-    if (reinterpret_cast<uintptr_t>(dptr<float>(t)) % 16) OD_FAIL(OD_ERR_LAYOUT, "box tensors must be 16-byte aligned");
   od_target_debug dbg;
   memset(&dbg, 0, sizeof(dbg));
   if (debug) dbg = *debug;
-  OD_CHECK(check_opt_nd(dbg.iou, "debug.iou", F32, &dev, {B, N, G}));
-  OD_CHECK(check_opt_nd(dbg.roi_iou_max, "debug.roi_iou_max", F32, &dev, {B, N}));
-  OD_CHECK(check_opt_nd(dbg.pos_indices, "debug.pos_indices", I32, &dev, {B, N}));
-  OD_CHECK(check_opt_nd(dbg.neg_indices, "debug.neg_indices", I32, &dev, {B, N}));
-  OD_CHECK(check_opt_nd(dbg.counts, "debug.counts", I32, &dev, {B, 6}));
-  OD_CHECK(check_opt_nd(dbg.sampled_pos, "debug.sampled_pos", I32, &dev, {B, R}));
-  OD_CHECK(check_opt_nd(dbg.sampled_neg, "debug.sampled_neg", I32, &dev, {B, R}));
-  OD_CHECK(check_opt_nd(dbg.gt_assignment, "debug.gt_assignment", I32, &dev, {B, R}));
+  OD_CHECK(check_opt_tensor(dbg.iou, "debug.iou", F32, {B, N, G}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.roi_iou_max, "debug.roi_iou_max", F32, {B, N}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.pos_indices, "debug.pos_indices", I32, {B, N}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.neg_indices, "debug.neg_indices", I32, {B, N}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.counts, "debug.counts", I32, {B, 6}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.sampled_pos, "debug.sampled_pos", I32, {B, R}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.sampled_neg, "debug.sampled_neg", I32, {B, R}, 4, scope));
+  OD_CHECK(check_opt_tensor(dbg.gt_assignment, "debug.gt_assignment", I32, {B, R}, 4, scope));
   if (B == 0 || R == 0) return OD_OK;
   if (!ws) OD_FAIL(OD_ERR_WORKSPACE, "workspace is NULL");
   Workspace w(ws, ws_bytes);

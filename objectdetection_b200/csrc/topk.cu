@@ -534,16 +534,12 @@ size_t od_topk_workspace_bytes(int64_t rows, int64_t cols, int64_t k) { return t
 
 int od_topk(const DLTensor* scores, int64_t k, DLTensor* values, DLTensor* indices, void* ws, size_t ws_bytes,
             void* stream) {
-  int dev = -1;
-  DeviceScope dev_scope;  // launches go to the tensors' device; the caller's current device is restored on return
-  OD_CHECK(check_tensor(scores, "scores", F32, 2, false, &dev));
-  OD_CHECK(check_tensor(indices, "indices", I32, 2, true, &dev));
+  DeviceScope scope;
+  OD_CHECK(check_tensor(scores, "scores", F32, {kAny, kAny}, 4, scope, /*any_strides=*/true));
   const int64_t rows = scores->shape[0], cols = scores->shape[1];
-  if (indices->shape[0] != rows || indices->shape[1] != k) OD_FAIL(OD_ERR_SHAPE, "indices must be [rows,k]");
-  if (values) {
-    OD_CHECK(check_tensor(values, "values", F32, 2, true, &dev));
-    if (values->shape[0] != rows || values->shape[1] != k) OD_FAIL(OD_ERR_SHAPE, "values must be [rows,k]");
-  }
+  if (k < 0) OD_FAIL(OD_ERR_SHAPE, "indices: k = %lld is negative", (long long)k);
+  OD_CHECK(check_tensor(indices, "indices", I32, {rows, k}, 4, scope));
+  OD_CHECK(check_opt_tensor(values, "values", F32, {rows, k}, 4, scope));
   return topk_launch(dptr<float>(scores), rows, cols, stride_of(scores, 0), stride_of(scores, 1), k,
                      dptr<int32_t>(indices), dptr<float>(values), ws, ws_bytes, static_cast<cudaStream_t>(stream));
 }

@@ -17,6 +17,8 @@ void set_error_detail(const char* fmt, ...) {
 
 static bool is_contiguous(const DLTensor* t) {
   if (!t->strides) return true;
+  for (int i = 0; i < t->ndim; ++i)
+    if (t->shape[i] == 0) return true;   // no element to address: any strides describe it (torch gives [B,0,4] stride 4)
   int64_t expect = 1;
   for (int i = t->ndim - 1; i >= 0; --i) {
     if (t->shape[i] != 1 && t->strides[i] != expect) return false;

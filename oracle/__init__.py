@@ -410,9 +410,15 @@ def mrcnn_losses(mrcnn_target_class_ids, mrcnn_pred_logits, batch_active_class_i
     ids = np.asarray(mrcnn_target_class_ids).astype(np.int64)
     lg, act = _f32(mrcnn_pred_logits), _f32(batch_active_class_ids)
     B, R, C = lg.shape
-    pred_cls = lg.argmax(-1)                                        # (:113)
+    # tf.argmax (:113) as a serial scan with a strict '>' (the rule of DetectionLayer's argmax too): the first maximum
+    # wins and a NaN never replaces the running maximum, where np.argmax would return the first NaN
+    pred_cls = np.zeros((B, R), np.int64)
+    m = lg[..., 0].copy()
+    for j in range(1, C):
+        up = lg[..., j] > m
+        pred_cls[up] = j
+        m[up] = lg[..., j][up]
     pred_active = act[0][pred_cls]                                  # tf.gather(batch_active_class_ids[0], .) (:115)
-    m = lg.max(-1)
     s = np.zeros((B, R), np.float32)
     for j in range(C):                                              # fp32 sum in class order
         s = s + _exp32(lg[..., j] - m)

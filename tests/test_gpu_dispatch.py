@@ -2,7 +2,7 @@
 The tests here reach the branches that the benchmark-sized inputs of test_gpu_parity.py never take, check the outputs
 against the CPU oracle as strictly as test_gpu_parity.py does, and read from a CUDA kernel trace that the intended
 kernel ran and its sibling did not, so that a retuned threshold cannot silently turn a test into a test of another
-branch. Non-power-of-two depths are also compared with a float64 numpy crop_and_resize written here.
+branch. Non-power-of-two depths are also compared with the float64 crop_and_resize of tests/_f64_refs.py.
 
 KERNEL_PATHS names, for every __global__ kernel in objectdetection_b200/csrc, the test that launches it;
 test_kernel_paths_cover_every_kernel (no GPU) fails when a kernel is missing from it."""
@@ -18,6 +18,7 @@ import pytest
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 import _synth  # noqa: E402
+from _f64_refs import crop_and_resize_f64  # noqa: E402
 
 import oracle  # noqa: E402
 from objectdetection_b200.config import ShapesConfig, config as Conf  # noqa: E402
@@ -166,49 +167,6 @@ def _cuda():
 
 
 # ------------------------------------------------------------------ float64 crop_and_resize
-def crop_and_resize_f64(image, boxes, box_ind, ph, pw, extrapolation=0.0, edge_tol=1e-4):
-    """tf.image.crop_and_resize (bilinear) in float64: in_y = y1*(H-1) + y*(y2-y1)*(H-1)/(ph-1) (the centre
-    0.5*(y1+y2)*(H-1) when ph == 1), samples outside [0, H-1] x [0, W-1] take the extrapolation value.
-    Returns (crops [n,ph,pw,D] float64, comparable [n,ph,pw] bool). Not comparable: crops of an out-of-range box_ind
-    (left untouched by the kernels), non-finite positions, and samples within edge_tol pixel of the feature map's edge,
-    whose in/out decision rests on the fp32 rounding of the kernels' sample position."""
-    img = np.asarray(image, np.float64)
-    B, H, W, D = img.shape
-    n = boxes.shape[0]
-    out = np.zeros((n, ph, pw, D))
-    ok = np.zeros((n, ph, pw), bool)
-
-    def axis(a1, a2, size, steps):
-        if steps > 1:
-            pos = a1 * (size - 1) + np.arange(steps) * ((a2 - a1) * (size - 1) / (steps - 1))
-        else:
-            pos = np.array([0.5 * (a1 + a2) * (size - 1)])
-        fin = np.isfinite(pos)
-        p = np.where(fin, pos, -1.0)
-        inside = (p >= 0) & (p <= size - 1)
-        far = fin & (np.abs(p) > edge_tol) & (np.abs(p - (size - 1)) > edge_tol)
-        p = np.clip(p, 0, size - 1)
-        lo = np.floor(p).astype(np.int64)
-        return lo, np.ceil(p).astype(np.int64), p - lo, inside, far
-
-    for i in range(n):
-        b = int(box_ind[i])
-        if not 0 <= b < B:
-            continue
-        y1, x1, y2, x2 = (float(v) for v in boxes[i])
-        with np.errstate(invalid="ignore"):
-            top, bot, yl, in_y, far_y = axis(y1, y2, H, ph)
-            left, right, xl, in_x, far_x = axis(x1, x2, W, pw)
-        f = img[b]
-        xl_, yl_ = xl[None, :, None], yl[:, None, None]
-        t = f[top][:, left] + (f[top][:, right] - f[top][:, left]) * xl_
-        bt = f[bot][:, left] + (f[bot][:, right] - f[bot][:, left]) * xl_
-        v = t + (bt - t) * yl_
-        out[i] = np.where((in_y[:, None] & in_x[None, :])[..., None], v, extrapolation)
-        ok[i] = far_y[:, None] & far_x[None, :]
-    return out, ok
-
-
 def _assert_close_f64(got, want, ok, what):
     assert ok.mean() > 0.5, f"{what}: only {ok.mean():.3f} of the bins are comparable"
     err = np.abs(got.astype(np.float64) - want)[ok]

@@ -368,12 +368,22 @@ typedef struct od_frcnn_params {
   double base_anchors[16 * 4]; /* (x1,y1,x2,y2) per anchor, proposals.py:188-196 */
 } od_frcnn_params;
 
+/* Largest batch the proposal layer takes: its kernels put the image on a grid y / z extent (at most 65535). A batch is
+ * also refused when batch * post_nms_top_n exceeds 2^31 - 1 (int32 proposal rows). */
+#define OD_FRCNN_MAX_BATCH 65535
+
+/* Workspace of a batch of `batch` images of an fh x fw feature map; 0 for a NULL p or a batch outside
+ * [0, OD_FRCNN_MAX_BATCH]. The single-image query below returns its value at batch 1. */
+size_t od_frcnn_proposal_workspace_bytes_batch(int64_t batch, int64_t fh, int64_t fw, const od_frcnn_params* p);
 size_t od_frcnn_proposal_workspace_bytes(int64_t fh, int64_t fw, const od_frcnn_params* p);
-/* rpn_box_class_prob [1,h,w,2*na] f32|f64 (channels [:na] are read as fg, proposals.py:477),
- * rpn_bbox [1,h,w,4*na] same dtype (dx,dy,dw,dh per anchor).
- * proposals [post_nms_top_n,5] f32 rows (0,x1,y1,x2,y2); rows >= num_out[0] are zero.
- * num_out [1] i32. Scores are ranked by a flattened stable descending order (the intended
- * semantics of proposals.py:352-358; see DESIGN.md for the reference's argsort quirk). */
+/* A batch of B images with one image size and one set of thresholds (params):
+ * rpn_box_class_prob [B,h,w,2*na] f32|f64 (channels [:na] are read as fg, proposals.py:477), B <= OD_FRCNN_MAX_BATCH,
+ * rpn_bbox [B,h,w,4*na] same dtype (dx,dy,dw,dh per anchor).
+ * proposals [B*post_nms_top_n,5] f32 rows (b,x1,y1,x2,y2): the kept boxes of image 0 in visiting order, then those
+ * of image 1, and so on; rows >= num_out[0] + ... + num_out[B-1] are zero.
+ * num_out [B] i32: rows of image b. Each image's rows are those a batch of one gives for it.
+ * Scores are ranked by a flattened stable descending order (the intended semantics of proposals.py:352-358; see
+ * DESIGN.md for the reference's argsort quirk). */
 int od_frcnn_proposal_forward(const DLTensor* rpn_box_class_prob, const DLTensor* rpn_bbox,
                               const od_frcnn_params* params, DLTensor* proposals, DLTensor* num_out,
                               void* ws, size_t ws_bytes, void* stream);

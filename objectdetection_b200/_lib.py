@@ -122,6 +122,7 @@ SIGNATURES = {
     "od_detection_forward": (c_int, [_P, _P, _P, _P, POINTER(DetectionParams), _P, POINTER(DetectionDebug), _P,
                                      c_size_t, _P]),
     "od_unmold_detections": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P]),
+    "od_frcnn_proposal_workspace_bytes_batch": (c_size_t, [c_int64, c_int64, c_int64, POINTER(FrcnnParams)]),
     "od_frcnn_proposal_workspace_bytes": (c_size_t, [c_int64, c_int64, POINTER(FrcnnParams)]),
     "od_frcnn_proposal_forward": (c_int, [_P, _P, POINTER(FrcnnParams), _P, _P, _P, c_size_t, _P]),
     "od_roi_pool_forward": (c_int, [_P, _P, c_float, c_float, _P, _P]),

@@ -1,6 +1,8 @@
 // frcnn.cu — Faster R-CNN single-level proposal layer (FasterRCNN/building_blocks/proposals.py:392-512):
 // 9 base anchors + stride-16 shifts -> decode (+1 pixel widths, x1y1x2y2) -> clip -> min-size filter -> top-N by
-// score -> greedy NMS (areas (w+1)(h+1), suppress iff ovr >= thr) -> [n,5] rows (0,x1,y1,x2,y2).
+// score -> greedy NMS (areas (w+1)(h+1), suppress iff ovr >= thr) -> [n,5] rows (b,x1,y1,x2,y2).
+// A batch of B images runs as one chain: every kernel takes the image from a grid dimension and works on that image's
+// segment of each buffer, so image b's result does not depend on the other images of the batch.
 //
 // Arithmetic is fp64 like the reference's numpy code (fp32 inputs are widened exactly). The reference's top-N
 // (proposals.py:352) argsorts an [n,1] array along its length-1 axis, which selects box 0 n times; this
@@ -31,11 +33,17 @@ struct FrcnnDev {
   double base[16 * 4];
 };
 
+// grid (ceil(total/256), B). Image b reads probs [b] / bbox [b] and writes its segment of boxes [B,total,4], keys
+// [B,total] (fp64) or fscore [B,total] (fp32), and its valid counter num_valid[b].
 template <typename T>
 __global__ void frcnn_decode_kernel(const T* __restrict__ probs, const T* __restrict__ bbox, FrcnnDev p, int64_t total,
-                                    int64_t n_pow2, double* __restrict__ boxes, Key128* __restrict__ keys,
-                                    int32_t* __restrict__ counters, float* __restrict__ fscore) {
+                                    double* __restrict__ boxes, Key128* __restrict__ keys, int32_t* __restrict__ num_valid,
+                                    float* __restrict__ fscore) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int b = blockIdx.y;
+  probs += (int64_t)b * total * 2;   // [h,w,2*na] = 2 * total values per image
+  bbox += (int64_t)b * total * 4;
+  boxes += (int64_t)b * total * 4;
   Key128 k;
   k.hi = 0ull;                                            // filtered-out rows: below every valid key, still unique
   k.lo = 0xFFFFFFFFFFFFFFFFull - (unsigned long long)i;
@@ -68,31 +76,37 @@ __global__ void frcnn_decode_kernel(const T* __restrict__ probs, const T* __rest
       k.lo = 0xFFFFFFFFFFFFFFFFull - (unsigned long long)i;
     }
   }
-  if (fscore) {   // fp32 inputs: the radix-select top-k orders (score desc, index asc) like the 128-bit keys do
-    if (i < total) fscore[i] = valid ? (float)probs[(i / p.num_anchors) * 2 * p.num_anchors + (i % p.num_anchors)] : -INFINITY;
-  } else if (i < n_pow2) {
-    keys[i] = k;
+  if (i < total) {
+    if (fscore)   // fp32 inputs: the radix-select top-k orders (score desc, index asc) like the 128-bit keys do
+      fscore[(int64_t)b * total + i] = valid ? (float)probs[(i / p.num_anchors) * 2 * p.num_anchors + (i % p.num_anchors)] : -INFINITY;
+    else
+      keys[(int64_t)b * total + i] = k;
   }
   const uint32_t bal = __ballot_sync(0xffffffffu, valid);
-  if ((threadIdx.x & 31) == 0 && bal) atomicAdd(&counters[0], __popc(bal));
+  if ((threadIdx.x & 31) == 0 && bal) atomicAdd(&num_valid[b], __popc(bal));
 }
 
-// Rank sort fused with the gather: keys are unique, the visiting position of a box is the number of keys greater
-// than its own. grid ceil(total/32); a CTA owns 32 keys, 8 thread groups each count over an 8th of every 1024-key
-// tile in shared memory. Position r < K receives the box (zeros for filtered-out rows); counters[1] = npre.
+// Rank sort fused with the gather: keys are unique, the visiting position of a box is the number of keys of its own
+// image greater than its own. grid (ceil(total/32), B); a CTA owns 32 keys of image blockIdx.y, 8 thread groups each
+// count over an 8th of every 1024-key tile in shared memory. Position r < K of the image's segment of sorted [B,K,4]
+// receives the box (zeros for filtered-out rows); npre[b] = min(num_valid[b], pre_n).
 constexpr int kFrRankThreads = 256;
 constexpr int kFrRankMine = 32;
 constexpr int kFrRankTile = 1024;
 __global__ void __launch_bounds__(kFrRankThreads)
 frcnn_rank_gather_kernel(const Key128* __restrict__ keys, const double* __restrict__ boxes, int64_t total, int pre_n, int K,
-                         double* __restrict__ sorted, int32_t* __restrict__ counters) {
+                         double* __restrict__ sorted, const int32_t* __restrict__ num_valid, int32_t* __restrict__ npre) {
   __shared__ unsigned long long tile_hi[kFrRankTile];   // score keys
   __shared__ unsigned long long tile_lo[kFrRankTile];
   __shared__ int32_t partial[kFrRankThreads];
   constexpr int kParts = kFrRankThreads / kFrRankMine;
   const int64_t me = (int64_t)blockIdx.x * kFrRankMine + (threadIdx.x & (kFrRankMine - 1));
   const int part = threadIdx.x / kFrRankMine;
-  if (blockIdx.x == 0 && threadIdx.x == 0) counters[1] = min(counters[0], pre_n);
+  const int b = blockIdx.y;
+  keys += (int64_t)b * total;
+  boxes += (int64_t)b * total * 4;
+  sorted += (int64_t)b * K * 4;
+  if (blockIdx.x == 0 && threadIdx.x == 0) npre[b] = min(num_valid[b], pre_n);
   Key128 mine;
   mine.hi = ~0ull;
   mine.lo = ~0ull;
@@ -143,14 +157,18 @@ __device__ __forceinline__ PBox load_pbox(const double* b) {
 // larger images send every pair to the fp64 path.
 constexpr int kFrcnnScreenMaxSide = 8192;
 
-// proposals.py:141-164 as 64x64 tiles (i = kept/earlier box, j = later box).
+// proposals.py:141-164 as 64x64 tiles (i = kept/earlier box, j = later box). grid (W, W, B): image blockIdx.z reads
+// its [K,4] segment of sorted boxes and writes mask [B,K,Ws] and diagT [B,W,64], the layout nms_scan_launch reads.
 __global__ void __launch_bounds__(64)
-frcnn_mask_kernel(const double* __restrict__ boxes, const int32_t* __restrict__ counters, int K, int W, int Ws, double thr,
+frcnn_mask_kernel(const double* __restrict__ boxes, const int32_t* __restrict__ npre, int K, int W, int Ws, double thr,
                   int screen, unsigned long long* __restrict__ mask, unsigned long long* __restrict__ diagT) {
-  const int cb = blockIdx.x, rb = blockIdx.y;
+  const int cb = blockIdx.x, rb = blockIdx.y, b = blockIdx.z;
   if (cb < rb) return;
-  const int n = min(counters[1], K);
+  const int n = min(npre[b], K);
   if (rb * 64 >= n || cb * 64 >= n) return;
+  boxes += (int64_t)b * K * 4;
+  mask += (int64_t)b * K * Ws;
+  diagT += (int64_t)b * W * 64;
   __shared__ PBox cbox[64];
   __shared__ float cf[64][5];   // fp32 copies for the screening pass: x1, y1, x2 + 1, y2 + 1, area
   const int t = threadIdx.x;
@@ -209,34 +227,79 @@ frcnn_mask_kernel(const double* __restrict__ boxes, const int32_t* __restrict__ 
   }
 }
 
-// fp32 path: position p of the visiting order holds box ix[p] (zeros past the valid ones); counters[1] = npre.
-__global__ void frcnn_gather_kernel(const int32_t* __restrict__ ix, const double* __restrict__ boxes, int pre_n, int K,
-                                    double* __restrict__ sorted, int32_t* __restrict__ counters) {
+// fp32 path: position p of image b's visiting order holds box ix[b,p] (zeros past the valid ones); grid
+// (ceil(K/256), B); npre[b] = min(num_valid[b], pre_n).
+__global__ void frcnn_gather_kernel(const int32_t* __restrict__ ix, const double* __restrict__ boxes, int64_t total,
+                                    int pre_n, int K, double* __restrict__ sorted, const int32_t* __restrict__ num_valid,
+                                    int32_t* __restrict__ npre) {
   const int p = blockIdx.x * blockDim.x + threadIdx.x;
-  const int npre = min(counters[0], pre_n);
-  if (p == 0) counters[1] = npre;
+  const int b = blockIdx.y;
+  const int n = min(num_valid[b], pre_n);
+  if (p == 0) npre[b] = n;
   if (p >= K) return;
-  const bool valid = p < npre;
-  const int64_t src = valid ? ix[p] : 0;
+  const bool valid = p < n;
+  const int64_t src = valid ? ix[(int64_t)b * K + p] : 0;
+  OD_DBG_IDX(src, total);
+  const double* bx = boxes + (int64_t)b * total * 4;
+  double* o = sorted + ((int64_t)b * K + p) * 4;
 #pragma unroll
-  for (int c = 0; c < 4; ++c) sorted[4 * (int64_t)p + c] = valid ? boxes[4 * src + c] : 0.0;
+  for (int c = 0; c < 4; ++c) o[c] = valid ? bx[4 * src + c] : 0.0;
 }
 
-__global__ void frcnn_emit_kernel(const double* __restrict__ sorted, const int32_t* __restrict__ keep_pos,
-                                  const int32_t* __restrict__ num_kept, int post_n, float* __restrict__ out,
-                                  int32_t* __restrict__ num_out) {
-  const int j = blockIdx.x * blockDim.x + threadIdx.x;
-  if (j == 0) num_out[0] = num_kept[0];
-  if (j >= post_n) return;
-  const int p = keep_pos[j];
-  float* o = out + 5 * (int64_t)j;
-  o[0] = 0.0f;
+// grid (ceil(post_n/256), B), 256 threads. Image b's kept boxes go to rows [off, off + num_kept[b]) of out
+// [B*post_n,5], off = num_kept[0] + ... + num_kept[b-1], as (b,x1,y1,x2,y2); rows from the batch's total on are zero.
+constexpr int kFrEmitThreads = 256;
+__global__ void __launch_bounds__(kFrEmitThreads)
+frcnn_emit_kernel(const double* __restrict__ sorted, const int32_t* __restrict__ keep_pos, const int32_t* __restrict__ num_kept,
+                  int B, int K, int post_n, float* __restrict__ out, int32_t* __restrict__ num_out) {
+  __shared__ int32_t red[2][kFrEmitThreads / 32];
+  const int j = blockIdx.x * kFrEmitThreads + threadIdx.x;
+  const int b = blockIdx.y;
+  int before = 0, all = 0;   // < B * post_n < 2^31: the entry point caps B
+  for (int q = threadIdx.x; q < B; q += kFrEmitThreads) {
+    const int v = num_kept[q];
+    all += v;
+    before += q < b ? v : 0;
+  }
 #pragma unroll
-  for (int c = 0; c < 4; ++c) o[1 + c] = (p >= 0) ? (float)sorted[4 * (int64_t)p + c] : 0.0f;
+  for (int o = 16; o > 0; o >>= 1) {
+    before += __shfl_xor_sync(0xffffffffu, before, o);
+    all += __shfl_xor_sync(0xffffffffu, all, o);
+  }
+  if ((threadIdx.x & 31) == 0) {
+    red[0][threadIdx.x >> 5] = before;
+    red[1][threadIdx.x >> 5] = all;
+  }
+  __syncthreads();
+  before = 0;
+  all = 0;
+#pragma unroll
+  for (int w = 0; w < kFrEmitThreads / 32; ++w) {
+    before += red[0][w];
+    all += red[1][w];
+  }
+  const int n = num_kept[b];
+  if (j == 0) num_out[b] = n;
+  if (j >= post_n) return;
+  if (j < n) {
+    const int p = keep_pos[(int64_t)b * post_n + j];
+    OD_DBG_IDX(p, K);
+    const double* s = sorted + ((int64_t)b * K + p) * 4;
+    float* o = out + 5 * ((int64_t)before + j);
+    o[0] = (float)b;
+#pragma unroll
+    for (int c = 0; c < 4; ++c) o[1 + c] = (float)s[c];
+  }
+  const int64_t r = (int64_t)b * post_n + j;   // every row index of the output is visited once
+  if (r >= all) {
+    float* o = out + 5 * r;
+#pragma unroll
+    for (int c = 0; c < 5; ++c) o[c] = 0.0f;
+  }
 }
 
 struct FrcnnWs {
-  int32_t* counters;   // [0] #valid, [1] npre, [2] num_kept
+  int32_t* counters;   // [3][B]: #valid, npre, num_kept of every image (nms_scan_launch reads [B] arrays)
   Key128* keys;
   double* boxes;
   double* sorted;
@@ -248,20 +311,19 @@ struct FrcnnWs {
   void* topk_ws;
   size_t topk_bytes;
 };
-static size_t carve_frcnn_ws(Workspace& w, int64_t total, int64_t K, int64_t post_n, FrcnnWs* out) {
+static size_t carve_frcnn_ws(Workspace& w, int64_t B, int64_t total, int64_t K, int64_t post_n, FrcnnWs* out) {
   FrcnnWs f;
-  const int64_t n_pow2 = next_pow2(total > 0 ? total : 1);
   const int64_t W = (K + 63) / 64;
-  f.counters = w.take<int32_t>(64);
-  f.keys = w.take<Key128>((size_t)n_pow2);
-  f.boxes = w.take<double>((size_t)(4 * total));
-  f.sorted = w.take<double>((size_t)(4 * K));
-  f.keep_pos = w.take<int32_t>((size_t)post_n);
-  f.mask = w.take<unsigned long long>((size_t)(K * nms_mask_stride(K)));
-  f.diagT = w.take<unsigned long long>((size_t)(W * 64));
-  f.fscore = w.take<float>((size_t)(total > 0 ? total : 1));
-  f.ix = w.take<int32_t>((size_t)(K > 0 ? K : 1));
-  f.topk_bytes = topk_workspace_bytes(1, total, K);
+  f.counters = w.take<int32_t>((size_t)(3 * B));
+  f.keys = w.take<Key128>((size_t)(B * total));
+  f.boxes = w.take<double>((size_t)(B * 4 * total));
+  f.sorted = w.take<double>((size_t)(B * 4 * K));
+  f.keep_pos = w.take<int32_t>((size_t)(B * post_n));
+  f.mask = w.take<unsigned long long>((size_t)(B * K * nms_mask_stride(K)));
+  f.diagT = w.take<unsigned long long>((size_t)(B * W * 64));
+  f.fscore = w.take<float>((size_t)(B * total));
+  f.ix = w.take<int32_t>((size_t)(B * K));
+  f.topk_bytes = topk_workspace_bytes(B, total, K);
   f.topk_ws = w.take<char>(f.topk_bytes);
   if (out) *out = f;
   return w.off + 256;
@@ -273,12 +335,16 @@ using namespace od;
 
 extern "C" {
 
-size_t od_frcnn_proposal_workspace_bytes(int64_t fh, int64_t fw, const od_frcnn_params* p) {
-  if (!p) return 0;
+size_t od_frcnn_proposal_workspace_bytes_batch(int64_t batch, int64_t fh, int64_t fw, const od_frcnn_params* p) {
+  if (!p || batch < 0 || batch > OD_FRCNN_MAX_BATCH || fh < 0 || fw < 0) return 0;
   const int64_t total = fh * fw * p->num_anchors;
   const int64_t K = total < p->pre_nms_top_n ? total : p->pre_nms_top_n;
   Workspace w(nullptr, 0);
-  return carve_frcnn_ws(w, total, K, p->post_nms_top_n, nullptr);
+  return carve_frcnn_ws(w, batch, total, K, p->post_nms_top_n, nullptr);
+}
+
+size_t od_frcnn_proposal_workspace_bytes(int64_t fh, int64_t fw, const od_frcnn_params* p) {
+  return od_frcnn_proposal_workspace_bytes_batch(1, fh, fw, p);
 }
 
 int od_frcnn_proposal_forward(const DLTensor* rpn_box_class_prob, const DLTensor* rpn_bbox, const od_frcnn_params* params,
@@ -293,51 +359,62 @@ int od_frcnn_proposal_forward(const DLTensor* rpn_box_class_prob, const DLTensor
   const int64_t post_n = params->post_nms_top_n;
   if (post_n < 0 || params->pre_nms_top_n < 0) OD_FAIL(OD_ERR_PARAM, "negative top-n");
   DeviceScope scope;
-  OD_CHECK(check_tensor(rpn_box_class_prob, "rpn_box_class_prob", f64 ? F64 : F32, {1, kAny, kAny, 2 * na}, f64 ? 8 : 4, scope));
-  const int64_t fh = rpn_box_class_prob->shape[1], fw = rpn_box_class_prob->shape[2];
-  OD_CHECK(check_tensor(rpn_bbox, "rpn_bbox", f64 ? F64 : F32, {1, fh, fw, 4 * na}, f64 ? 8 : 4, scope));
-  OD_CHECK(check_tensor(proposals, "proposals", F32, {post_n, 5}, 4, scope));
-  OD_CHECK(check_tensor(num_out, "num_out", I32, {1}, 4, scope));
+  // the batch size is read from rpn_box_class_prob; every other tensor is checked against it
+  OD_CHECK(check_tensor(rpn_box_class_prob, "rpn_box_class_prob", f64 ? F64 : F32, {kAny, kAny, kAny, 2 * na}, f64 ? 8 : 4, scope));
+  const int64_t B = rpn_box_class_prob->shape[0], fh = rpn_box_class_prob->shape[1], fw = rpn_box_class_prob->shape[2];
+  // grid y / z extents are at most 65535, and output rows are int32 indices
+  if (B > OD_FRCNN_MAX_BATCH)
+    OD_FAIL(OD_ERR_PARAM, "rpn_box_class_prob: batch %lld > %d images", (long long)B, OD_FRCNN_MAX_BATCH);
+  if (B * post_n > INT32_MAX)
+    OD_FAIL(OD_ERR_PARAM, "batch %lld x post_nms_top_n %lld proposal rows exceed 2^31 - 1", (long long)B, (long long)post_n);
+  OD_CHECK(check_tensor(rpn_bbox, "rpn_bbox", f64 ? F64 : F32, {B, fh, fw, 4 * na}, f64 ? 8 : 4, scope));
+  OD_CHECK(check_tensor(proposals, "proposals", F32, {B * post_n, 5}, 4, scope));
+  OD_CHECK(check_tensor(num_out, "num_out", I32, {B}, 4, scope));
   const int64_t total = fh * fw * na;
   const int64_t K = total < params->pre_nms_top_n ? total : params->pre_nms_top_n;
-  if (post_n == 0) return OD_OK;
+  if (post_n == 0 || B == 0) return OD_OK;
   if (!ws) OD_FAIL(OD_ERR_WORKSPACE, "workspace is NULL");
   Workspace w(ws, ws_bytes);
   FrcnnWs f;
-  carve_frcnn_ws(w, total, K, post_n, &f);
+  carve_frcnn_ws(w, B, total, K, post_n, &f);
   if (!w.ok()) OD_FAIL(OD_ERR_WORKSPACE, "workspace %zu < %zu bytes", ws_bytes, w.off);
-  OD_CUDA(cudaMemsetAsync(f.counters, 0, 64 * sizeof(int32_t), st));
+  int32_t* num_valid = f.counters;
+  int32_t* npre = f.counters + B;
+  int32_t* num_kept = f.counters + 2 * B;
+  OD_CUDA(cudaMemsetAsync(f.counters, 0, (size_t)(3 * B) * sizeof(int32_t), st));
   FrcnnDev d;
   d.feat_stride = params->feat_stride; d.image_h = params->image_h; d.image_w = params->image_w;
   d.min_box_hw = params->min_box_hw; d.num_anchors = na; d.fw = (int32_t)fw;
   for (int i = 0; i < 4 * na; ++i) d.base[i] = params->base_anchors[i];
-  const int64_t n_pow2 = next_pow2(total > 0 ? total : 1);
-  const unsigned blocks = (unsigned)((n_pow2 + 255) / 256);
+  const dim3 dgrid((unsigned)((total + 255) / 256 > 0 ? (total + 255) / 256 : 1), (unsigned)B);
   if (f64)
-    frcnn_decode_kernel<double><<<blocks, 256, 0, st>>>(dptr<double>(rpn_box_class_prob), dptr<double>(rpn_bbox), d, total, n_pow2, f.boxes, f.keys, f.counters, nullptr);
+    frcnn_decode_kernel<double><<<dgrid, 256, 0, st>>>(dptr<double>(rpn_box_class_prob), dptr<double>(rpn_bbox), d, total, f.boxes, f.keys, num_valid, nullptr);
   else
-    frcnn_decode_kernel<float><<<blocks, 256, 0, st>>>(dptr<float>(rpn_box_class_prob), dptr<float>(rpn_bbox), d, total, n_pow2, f.boxes, f.keys, f.counters, f.fscore);
+    frcnn_decode_kernel<float><<<dgrid, 256, 0, st>>>(dptr<float>(rpn_box_class_prob), dptr<float>(rpn_bbox), d, total, f.boxes, f.keys, num_valid, f.fscore);
   OD_LAUNCH_CHECK("frcnn_decode_kernel");
   const int W = (int)((K + 63) / 64);
   if (K > 0) {
     if (f64) {   // fp64 scores: 128-bit keys, rank sort
-      frcnn_rank_gather_kernel<<<(unsigned)((total + kFrRankMine - 1) / kFrRankMine), kFrRankThreads, 0, st>>>(
-          f.keys, f.boxes, total, params->pre_nms_top_n, (int)K, f.sorted, f.counters);
+      const dim3 grid((unsigned)((total + kFrRankMine - 1) / kFrRankMine), (unsigned)B);
+      frcnn_rank_gather_kernel<<<grid, kFrRankThreads, 0, st>>>(f.keys, f.boxes, total, params->pre_nms_top_n, (int)K, f.sorted,
+                                                                num_valid, npre);
       OD_LAUNCH_CHECK("frcnn_rank_gather_kernel");
     } else {     // fp32 scores: the radix-select top-k of the Mask R-CNN path, filtered-out boxes at -inf
-      OD_CHECK(topk_launch(f.fscore, 1, total, total, 1, K, f.ix, nullptr, f.topk_ws, f.topk_bytes, st));
-      frcnn_gather_kernel<<<(unsigned)((K + 255) / 256), 256, 0, st>>>(f.ix, f.boxes, params->pre_nms_top_n, (int)K, f.sorted, f.counters);
+      OD_CHECK(topk_launch(f.fscore, B, total, total, 1, K, f.ix, nullptr, f.topk_ws, f.topk_bytes, st));
+      const dim3 grid((unsigned)((K + 255) / 256), (unsigned)B);
+      frcnn_gather_kernel<<<grid, 256, 0, st>>>(f.ix, f.boxes, total, params->pre_nms_top_n, (int)K, f.sorted, num_valid, npre);
       OD_LAUNCH_CHECK("frcnn_gather_kernel");
     }
-    const dim3 grid((unsigned)W, (unsigned)W, 1);
+    const dim3 grid((unsigned)W, (unsigned)W, (unsigned)B);
     const int screen = params->image_h <= kFrcnnScreenMaxSide && params->image_w <= kFrcnnScreenMaxSide;
-    frcnn_mask_kernel<<<grid, 64, 0, st>>>(f.sorted, f.counters, (int)K, W, (int)nms_mask_stride(K), params->nms_threshold, screen,
+    frcnn_mask_kernel<<<grid, 64, 0, st>>>(f.sorted, npre, (int)K, W, (int)nms_mask_stride(K), params->nms_threshold, screen,
                                            f.mask, f.diagT);
     OD_LAUNCH_CHECK("frcnn_mask_kernel");
   }
-  OD_CHECK(nms_scan_launch(f.mask, f.diagT, f.counters + 1, 1, K, nms_mask_stride(K), post_n, f.keep_pos, f.counters + 2, nullptr, st));
-  frcnn_emit_kernel<<<(unsigned)((post_n + 255) / 256), 256, 0, st>>>(f.sorted, f.keep_pos, f.counters + 2, (int)post_n,
-                                                                     dptr<float>(proposals), dptr<int32_t>(num_out));
+  OD_CHECK(nms_scan_launch(f.mask, f.diagT, npre, B, K, nms_mask_stride(K), post_n, f.keep_pos, num_kept, nullptr, st));
+  const dim3 egrid((unsigned)((post_n + kFrEmitThreads - 1) / kFrEmitThreads), (unsigned)B);
+  frcnn_emit_kernel<<<egrid, kFrEmitThreads, 0, st>>>(f.sorted, f.keep_pos, num_kept, (int)B, (int)K, (int)post_n,
+                                                      dptr<float>(proposals), dptr<int32_t>(num_out));
   OD_LAUNCH_CHECK("frcnn_emit_kernel");
   return OD_OK;
 }

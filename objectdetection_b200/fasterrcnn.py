@@ -21,7 +21,10 @@ def get_anchors():
 
 class Proposals():
     """``Proposals(mode, rpn_box_class_prob, rpn_bbox)`` (proposals.py:374): numpy/torch inputs of shape
-    [1,h,w,18] and [1,h,w,36] -> ``get_proposals()`` [n,5] float32 rows (0, x1, y1, x2, y2).
+    [B,h,w,18] and [B,h,w,36] -> ``get_proposals()`` [n,5] float32 rows (b, x1, y1, x2, y2): the kept boxes of image 0,
+    then those of image 1, and so on, ready for ``roi_pool`` on a [B,h',w',D] feature map. ``num_proposals`` [B] int32
+    holds the rows of each image and ``proposals_padded`` [B*post_nms_top_n,5] the same rows followed by zeros.
+    Every image is processed as in a batch of one, with one image shape and one set of thresholds for the batch.
 
     ``image_shape`` / thresholds default to the reference's hard-coded values (proposals.py:378-389) and can be
     overridden for other configurations (e.g. 600x1000, 12000 -> 2000, thr 0.7).
@@ -59,14 +62,16 @@ class Proposals():
         p.nms_threshold, p.num_anchors = float(self.NMS_THRESHOLD), base.shape[0]
         for i, v in enumerate(base.reshape(-1)):
             p.base_anchors[i] = float(v)
-        out = torch.empty((self.POST_NMS_TOP_N, 5), dtype=torch.float32, device=dev)
-        num = torch.empty((1,), dtype=torch.int32, device=dev)
-        ws = _lib.workspace(L.od_frcnn_proposal_workspace_bytes(probs.shape[1], probs.shape[2], ctypes.byref(p)), dev)
+        B = probs.shape[0]
+        out = torch.empty((B * self.POST_NMS_TOP_N, 5), dtype=torch.float32, device=dev)
+        num = torch.empty((B,), dtype=torch.int32, device=dev)
+        ws = _lib.workspace(L.od_frcnn_proposal_workspace_bytes_batch(B, probs.shape[1], probs.shape[2], ctypes.byref(p)),
+                            dev)
         dl = _lib.DL()
         _lib.check(L.od_frcnn_proposal_forward(dl(probs), dl(bbox), ctypes.byref(p), dl(out), dl(num), ws.data_ptr(),
                                                ws.numel(), _lib.stream_ptr(dev)), "od_frcnn_proposal_forward")
         self.proposals_padded, self.num_proposals = out, num
-        self.proposals = out[:int(num.item())]
+        self.proposals = out[:int(num.sum().item())]   # one host read for the whole batch
 
     def get_proposals(self):
         return self.proposals

@@ -194,10 +194,15 @@ int od_proposal_forward_levels(const DLTensor* const* class_logits, const DLTens
                                void* ws, size_t ws_bytes, void* stream);
 
 /* ---- PyramidROIAlign (maskrcnn.py:74-187) ---------------------------------- */
-/* fmaps[l]: [B,H_l,W_l,D] f32 NHWC for level (min_level + l), l < num_levels;
+/* fmaps[l]: [B,H_l,W_l,D] f32 or bf16 NHWC for level (min_level + l), l < num_levels, every level of one dtype;
  * rois [B,N,4] f32 normalised (y1,x1,y2,x2);
- * pooled: [1,B*N,P_h,P_w,D] (or [B*N,P_h,P_w,D]) f32; row b*N+n <-> rois[b,n];
- * roi_level: [B,N] i32 or NULL. D must be a multiple of 4. */
+ * pooled: [1,B*N,P_h,P_w,D] (or [B*N,P_h,P_w,D]) f32 or bf16, whatever the maps' dtype; row b*N+n <-> rois[b,n];
+ * roi_level: [B,N] i32 or NULL. D must be a multiple of 4, and of 8 when the maps or pooled are bf16 (kDLBfloat, 16 bits;
+ * float16 is refused like every other dtype).
+ * Numerics: the blend is fp32 in the reference's order; bf16 map values are widened exactly, so an f32 pooled result from
+ * bf16 maps equals the f32 path on the widened maps bit for bit. A bf16 pooled value is that fp32 value rounded to the
+ * nearest bf16, ties to even (overflow to inf; NaN stays NaN, its payload may differ). The same holds for
+ * od_crop_and_resize, whose extrapolation_value is rounded the same way. */
 int od_pyramid_roi_align_forward(const DLTensor* const* fmaps, int32_t num_levels, int32_t min_level,
                                  const DLTensor* rois, int32_t image_h, int32_t image_w,
                                  int32_t pool_h, int32_t pool_w,
@@ -228,9 +233,9 @@ int od_pyramid_roi_align_forward_ws(const DLTensor* const* fmaps, int32_t num_le
                                     int32_t pool_h, int32_t pool_w,
                                     DLTensor* pooled, DLTensor* roi_level, void* ws, size_t ws_bytes, void* stream);
 
-/* tf.image.crop_and_resize(method="bilinear"): image [B,H,W,D] f32 NHWC,
+/* tf.image.crop_and_resize(method="bilinear"): image [B,H,W,D] f32 or bf16 NHWC,
  * boxes [n,4] f32, box_ind [n] i32 (out-of-range -> that crop is left untouched),
- * out [n,crop_h,crop_w,D] f32. */
+ * out [n,crop_h,crop_w,D] f32 or bf16 (dtypes, D and numerics as od_pyramid_roi_align_forward). */
 int od_crop_and_resize(const DLTensor* image, const DLTensor* boxes, const DLTensor* box_ind,
                        int32_t crop_h, int32_t crop_w, float extrapolation_value,
                        DLTensor* out, void* stream);

@@ -71,7 +71,7 @@ struct DeviceScope {
 };
 
 // ----------------------------------------------------------------------------- DLPack checks
-enum DType { F32, F64, I32 };
+enum DType { F32, F64, I32, BF16 };   // BF16: kDLBfloat, 16 bits (float16 is kDLFloat, 16 bits, and matches none)
 // An extent check_tensor accepts at any value. A caller's int64 parameter is checked for a negative value before it is
 // used as an extent, so that it cannot pass as kAny.
 constexpr int64_t kAny = INT64_MIN;

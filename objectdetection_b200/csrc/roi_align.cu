@@ -20,19 +20,23 @@
 //      i.e. 8 loads in flight per thread), 3 lerps on packed fp32 pairs (FADD2) and one streaming
 //      16-byte store. No meta kernel, no per-call allocation.
 //   crop_pool_bins_kernel : FasterRCNN roi_pool = crop 14x14 fused with 2x2 max-pool, same scheme over pooled bins.
+#include <cuda_bf16.h>
+
+#include <type_traits>
+
 #include "common.cuh"
 #include "tma.cuh"
 
 namespace od {
 
 struct __align__(16) RoiMeta {
-  const float* base;  // image (level, batch) base; nullptr -> crop skipped (box_ind out of range)
+  const void* base;   // image (level, batch) base, an fp32 or bf16 array
   int32_t H, W;
   float in_y0, hs, in_x0, ws;  // in_y = in_y0 + y * hs   (TF: y1*(H-1) + y*height_scale)
 };
 
 struct LevelTable {
-  const float* ptr[OD_MAX_LEVELS];
+  const void* ptr[OD_MAX_LEVELS];               // NHWC maps of one dtype: fp32 or bf16
   int32_t H[OD_MAX_LEVELS];
   int32_t W[OD_MAX_LEVELS];
 };
@@ -156,11 +160,81 @@ __device__ __forceinline__ float4 lerp4p(float4 a, float4 b, float t) {
   return r;
 }
 
+// ----------------------------------------------------------------------------- fp32 and bf16 units
+// The kernels move a feature pixel in 16-byte units: 4 fp32 channels, or 8 bf16 channels. A bf16 unit is widened to fp32
+// exactly (a bf16 is the upper half of an fp32) and blended like two fp32 units, so the fp32 result does not depend on
+// the map dtype. The result is stored as fp32, or rounded to the nearest bf16, ties to even (cvt.rn.bf16x2.f32).
+struct float8 {                                    // the 8 channels of one bf16 unit, widened
+  float4 lo, hi;
+};
+struct __align__(8) bf16x4 {                       // pooled output unit, fp32 maps -> bf16
+  __nv_bfloat162 v[2];
+};
+struct __align__(16) bf16x8 {                      // pooled output unit, bf16 maps -> bf16
+  __nv_bfloat162 v[4];
+};
+template <typename TMap> struct MapUnit;           // Raw: as loaded; Val: widened to fp32; kCh channels
+template <> struct MapUnit<float> {
+  using Raw = float4;
+  using Val = float4;
+  static constexpr int kCh = 4;
+};
+template <> struct MapUnit<__nv_bfloat16> {
+  using Raw = uint4;
+  using Val = float8;
+  static constexpr int kCh = 8;
+};
+template <typename TMap, typename TOut> struct OutUnit;   // one map unit's channels in the pooled dtype
+template <> struct OutUnit<float, float> { using T = float4; };
+template <> struct OutUnit<__nv_bfloat16, float> { using T = float8; };
+template <> struct OutUnit<float, __nv_bfloat16> { using T = bf16x4; };
+template <> struct OutUnit<__nv_bfloat16, __nv_bfloat16> { using T = bf16x8; };
+
+__device__ __forceinline__ float4 widen_unit(float4 v) { return v; }
+__device__ __forceinline__ float8 widen_unit(uint4 v) {
+  float8 r;
+  r.lo = make_float4(__uint_as_float(v.x << 16), __uint_as_float(v.x & 0xFFFF0000u), __uint_as_float(v.y << 16),
+                     __uint_as_float(v.y & 0xFFFF0000u));
+  r.hi = make_float4(__uint_as_float(v.z << 16), __uint_as_float(v.z & 0xFFFF0000u), __uint_as_float(v.w << 16),
+                     __uint_as_float(v.w & 0xFFFF0000u));
+  return r;
+}
+__device__ __forceinline__ float4 ldg_unit(const float4* p) { return ldg_f4(p); }
+__device__ __forceinline__ float8 ldg_unit(const uint4* p) { return widen_unit(__ldg(p)); }
+template <typename V> __device__ __forceinline__ V splat_unit(float v);
+template <> __device__ __forceinline__ float4 splat_unit<float4>(float v) { return make_float4(v, v, v, v); }
+template <> __device__ __forceinline__ float8 splat_unit<float8>(float v) {
+  return {make_float4(v, v, v, v), make_float4(v, v, v, v)};
+}
+// the fp32 blends of a bf16 unit: the same operations on both halves
+__device__ __forceinline__ float8 sub4p(float8 b, float8 a) { return {sub4p(b.lo, a.lo), sub4p(b.hi, a.hi)}; }
+__device__ __forceinline__ float8 axpy4p(float8 a, float8 d, float t) { return {axpy4p(a.lo, d.lo, t), axpy4p(a.hi, d.hi, t)}; }
+__device__ __forceinline__ float8 lerp4p(float8 a, float8 b, float t) { return {lerp4p(a.lo, b.lo, t), lerp4p(a.hi, b.hi, t)}; }
+// streaming stores of one output unit
+__device__ __forceinline__ uint32_t bf16x2_rn(float lo, float hi) {
+  const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+  return *reinterpret_cast<const uint32_t*>(&h);
+}
+__device__ __forceinline__ void st_unit(float4* p, float4 v) { stg_cs_f4(p, v); }
+__device__ __forceinline__ void st_unit(float8* p, float8 v) {
+  stg_cs_f4(&p->lo, v.lo);
+  stg_cs_f4(&p->hi, v.hi);
+}
+__device__ __forceinline__ void st_unit(bf16x4* p, float4 v) {
+  __stcs(reinterpret_cast<uint2*>(p), make_uint2(bf16x2_rn(v.x, v.y), bf16x2_rn(v.z, v.w)));
+}
+__device__ __forceinline__ void st_unit(bf16x8* p, float8 v) {
+  __stcs(reinterpret_cast<uint4*>(p), make_uint4(bf16x2_rn(v.lo.x, v.lo.y), bf16x2_rn(v.lo.z, v.lo.w),
+                                                 bf16x2_rn(v.hi.x, v.hi.y), bf16x2_rn(v.hi.z, v.hi.w)));
+}
+
 // One entry of a CTA's bin table: level assignment + crop_and_resize grid of ROI `roi`, sampled at bin (y, x) ->
-// base pointer | flag, the four tap offsets (16-byte units) and the two lerp weights.
+// base pointer | flag, the four tap offsets (16-byte units, D4 of them per pixel) and the two lerp weights.
+template <typename TMap>
 __device__ __forceinline__ void bin_table_entry(const RoiSource& src, int64_t roi, int32_t y, int32_t x, bool first_bin,
                                                 int32_t ph, int32_t pw, int32_t D4, int32_t* __restrict__ level_out,
                                                 BinTaps* tp_out, BinInfo* bi_out) {
+  constexpr int64_t kUnitElems = 16 / sizeof(TMap);
   float4 box;
   RoiMeta m;
   uintptr_t flag = kBinSample;
@@ -170,7 +244,7 @@ __device__ __forceinline__ void bin_table_entry(const RoiSource& src, int64_t ro
     const int32_t l = level - src.min_level;
     m.H = src.lt.H[l];
     m.W = src.lt.W[l];
-    m.base = src.lt.ptr[l] + (roi / src.rois_per_image) * ((int64_t)m.H * m.W * D4 * 4);
+    m.base = static_cast<const TMap*>(src.lt.ptr[l]) + (roi / src.rois_per_image) * ((int64_t)m.H * m.W * D4 * kUnitElems);
     if (level_out && first_bin) level_out[roi] = level;
   } else {
     int32_t b;
@@ -185,7 +259,7 @@ __device__ __forceinline__ void bin_table_entry(const RoiSource& src, int64_t ro
     m.H = src.lt.H[0];
     m.W = src.lt.W[0];
     if (b >= 0 && b < src.batch) {
-      m.base = src.lt.ptr[0] + (int64_t)b * ((int64_t)m.H * m.W * D4 * 4);
+      m.base = static_cast<const TMap*>(src.lt.ptr[0]) + (int64_t)b * ((int64_t)m.H * m.W * D4 * kUnitElems);
     } else {  // box_ind out of range: TF skips the crop, the output rows are left untouched
       m.base = src.lt.ptr[0];
       flag = kBinSkip;
@@ -219,10 +293,15 @@ __device__ __forceinline__ void bin_table_entry(const RoiSource& src, int64_t ro
   *bi_out = bi;
 }
 
-template <int BINS, int UNROLL, bool POW2, bool ORDERED>
-__global__ void __launch_bounds__(kBinThreads, 1)
-crop_bins_kernel(RoiSource src, int64_t total_bins, int32_t bins_per_roi, int32_t ph, int32_t pw, int32_t D4,
-                 int32_t lgD4, float extrap, float4* __restrict__ out, int32_t* __restrict__ level_out) {
+// D4: 16-byte units per pixel (D / 4 fp32 or D / 8 bf16 channels); `out` is addressed in the same units
+template <typename TMap, typename TOut, int BINS, int UNROLL, bool POW2, bool ORDERED>
+__device__ __forceinline__ void crop_bins_body(const RoiSource& src, int64_t total_bins, int32_t bins_per_roi, int32_t ph,
+                                               int32_t pw, int32_t D4, int32_t lgD4, float extrap,
+                                               typename OutUnit<TMap, TOut>::T* __restrict__ out,
+                                               int32_t* __restrict__ level_out) {
+  using Raw = typename MapUnit<TMap>::Raw;
+  using Val = typename MapUnit<TMap>::Val;
+  using Out = typename OutUnit<TMap, TOut>::T;
   pdl_prologue();
   __shared__ BinTaps s_taps[BINS];
   __shared__ BinInfo s_info[BINS];
@@ -243,19 +322,20 @@ crop_bins_kernel(RoiSource src, int64_t total_bins, int32_t bins_per_roi, int32_
       s_obin[i] = (uint32_t)(roi * bins_per_roi + bin);
     }
     const int32_t y = bin / pw;
-    bin_table_entry(src, roi, y, bin - y * pw, bin == 0 && valid, ph, pw, D4, valid ? level_out : nullptr, &s_taps[i], &s_info[i]);
+    bin_table_entry<TMap>(src, roi, y, bin - y * pw, bin == 0 && valid, ph, pw, D4, valid ? level_out : nullptr, &s_taps[i],
+                          &s_info[i]);
     if (ORDERED && !valid) s_info[i].base_flag = (s_info[i].base_flag & ~(uintptr_t)3) | kBinSkip;
   }
   __syncthreads();
 
   const int32_t total = nb * D4;
-  float4* __restrict__ o = out + bin0 * D4;
-  const float4 ext4 = make_float4(extrap, extrap, extrap, extrap);
+  Out* __restrict__ o = out + bin0 * D4;
+  const Val ext4 = splat_unit<Val>(extrap);
   for (int32_t e0 = t; e0 < total; e0 += kBinThreads * UNROLL) {
-    float4 tl[UNROLL], tr[UNROLL], bl[UNROLL], br[UNROLL];
+    Raw tl[UNROLL], tr[UNROLL], bl[UNROLL], br[UNROLL];   // bf16 units are widened at the blend: half the registers
     float xl[UNROLL], yl[UNROLL];
     uint32_t fl[UNROLL];
-    float4* op[UNROLL];
+    Out* op[UNROLL];
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
       const int32_t e = min(e0 + u * kBinThreads, total - 1);  // clamped: loads are unconditional
@@ -264,26 +344,43 @@ crop_bins_kernel(RoiSource src, int64_t total_bins, int32_t bins_per_roi, int32_
       OD_DBG_IDX(bin, BINS);
       const BinTaps tp = s_taps[bin];
       const BinInfo bi = s_info[bin];
-      const float4* __restrict__ base = reinterpret_cast<const float4*>(bi.base_flag & ~(uintptr_t)15);
+      const Raw* __restrict__ base = reinterpret_cast<const Raw*>(bi.base_flag & ~(uintptr_t)15);
       fl[u] = (uint32_t)(bi.base_flag & 3u);
       xl[u] = bi.xl;
       yl[u] = bi.yl;
       op[u] = ORDERED ? out + ((int64_t)s_obin[bin] * D4 + c) : o + e;
-      tl[u] = ldg_f4(base + (tp.tl + c));
-      tr[u] = ldg_f4(base + (tp.tr + c));
-      bl[u] = ldg_f4(base + (tp.bl + c));
-      br[u] = ldg_f4(base + (tp.br + c));
+      tl[u] = __ldg(base + (tp.tl + c));
+      tr[u] = __ldg(base + (tp.tr + c));
+      bl[u] = __ldg(base + (tp.bl + c));
+      br[u] = __ldg(base + (tp.br + c));
     }
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
       const int32_t e = e0 + u * kBinThreads;
-      const float4 top = lerp4p(tl[u], tr[u], xl[u]);
-      const float4 bot = lerp4p(bl[u], br[u], xl[u]);
-      float4 v = lerp4p(top, bot, yl[u]);
+      const Val top = lerp4p(widen_unit(tl[u]), widen_unit(tr[u]), xl[u]);
+      const Val bot = lerp4p(widen_unit(bl[u]), widen_unit(br[u]), xl[u]);
+      Val v = lerp4p(top, bot, yl[u]);
       if (fl[u] == (uint32_t)kBinExtrapolate) v = ext4;
-      if (e < total && fl[u] != (uint32_t)kBinSkip) stg_cs_f4(op[u], v);
+      if (e < total && fl[u] != (uint32_t)kBinSkip) st_unit(op[u], v);
     }
   }
+}
+
+template <int BINS, int UNROLL, bool POW2, bool ORDERED>
+__global__ void __launch_bounds__(kBinThreads, 1)
+crop_bins_kernel(RoiSource src, int64_t total_bins, int32_t bins_per_roi, int32_t ph, int32_t pw, int32_t D4,
+                 int32_t lgD4, float extrap, float4* __restrict__ out, int32_t* __restrict__ level_out) {
+  crop_bins_body<float, float, BINS, UNROLL, POW2, ORDERED>(src, total_bins, bins_per_roi, ph, pw, D4, lgD4, extrap, out,
+                                                            level_out);
+}
+// bf16 maps and / or a bf16 output: the same body, an overload of the same name (the fp32 kernel above keeps its name)
+template <typename TMap, typename TOut, int BINS, int UNROLL, bool POW2, bool ORDERED>
+__global__ void __launch_bounds__(kBinThreads, 1)
+crop_bins_kernel(RoiSource src, int64_t total_bins, int32_t bins_per_roi, int32_t ph, int32_t pw, int32_t D4,
+                 int32_t lgD4, float extrap, typename OutUnit<TMap, TOut>::T* __restrict__ out,
+                 int32_t* __restrict__ level_out) {
+  crop_bins_body<TMap, TOut, BINS, UNROLL, POW2, ORDERED>(src, total_bins, bins_per_roi, ph, pw, D4, lgD4, extrap, out,
+                                                          level_out);
 }
 
 // ----------------------------------------------------------------------------- roi_order_kernel
@@ -395,14 +492,15 @@ constexpr int kRowsMinPool = 10;                // smaller pools leave too few c
 constexpr int kRowsEntries = 32;                // outstanding ring entries (one feature row each)
 constexpr int kRowsPlans = 3;                   // plans in flight
 constexpr int kRowsD4 = 64;                     // D = 256 floats = 64 quads = 1 KiB per pixel
-constexpr uint32_t kRowsPixelBytes = 1024;
+constexpr uint32_t kRowsPixelBytes = 1024;      // fp32 maps; a bf16 pixel is 512 bytes (32 units of 8 channels)
+template <typename TMap> constexpr int kRowsUnits = 4 * kRowsD4 / MapUnit<TMap>::kCh;   // 16-byte units per pixel
 // Ring size: 176 KiB. The kernel alone is ~1 % faster with everything an SM has (221 KiB), but leaving ~45 KiB lets the
 // small CTAs of concurrently running kernels (the other steps' proposal front and 7x7 ROIAlign) become resident next to
 // it, which is worth 8 % of whole-step throughput (profiles/r2_roialign.md).
 constexpr uint32_t kRowsRingBytes = 176 * 1024;
 // A row may have to skip the tail of the ring (it never straddles the end): row + skipped tail must fit an EMPTY ring,
 // which holds for every head position only if a row is at most half the ring. A row holds the distinct columns of one
-// ROI, at most two per x sample.
+// ROI, at most two per x sample. (The fp32 pixel is the larger one.)
 static_assert(2u * (2 * kRowsMaxWidth) * kRowsPixelBytes <= kRowsRingBytes, "a ring row can exceed half the ring");
 
 struct RowsPlan {
@@ -416,9 +514,9 @@ struct RowsPlan {
   int32_t run_col[kRowsMaxPool], run_rank[kRowsMaxPool], run_len[kRowsMaxPool];
   int32_t nr, ncols, nruns, mode;
   int32_t W;
-  uint32_t row_bytes;                           // ncols KiB: one ring entry
+  uint32_t row_bytes;                           // ncols pixels: one ring entry
   int64_t roi;
-  const float* base;
+  const void* base;
 };
 // ring: every bin of the ROI has four valid taps and the grid steps are non-negative (the streaming fast path);
 // flat: anything else (extrapolated bins, flipped / NaN boxes) - per-bin direct loads;
@@ -434,6 +532,7 @@ struct RowsShared {
 
 // geometry of one ROI (level assignment, image base, sampling grid) from its preloaded box (and batch index in
 // crop_and_resize mode); returns the kBin* flag
+template <typename TMap>
 __device__ __forceinline__ uintptr_t roi_geometry(const RoiSource& src, int64_t roi, float4 box, int32_t b, int32_t ph,
                                                   int32_t pw, RoiMeta& m, int32_t* level) {
   uintptr_t flag = kBinSample;
@@ -443,13 +542,14 @@ __device__ __forceinline__ uintptr_t roi_geometry(const RoiSource& src, int64_t 
     const int32_t l = *level - src.min_level;
     m.H = src.lt.H[l];
     m.W = src.lt.W[l];
-    m.base = src.lt.ptr[l] + (int64_t)((uint32_t)roi / (uint32_t)src.rois_per_image) * ((int64_t)m.H * m.W * D);
+    m.base = static_cast<const TMap*>(src.lt.ptr[l]) + (int64_t)((uint32_t)roi / (uint32_t)src.rois_per_image) * ((int64_t)m.H * m.W * D);
   } else {
     m.H = src.lt.H[0];
     m.W = src.lt.W[0];
-    m.base = src.lt.ptr[0];
-    if (b >= 0 && b < src.batch) m.base += (int64_t)b * ((int64_t)m.H * m.W * D);
+    const TMap* base = static_cast<const TMap*>(src.lt.ptr[0]);
+    if (b >= 0 && b < src.batch) base += (int64_t)b * ((int64_t)m.H * m.W * D);
     else flag = kBinSkip;
+    m.base = base;
   }
   fill_grid(m, box, ph, pw);
   return flag;
@@ -460,11 +560,12 @@ __device__ __forceinline__ uintptr_t roi_geometry(const RoiSource& src, int64_t 
 // hi - lo is 0 or 1, so a tap is NEW (not seen before) exactly when it differs from both taps of the previous
 // sample; first-use order is ascending order, the rank of a new tap is the number of new taps before it (two
 // ballots and a popcount) and a repeated tap is the largest or second largest value seen so far.
+template <typename TMap>
 __device__ __forceinline__ void rows_make_plan(const RoiSource& src, int64_t roi, float4 box, int32_t bidx, int32_t ph,
                                                int32_t pw, int32_t lane, RowsPlan& P, RowsShared& S, int32_t* level_out) {
   RoiMeta m;
   int32_t level = 0;
-  const uintptr_t flag = roi_geometry(src, roi, box, bidx, ph, pw, m, &level);
+  const uintptr_t flag = roi_geometry<TMap>(src, roi, box, bidx, ph, pw, m, &level);
   const bool mono = (m.hs >= 0.0f) && (m.ws >= 0.0f);
   const int32_t half = lane >> 4, i = lane & 15;
   const int32_t n = half ? pw : ph;
@@ -541,7 +642,7 @@ __device__ __forceinline__ void rows_make_plan(const RoiSource& src, int64_t roi
       P.nr = nr;
       P.ncols = nc;
       P.nruns = __popc(sm);
-      P.row_bytes = (uint32_t)nc * kRowsPixelBytes;
+      P.row_bytes = (uint32_t)nc * (16u * kRowsUnits<TMap>);
     }
   }
   if (lane == 0) {
@@ -557,9 +658,19 @@ __device__ __forceinline__ void rows_make_plan(const RoiSource& src, int64_t roi
 // counter[0]: next ROI ticket, counter[1]: CTAs that have drawn their last ticket. Both are zero between launches: the
 // last CTA to finish resets them (the workspace is zero-initialised once by its owner).
 // Warps 0 .. pw-1 are the consumers (warp = x bin), warp pw the issuer, warp pw+1 the planner.
-__global__ void __launch_bounds__(kRowsThreads, 1)
-crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, float extrap, float4* __restrict__ out,
-                 int32_t* __restrict__ level_out, unsigned int* __restrict__ counter) {
+// `out` is addressed in 16-byte map units (OutUnit): a pixel is kRowsUnits<TMap> of them.
+template <typename TMap, typename TOut>
+__device__ __forceinline__ void crop_rows_body(const RoiSource& src, int64_t n_rois, int32_t ph, int32_t pw, float extrap,
+                                               typename OutUnit<TMap, TOut>::T* __restrict__ out,
+                                               int32_t* __restrict__ level_out, unsigned int* __restrict__ counter) {
+  using Raw = typename MapUnit<TMap>::Raw;
+  using Val = typename MapUnit<TMap>::Val;
+  using Out = typename OutUnit<TMap, TOut>::T;
+  constexpr int kPixUnits = kRowsUnits<TMap>;             // 64 fp32 quads or 32 bf16 octets
+  constexpr int kPixShift = kPixUnits == 64 ? 6 : 5;
+  static_assert((1 << kPixShift) == kPixUnits, "a pixel is 64 or 32 units");
+  constexpr int kLaneUnits = kPixUnits / 32;              // units per consumer lane and pixel: 8 channels either way
+  constexpr uint32_t kPixBytes = 16u * kPixUnits;
   pdl_prologue();
   extern __shared__ __align__(128) unsigned char s_ring[];
   __shared__ RowsShared S;
@@ -638,7 +749,7 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, float ex
         }
         __syncwarp();
       } else {
-        rows_make_plan(src, roi, box, bi, ph, pw, lane, P, S, level_out);
+        rows_make_plan<TMap>(src, roi, box, bi, ph, pw, lane, P, S, level_out);
       }
       if (lane == 0) mbar_arrive(&S.plan_full[ps]);
       if (++ps == kRowsPlans) {
@@ -668,13 +779,13 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, float ex
       if (mode == kRowsRing) {
         const int32_t nr = P.nr, nruns = P.nruns;
         const uint32_t bytes = P.row_bytes;
-        const char* __restrict__ gbase = reinterpret_cast<const char*>(P.base);
-        const size_t row_pitch = (size_t)P.W * kRowsPixelBytes;
+        const char* __restrict__ gbase = static_cast<const char*>(P.base);
+        const size_t row_pitch = (size_t)P.W * kPixBytes;
         // this lane's column run (nruns <= 16): smem offset inside the row, global offset inside the feature row, bytes
         const int32_t jr = lane < nruns ? lane : 0;
-        const uint32_t run_dst = (uint32_t)P.run_rank[jr] * kRowsPixelBytes;
-        const size_t run_src = (size_t)P.run_col[jr] * kRowsPixelBytes;
-        const uint32_t run_bytes = (uint32_t)P.run_len[jr] * kRowsPixelBytes;
+        const uint32_t run_dst = (uint32_t)P.run_rank[jr] * kPixBytes;
+        const size_t run_src = (size_t)P.run_col[jr] * kPixBytes;
+        const uint32_t run_bytes = (uint32_t)P.run_len[jr] * kPixBytes;
         int32_t my_row = lane < nr ? P.rows[lane] : 0;           // rank k's feature row lives on lane k (nr <= 32)
         for (int32_t k = 0; k < nr; ++k) {
           const bool wrap = head + bytes > kRowsRingBytes;        // the tail a wrapped row skips counts as part of it
@@ -715,9 +826,10 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, float ex
   }
 
   // -------------------------------------------------------------------- consumers
-  // warp = x bin, lane = channel quads `lane` and `lane + 32`: one output pixel (1 KiB) per warp and output row.
+  // warp = x bin, lane = channel quads `lane` and `lane + 32` (fp32 maps) or channel octet `lane` (bf16 maps, one 16-byte
+  // LDS per tap pixel): one output pixel per warp and output row.
   const int32_t x = warp;
-  const float4 ext4 = make_float4(extrap, extrap, extrap, extrap);
+  const Val ext4 = splat_unit<Val>(extrap);
   int32_t e_idx = 0;
   uint32_t e_phase = 0, c_head = 0;              // ring entry, its phase, and the issuer's head replayed locally
   for (;;) {
@@ -725,27 +837,28 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, float ex
     const RowsPlan& P = S.plan[ps];
     const int32_t mode = P.mode;
     if (mode == kRowsDone) break;
-    float4* __restrict__ o = out + P.roi * ((int64_t)ph * pw * kRowsD4);
+    Out* __restrict__ o = out + P.roi * ((int64_t)ph * pw * kPixUnits);
     if (mode == kRowsRing) {
-      // Column ranks -> float4 index inside a ring row (+ the channel quad).
-      const int32_t xcl = P.x_cl[x] * kRowsD4 + lane, xcr = P.x_cr[x] * kRowsD4 + lane;
+      // Column ranks -> unit index inside a ring row (+ the lane's channel unit).
+      const int32_t xcl = P.x_cl[x] * kPixUnits + lane, xcr = P.x_cr[x] * kPixUnits + lane;
       const float xl = P.x_lerp[x];
       const int32_t nr = P.nr;
       const uint32_t row_bytes = P.row_bytes;
       // Rank-major walk: the y's whose top row has rank k are contiguous (P.yfirst), their bottom row is rank k or k+1.
       // Rows alternate between RA (even ranks) and RB (odd ranks). bottom - top is recomputed per y: a group holds 1.2 y's
       // on average, caching the difference would only cost registers.
-      float4 RA[2], RB[2];
-      RA[0] = RA[1] = RB[0] = RB[1] = ext4;
+      Val RA[kLaneUnits], RB[kLaneUnits];
+      for (int i = 0; i < kLaneUnits; ++i) RA[i] = RB[i] = ext4;
 #define OD_ROWS_LOAD(V)                                                                              \
   do {                                                                                               \
     const uint32_t off_ = (c_head + row_bytes > kRowsRingBytes) ? 0u : c_head;                       \
     c_head = off_ + row_bytes;                                                                       \
-    OD_DBG_ASSERT(c_head <= kRowsRingBytes && (uint32_t)(xcr + 32) * 16u < row_bytes && xcl <= xcr, "ring read outside the row"); \
+    OD_DBG_ASSERT(c_head <= kRowsRingBytes && (uint32_t)(xcr + 32 * (kLaneUnits - 1)) * 16u < row_bytes && xcl <= xcr, \
+                  "ring read outside the row");                                                      \
     mbar_wait(&S.full[e_idx], e_phase);                                                              \
-    const float4* rowp = reinterpret_cast<const float4*>(s_ring + off_);                             \
-    _Pragma("unroll") for (int i = 0; i < 2; ++i) {                                                  \
-      const float4 l_ = rowp[xcl + 32 * i], r_ = rowp[xcr + 32 * i];                                 \
+    const Raw* rowp = reinterpret_cast<const Raw*>(s_ring + off_);                                   \
+    _Pragma("unroll") for (int i = 0; i < kLaneUnits; ++i) {                                         \
+      const Val l_ = widen_unit(rowp[xcl + 32 * i]), r_ = widen_unit(rowp[xcr + 32 * i]);            \
       V[i] = axpy4p(l_, sub4p(r_, l_), xl);                                                          \
     }                                                                                                \
     __syncwarp();                                                                                    \
@@ -765,22 +878,22 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, float ex
     _Pragma("unroll 1") while (y < yend) {                                                           \
       const int2 nxt_ = P.ytab[y + 2];      /* two rows ahead: the read is off the critical path */    \
       const float yl = __int_as_float(ent.x);                                                        \
-      float4 v_[2];                                                                                  \
+      Val v_[kLaneUnits];                                                                            \
       if (ent.y) {                    /* top row == bottom row: (top - top) * yl, as the reference */ \
-        _Pragma("unroll") for (int i = 0; i < 2; ++i) v_[i] = axpy4p(CUR[i], sub4p(CUR[i], CUR[i]), yl); \
+        _Pragma("unroll") for (int i = 0; i < kLaneUnits; ++i) v_[i] = axpy4p(CUR[i], sub4p(CUR[i], CUR[i]), yl); \
       } else {                                                                                       \
-        _Pragma("unroll") for (int i = 0; i < 2; ++i) v_[i] = axpy4p(CUR[i], sub4p(NXT[i], CUR[i]), yl); \
+        _Pragma("unroll") for (int i = 0; i < kLaneUnits; ++i) v_[i] = axpy4p(CUR[i], sub4p(NXT[i], CUR[i]), yl); \
       }                                                                                              \
-      _Pragma("unroll") for (int i = 0; i < 2; ++i) stg_cs_f4(orow + lane + 32 * i, v_[i]);          \
+      _Pragma("unroll") for (int i = 0; i < kLaneUnits; ++i) st_unit(orow + lane + 32 * i, v_[i]);   \
       ent = ent1;                                                                                    \
       ent1 = nxt_;                                                                                   \
       ++y;                                                                                           \
-      orow += pw * kRowsD4;                                                                          \
+      orow += pw * kPixUnits;                                                                        \
     }                                                                                                \
     if (!more) break;                                                                                \
     ++k;                                                                                             \
   }
-      float4* __restrict__ orow = o + x * kRowsD4;    // this warp's pixel of output row 0
+      Out* __restrict__ orow = o + x * kPixUnits;     // this warp's pixel of output row 0
       int2 ent = P.ytab[0], ent1 = P.ytab[1];
       int32_t y = 0, k = 0;
       OD_ROWS_LOAD(RA);
@@ -791,25 +904,25 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, float ex
 #undef OD_ROWS_LOAD
 #undef OD_ROWS_GROUP
     } else if (mode == kRowsFlat) {   // per-bin path: 4 direct loads per output quad
-      const float4* __restrict__ base = reinterpret_cast<const float4*>(P.base);
+      const Raw* __restrict__ base = static_cast<const Raw*>(P.base);
       const uint32_t W = (uint32_t)P.W;
-      const int32_t total = ph * pw * kRowsD4;
+      const int32_t total = ph * pw * kPixUnits;
       for (int32_t e = t; e < total; e += n_cons) {
-        const int32_t bin = e >> 6;
-        const uint32_t c = (uint32_t)(e & 63);
+        const int32_t bin = e >> kPixShift;
+        const uint32_t c = (uint32_t)(e & (kPixUnits - 1));
         const int32_t y = bin / pw, xb = bin - y * pw;
-        float4 v = ext4;
+        Val v = ext4;
         if (P.y_ok[y] && P.x_ok[xb]) {
           const uint32_t top = (uint32_t)P.y_top[y], bot = (uint32_t)P.y_bot[y];
           const uint32_t left = (uint32_t)P.x_left[xb], right = (uint32_t)P.x_right[xb];
-          const float4 tl = ldg_f4(base + ((top * W + left) * kRowsD4 + c));
-          const float4 tr = ldg_f4(base + ((top * W + right) * kRowsD4 + c));
-          const float4 bl = ldg_f4(base + ((bot * W + left) * kRowsD4 + c));
-          const float4 br = ldg_f4(base + ((bot * W + right) * kRowsD4 + c));
+          const Val tl = ldg_unit(base + ((top * W + left) * kPixUnits + c));
+          const Val tr = ldg_unit(base + ((top * W + right) * kPixUnits + c));
+          const Val bl = ldg_unit(base + ((bot * W + left) * kPixUnits + c));
+          const Val br = ldg_unit(base + ((bot * W + right) * kPixUnits + c));
           const float xl = P.x_lerp[xb];
           v = lerp4p(lerp4p(tl, tr, xl), lerp4p(bl, br, xl), P.y_lerp[y]);
         }
-        stg_cs_f4(o + e, v);
+        st_unit(o + e, v);
       }
     }
     __syncwarp();
@@ -819,6 +932,20 @@ crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, float ex
       pphase ^= 1u;
     }
   }
+}
+
+__global__ void __launch_bounds__(kRowsThreads, 1)
+crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, float extrap, float4* __restrict__ out,
+                 int32_t* __restrict__ level_out, unsigned int* __restrict__ counter) {
+  crop_rows_body<float, float>(src, n_rois, ph, pw, extrap, out, level_out, counter);
+}
+// bf16 maps and / or a bf16 output: the same body, an overload of the same name (the fp32 kernel above keeps its name)
+template <typename TMap, typename TOut>
+__global__ void __launch_bounds__(kRowsThreads, 1)
+crop_rows_kernel(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, float extrap,
+                 typename OutUnit<TMap, TOut>::T* __restrict__ out, int32_t* __restrict__ level_out,
+                 unsigned int* __restrict__ counter) {
+  crop_rows_body<TMap, TOut>(src, n_rois, ph, pw, extrap, out, level_out, counter);
 }
 
 // FasterRCNN roi_pool (fastrcnn.py:22-70): crop_and_resize to (2*oh) x (2*ow) fused with max_pool 2x2 / stride 2.
@@ -840,7 +967,7 @@ crop_pool_bins_kernel(RoiSource src, int64_t total_bins, int32_t oh, int32_t ow,
     const int64_t roi = fb / bins_per_roi;
     const int32_t ob = (int32_t)(fb - roi * bins_per_roi);
     const int32_t oy = ob / ow, ox = ob - oy * ow;
-    bin_table_entry(src, roi, 2 * oy + ((i >> 1) & 1), 2 * ox + (i & 1), false, 2 * oh, 2 * ow, D4, nullptr, &s_taps[i], &s_info[i]);
+    bin_table_entry<float>(src, roi, 2 * oy + ((i >> 1) & 1), 2 * ox + (i & 1), false, 2 * oh, 2 * ow, D4, nullptr, &s_taps[i], &s_info[i]);
   }
   __syncthreads();
   const int32_t total = nb * D4;
@@ -885,24 +1012,42 @@ static bool crop_rows_serves(const RoiSource& src, int64_t n_rois, int32_t ph, i
   return n_rois + 4096 <= 0x7FFFFFFFll;
 }
 
+// The kernels of one (maps, pooled) dtype pair: the fp32 kernels for fp32 -> fp32, their bf16 overloads otherwise.
+template <typename TMap, typename TOut>
+constexpr bool kFp32Pair = std::is_same<TMap, float>::value && std::is_same<TOut, float>::value;
+template <typename TMap, typename TOut>
+static auto rows_kernel() {
+  if constexpr (kFp32Pair<TMap, TOut>)
+    return static_cast<void (*)(RoiSource, int64_t, int32_t, int32_t, float, float4*, int32_t*, unsigned int*)>(crop_rows_kernel);
+  else
+    return &crop_rows_kernel<TMap, TOut>;
+}
+template <typename TMap, typename TOut, int BINS, int UNROLL, bool POW2, bool ORDERED>
+static auto bins_kernel() {
+  if constexpr (kFp32Pair<TMap, TOut>) return &crop_bins_kernel<BINS, UNROLL, POW2, ORDERED>;
+  else return &crop_bins_kernel<TMap, TOut, BINS, UNROLL, POW2, ORDERED>;
+}
+
 // returns OD_OK after launching, or 1 when the shape is not served by this kernel (caller falls back to crop_bins).
 // `counter`: two zeroed uint32 in the caller's workspace (dynamic ROI scheduling) or NULL (static round robin).
-static int launch_crop_rows(const RoiSource& src, int64_t n_rois, int32_t ph, int32_t pw, int32_t D, float extrap, float* out,
+template <typename TMap, typename TOut>
+static int launch_crop_rows(const RoiSource& src, int64_t n_rois, int32_t ph, int32_t pw, int32_t D, float extrap, void* out,
                             int32_t* level_out, unsigned int* counter, cudaStream_t st) {
   if (!crop_rows_serves(src, n_rois, ph, pw, D)) return 1;
-  static bool configured[64] = {false};    // dynamic shared memory opted in, per device
+  static bool configured[64] = {false};    // dynamic shared memory opted in, per device (and dtype pair)
   static int sms[64] = {0};
+  const auto kernel = rows_kernel<TMap, TOut>();
   int dev = 0;
   OD_CUDA(cudaGetDevice(&dev));
   if (dev < 0 || dev >= 64) OD_FAIL(OD_ERR_DEVICE, "device index %d not supported", dev);
   if (!configured[dev]) {
-    OD_CUDA(cudaFuncSetAttribute(crop_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRowsRingBytes));
+    OD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRowsRingBytes));
     configured[dev] = true;
   }
   if (!sms[dev]) OD_CUDA(cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev));
   const int64_t grid = n_rois < (int64_t)sms[dev] ? n_rois : (int64_t)sms[dev];
-  OD_CUDA(launch_pdl(crop_rows_kernel, dim3((unsigned)grid), dim3((unsigned)(32 * pw + 64)), (size_t)kRowsRingBytes, st, src,
-                     n_rois, ph, pw, extrap, reinterpret_cast<float4*>(out), level_out, counter));
+  OD_CUDA(launch_pdl(kernel, dim3((unsigned)grid), dim3((unsigned)(32 * pw + 64)), (size_t)kRowsRingBytes, st, src,
+                     n_rois, ph, pw, extrap, static_cast<typename OutUnit<TMap, TOut>::T*>(out), level_out, counter));
   OD_LAUNCH_CHECK("crop_rows_kernel");
   return OD_OK;
 }
@@ -916,11 +1061,14 @@ static int launch_roi_order(const RoiSource& src, int32_t* order_buf, cudaStream
 
 // `order_buf`: scratch for the pre-pass (or NULL); `order_in`: an order the caller already has (od_roi_processing_order),
 // which saves the pre-pass - e.g. the 7x7 and the 14x14 pooling of one step walk the same ROIs.
+// D: channels; D4: 16-byte units per pixel.
+template <typename TMap, typename TOut>
 static int launch_crop_bins(RoiSource src, int64_t n_rois, int32_t ph, int32_t pw, int32_t D, float extrap,
-                            float* out, int32_t* level_out, cudaStream_t st, unsigned int* counter = nullptr,
+                            void* out, int32_t* level_out, cudaStream_t st, unsigned int* counter = nullptr,
                             int32_t* order_buf = nullptr, const int32_t* order_in = nullptr) {
+  using Out = typename OutUnit<TMap, TOut>::T;
   if (n_rois == 0) return OD_OK;
-  const int32_t D4 = D / 4;
+  const int32_t D4 = D / MapUnit<TMap>::kCh;
   // processing order (PyramidROIAlign with a sized workspace, enough ROIs for the order to matter). Measured: +3 % on the
   // persistent 14x14 kernel. For the flat 7x7 kernel the launch itself gets ~2 us faster but its pre-pass adds more than
   // that to a stand-alone call; with several steps in flight (the throughput case) that latency is hidden and the order is
@@ -940,7 +1088,7 @@ static int launch_crop_bins(RoiSource src, int64_t n_rois, int32_t ph, int32_t p
     if ((int64_t)src.lt.H[l] * src.lt.W[l] * D4 > 0xFFFFFFFFll)
       OD_FAIL(OD_ERR_PARAM, "one image of level %d exceeds 2^32 16-byte units", l);
   {
-    const int rc = launch_crop_rows(src, n_rois, ph, pw, D, extrap, out, level_out, counter, st);
+    const int rc = launch_crop_rows<TMap, TOut>(src, n_rois, ph, pw, D, extrap, out, level_out, counter, st);
     if (rc != 1) return rc;
   }
   int32_t lg = -1;
@@ -948,31 +1096,48 @@ static int launch_crop_bins(RoiSource src, int64_t n_rois, int32_t ph, int32_t p
     lg = 0;
     while ((1 << lg) < D4) ++lg;
   }
+  // The tier is chosen on 16-byte units per pixel, i.e. on bytes per pixel, not on channels: bf16 maps with D = 64 (8
+  // units) take the 512-bin kernel like fp32 maps with D = 32, while fp32 maps with D = 64 (16 units) take the 32-bin one.
   if (lg >= 0 && D4 >= 16) {
     if ((int64_t)64 * D4 > 0x7FFFFFFFll) OD_FAIL(OD_ERR_PARAM, "depth %d too large", D);
     const int64_t grid = (total_bins + kBinBins - 1) / kBinBins;
     if (grid > 0x7FFFFFFFll) OD_FAIL(OD_ERR_PARAM, "too many bins: %lld", (long long)total_bins);
     if (src.order)
-      OD_CUDA(launch_pdl(crop_bins_kernel<kBinBins, kBinUnroll, true, true>, dim3((unsigned)grid), dim3(kBinThreads), 0, st,
-          src, total_bins, (int32_t)bins_per_roi, ph, pw, D4, lg, extrap, reinterpret_cast<float4*>(out), level_out));
+      OD_CUDA(launch_pdl(bins_kernel<TMap, TOut, kBinBins, kBinUnroll, true, true>(), dim3((unsigned)grid), dim3(kBinThreads), 0,
+          st, src, total_bins, (int32_t)bins_per_roi, ph, pw, D4, lg, extrap, static_cast<Out*>(out), level_out));
     else
-      OD_CUDA(launch_pdl(crop_bins_kernel<kBinBins, kBinUnroll, true, false>, dim3((unsigned)grid), dim3(kBinThreads), 0, st,
-          src, total_bins, (int32_t)bins_per_roi, ph, pw, D4, lg, extrap, reinterpret_cast<float4*>(out), level_out));
+      OD_CUDA(launch_pdl(bins_kernel<TMap, TOut, kBinBins, kBinUnroll, true, false>(), dim3((unsigned)grid), dim3(kBinThreads), 0,
+          st, src, total_bins, (int32_t)bins_per_roi, ph, pw, D4, lg, extrap, static_cast<Out*>(out), level_out));
   } else {
     // thin or non-power-of-two depth: more bins per CTA so that the table build is amortised
     constexpr int BINS = 512;
     if ((int64_t)BINS * D4 > 0x7FFFFFFFll) OD_FAIL(OD_ERR_PARAM, "depth %d too large", D);
     const int64_t grid = (total_bins + BINS - 1) / BINS;
     if (grid > 0x7FFFFFFFll) OD_FAIL(OD_ERR_PARAM, "too many bins: %lld", (long long)total_bins);
-    if (lg >= 0)
-      crop_bins_kernel<BINS, 2, true, false><<<(unsigned)grid, kBinThreads, 0, st>>>(src, total_bins, (int32_t)bins_per_roi, ph, pw,
-                                                                           D4, lg, extrap, reinterpret_cast<float4*>(out), level_out);
-    else
-      crop_bins_kernel<BINS, 2, false, false><<<(unsigned)grid, kBinThreads, 0, st>>>(src, total_bins, (int32_t)bins_per_roi, ph, pw,
-                                                                            D4, lg, extrap, reinterpret_cast<float4*>(out), level_out);
+    const auto kernel = lg >= 0 ? bins_kernel<TMap, TOut, BINS, 2, true, false>() : bins_kernel<TMap, TOut, BINS, 2, false, false>();
+    kernel<<<(unsigned)grid, kBinThreads, 0, st>>>(src, total_bins, (int32_t)bins_per_roi, ph, pw, D4, lg, extrap,
+                                                   static_cast<Out*>(out), level_out);
   }
   OD_LAUNCH_CHECK("crop_bins_kernel");
   return OD_OK;
+}
+
+// The dtype a ROIAlign map or output tensor is checked against: BF16 for a bfloat16 tensor, F32 for anything else, which
+// check_tensor then refuses unless it is fp32 (float16 included).
+static DType map_or_out_dtype(const DLTensor* t) {
+  return (t && t->dtype.code == kDLBfloat && t->dtype.bits == 16 && t->dtype.lanes == 1) ? BF16 : F32;
+}
+// With a bf16 map or output a pixel must be whole 16-byte units of 8 channels.
+static int check_bf16_depth(DType map_dt, DType out_dt, int64_t D) {
+  if ((map_dt == BF16 || out_dt == BF16) && D % 8)
+    OD_FAIL(OD_ERR_SHAPE, "depth %lld must be a multiple of 8 with bfloat16 maps or output", (long long)D);
+  return OD_OK;
+}
+template <typename... Args>
+static int launch_crop(DType map_dt, DType out_dt, Args... args) {
+  if (map_dt == BF16)
+    return out_dt == BF16 ? launch_crop_bins<__nv_bfloat16, __nv_bfloat16>(args...) : launch_crop_bins<__nv_bfloat16, float>(args...);
+  return out_dt == BF16 ? launch_crop_bins<float, __nv_bfloat16>(args...) : launch_crop_bins<float, float>(args...);
 }
 
 }  // namespace od
@@ -1030,16 +1195,19 @@ int od_pyramid_roi_align_forward_ordered(const DLTensor* const* fmaps, int32_t n
   const int64_t B = rois->shape[0], N = rois->shape[1];
   LevelTable lt;
   int64_t D = kAny;   // that of the first level
+  const DType map_dt = map_or_out_dtype(fmaps[0]);   // every level must have the first level's dtype
   for (int l = 0; l < num_levels; ++l) {
-    OD_CHECK(check_tensor(fmaps[l], "fmaps[l]", F32, {B, kAny, kAny, D}, 16, scope));
+    OD_CHECK(check_tensor(fmaps[l], "fmaps[l]", map_dt, {B, kAny, kAny, D}, 16, scope));
     D = fmaps[l]->shape[3];
-    lt.ptr[l] = dptr<float>(fmaps[l]);
+    lt.ptr[l] = dptr<char>(fmaps[l]);
     lt.H[l] = (int32_t)fmaps[l]->shape[1];
     lt.W[l] = (int32_t)fmaps[l]->shape[2];
   }
   if (D % 4) OD_FAIL(OD_ERR_SHAPE, "depth %lld must be a multiple of 4", (long long)D);
-  if (pooled && pooled->ndim == 5) OD_CHECK(check_tensor(pooled, "pooled", F32, {1, B * N, pool_h, pool_w, D}, 16, scope));
-  else OD_CHECK(check_tensor(pooled, "pooled", F32, {B * N, pool_h, pool_w, D}, 16, scope));
+  const DType out_dt = map_or_out_dtype(pooled);
+  if (pooled && pooled->ndim == 5) OD_CHECK(check_tensor(pooled, "pooled", out_dt, {1, B * N, pool_h, pool_w, D}, 16, scope));
+  else OD_CHECK(check_tensor(pooled, "pooled", out_dt, {B * N, pool_h, pool_w, D}, 16, scope));
+  OD_CHECK(check_bf16_depth(map_dt, out_dt, D));
   OD_CHECK(check_opt_tensor(roi_level, "roi_level", I32, {B, N}, 4, scope));
   const int64_t total = B * N;
   if (total == 0) return OD_OK;
@@ -1060,8 +1228,8 @@ int od_pyramid_roi_align_forward_ordered(const DLTensor* const* fmaps, int32_t n
   int32_t* order_buf = (ws && ws_bytes >= od_pyramid_roi_align_workspace_bytes_n(total))
                            ? reinterpret_cast<int32_t*>(static_cast<char*>(ws) + 256) : nullptr;
   OD_CHECK(check_opt_tensor(order, "order", I32, {total}, 4, scope));
-  return launch_crop_bins(src, total, pool_h, pool_w, (int32_t)D, 0.0f, dptr<float>(pooled), dptr<int32_t>(roi_level), st,
-                          static_cast<unsigned int*>(ws), order_buf, dptr<int32_t>(order));
+  return launch_crop(map_dt, out_dt, src, total, pool_h, pool_w, (int32_t)D, 0.0f, dptr<void>(pooled), dptr<int32_t>(roi_level),
+                     st, static_cast<unsigned int*>(ws), order_buf, dptr<int32_t>(order));
 }
 
 int od_pyramid_roi_align_forward(const DLTensor* const* fmaps, int32_t num_levels, int32_t min_level,
@@ -1076,24 +1244,26 @@ int od_crop_and_resize(const DLTensor* image, const DLTensor* boxes, const DLTen
                        int32_t crop_w, float extrapolation_value, DLTensor* out, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   DeviceScope scope;
-  OD_CHECK(check_tensor(image, "image", F32, {kAny, kAny, kAny, kAny}, 16, scope));
+  const DType map_dt = map_or_out_dtype(image), out_dt = map_or_out_dtype(out);
+  OD_CHECK(check_tensor(image, "image", map_dt, {kAny, kAny, kAny, kAny}, 16, scope));
   OD_CHECK(check_tensor(boxes, "boxes", F32, {kAny, 4}, 16, scope));
   const int64_t n = boxes->shape[0], D = image->shape[3];
   OD_CHECK(check_tensor(box_ind, "box_ind", I32, {n}, 4, scope));
   if (crop_h < 1 || crop_w < 1) OD_FAIL(OD_ERR_PARAM, "crop size %dx%d unsupported", crop_h, crop_w);
-  OD_CHECK(check_tensor(out, "out", F32, {n, crop_h, crop_w, D}, 16, scope));
+  OD_CHECK(check_tensor(out, "out", out_dt, {n, crop_h, crop_w, D}, 16, scope));
   if (D % 4) OD_FAIL(OD_ERR_SHAPE, "depth %lld must be a multiple of 4", (long long)D);
+  OD_CHECK(check_bf16_depth(map_dt, out_dt, D));
   if (n == 0) return OD_OK;
   RoiSource src;
   memset(&src, 0, sizeof(src));
   src.mode = 1;
   src.batch = (int32_t)image->shape[0];
-  src.lt.ptr[0] = dptr<float>(image);
+  src.lt.ptr[0] = dptr<char>(image);
   src.lt.H[0] = (int32_t)image->shape[1];
   src.lt.W[0] = (int32_t)image->shape[2];
   src.boxes = dptr<float4>(boxes);
   src.box_ind = dptr<int32_t>(box_ind);
-  return launch_crop_bins(src, n, crop_h, crop_w, (int32_t)D, extrapolation_value, dptr<float>(out), nullptr, st);
+  return launch_crop(map_dt, out_dt, src, n, crop_h, crop_w, (int32_t)D, extrapolation_value, dptr<void>(out), nullptr, st);
 }
 
 int od_roi_pool_forward(const DLTensor* feature_map, const DLTensor* proposals, float image_h, float image_w,
@@ -1112,7 +1282,7 @@ int od_roi_pool_forward(const DLTensor* feature_map, const DLTensor* proposals, 
   memset(&src, 0, sizeof(src));
   src.mode = 2;
   src.batch = (int32_t)feature_map->shape[0];
-  src.lt.ptr[0] = dptr<float>(feature_map);
+  src.lt.ptr[0] = dptr<char>(feature_map);
   src.lt.H[0] = (int32_t)feature_map->shape[1];
   src.lt.W[0] = (int32_t)feature_map->shape[2];
   src.boxes5 = dptr<float>(proposals);

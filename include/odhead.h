@@ -167,7 +167,17 @@ typedef struct od_proposal_debug {
 } od_proposal_debug;
 
 size_t od_proposal_workspace_bytes(int64_t batch, int64_t num_anchors, const od_proposal_params* p);
-/* rpn_class_probs [B,A,2] f32 (bg,fg), rpn_bbox [B,A,4] f32 (dy,dx,log dh,log dw),
+/* Head outputs in bf16. The arguments that carry a network head's output (the RPN logits and deltas here, mrcnn_bbox
+ * and mrcnn_class_probs of od_detection_forward, the predictions of the two loss entry points) are f32 or bf16
+ * (kDLBfloat, 16 bits; float16 and every other dtype are refused with OD_ERR_DTYPE), each argument on its own and
+ * every level of a level list of one dtype (a mixed list is refused with OD_ERR_DTYPE, naming the level). A bf16
+ * tensor must be aligned to the kernel's load (OD_ERR_LAYOUT otherwise): 2 bytes for a scalar, 4 for a (bg,fg) logit
+ * pair, 8 for a 4-value delta or box row. A bf16 value is widened to fp32 exactly (bits << 16: sign, NaN payload and
+ * subnormals survive; the library is built without flush-to-zero) and everything after the load is the f32 path, so
+ * every output and DEBUG tensor (all f32) equals that of the call on the widened f32 tensors bit for bit. Every other
+ * argument keeps its f32 / i32 dtype.
+ *
+ * rpn_class_probs [B,A,2] f32 (bg,fg), rpn_bbox [B,A,4] f32 or bf16 (dy,dx,log dh,log dw),
  * anchors [B,A,4] f32 normalised, or NULL with a non-NULL `spec` (anchors are then
  * regenerated in fp64 from the index inside the decode kernel).
  * proposals [B,N,4] f32, rows after the kept ones are zero. */
@@ -179,8 +189,9 @@ int od_proposal_forward(const DLTensor* rpn_class_probs, const DLTensor* rpn_bbo
 
 /* The same layer fed by the RPN head's conv outputs in their native per-level layout (SURVEY 8(f)3): no
  * [B,A,2] / [B,A,4] concatenation is materialised.
- * class_logits[l]: [B,H_l,W_l,2a] f32 NHWC ('rpn_class_raw', rpn.py:50; a anchors per location, (bg,fg) pairs),
- * bbox[l]:         [B,H_l,W_l,4a] f32 NHWC ('rpn_bbox_pred', rpn.py:63), l < num_levels.
+ * class_logits[l]: [B,H_l,W_l,2a] f32 or bf16 NHWC ('rpn_class_raw', rpn.py:50; a anchors per location, (bg,fg) pairs),
+ * bbox[l]:         [B,H_l,W_l,4a] f32 or bf16 NHWC ('rpn_bbox_pred', rpn.py:63), l < num_levels. The logits and the
+ * deltas each have one dtype for every level, chosen independently (bf16 as for od_proposal_forward).
  * The reference reshapes each to [B,-1,2] / [B,-1,4], takes the softmax of the pairs (rpn.py:54-59) and concatenates
  * the levels along the anchor axis (training.py:163-166); anchor i of that concatenation is what `anchors`/`spec`,
  * debug.ix etc. refer to. The fg probability exp(fg-m)/(exp(bg-m)+exp(fg-m)), m = max(bg,fg), is computed in fp32
@@ -305,8 +316,10 @@ int od_rpn_target_forward(const DLTensor* anchors, const DLTensor* gt_boxes, con
  * rounded to fp32 once (deterministic; equal to TensorFlow's fp32 reductions to ~1e-7 relative).
  *
  * od_rpn_loss_forward: Loss.rpn_class_loss (:11-44) and Loss.rpn_box_loss (:47-87).
- *   rpn_target_class [B,A] or [B,A,1] i32 (+1 positive, -1 negative, 0 neutral), rpn_class_logits [B,A,2] f32 (bg,fg),
- *   rpn_target_bbox [B,T,4] f32 zero padded, rpn_pred_box [B,A,4] f32 (both NULL: class loss only).
+ *   rpn_target_class [B,A] or [B,A,1] i32 (+1 positive, -1 negative, 0 neutral), rpn_class_logits [B,A,2] f32 or bf16
+ *   (bg,fg), rpn_target_bbox [B,T,4] f32 zero padded, rpn_pred_box [B,A,4] f32 or bf16 (both NULL: class loss only).
+ *   bf16 predictions follow the head-output contract of od_proposal_forward: widened exactly, so the losses and
+ *   pred_box_pos (the widened values) equal those of the f32 call on the widened tensors bit for bit.
  *   losses [2] f32 = (rpn_class_loss, rpn_box_loss); either is 0 when nothing contributes (K.switch).
  *   The r-th positive anchor of image b (ascending) pairs with rpn_target_bbox[b,r]; positives beyond T rows are
  *   ignored (the reference's shapes would not match there). pred_box_pos [P,4] f32 or NULL receives the gathered
@@ -317,8 +330,9 @@ int od_rpn_loss_forward(const DLTensor* rpn_target_class, const DLTensor* rpn_cl
                         DLTensor* losses, DLTensor* pred_box_pos, DLTensor* num_pos,
                         void* ws, size_t ws_bytes, void* stream);
 /* od_mrcnn_loss_forward: Loss.mrcnn_class_loss (:89-151) and Loss.mrcnn_box_loss (:154-201).
- *   mrcnn_target_class_ids [B,R] i32 zero padded; pred_logits [B,R,C] f32 with batch_active_class_ids [B,C] f32
- *   (row 0 is the one the reference gathers, :115) and / or target_box [B,R,4] f32 with pred_box [B,R,C,4] f32.
+ *   mrcnn_target_class_ids [B,R] i32 zero padded; pred_logits [B,R,C] f32 or bf16 with batch_active_class_ids [B,C]
+ *   f32 (row 0 is the one the reference gathers, :115) and / or target_box [B,R,4] f32 with pred_box [B,R,C,4] f32 or
+ *   bf16 (bf16 as for od_rpn_loss_forward; pred_active stays f32).
  *   losses [2] f32 = (sum(ce * pred_active) / sum(pred_active), mean binary cross-entropy over the positive ROIs'
  *   boxes of their target class — K.binary_crossentropy as the reference has it — or 0 without positives);
  *   pred_active [B,R] f32 or NULL. A pair that is not passed leaves its loss at 0. */
@@ -345,7 +359,9 @@ typedef struct od_detection_debug {
 } od_detection_debug;
 
 size_t od_detection_workspace_bytes(int64_t batch, int64_t num_rois, int64_t num_classes);
-/* proposals [B,N,4] f32, mrcnn_class_probs [B,N,C] f32, mrcnn_bbox [B,N,C,4] f32,
+/* proposals [B,N,4] f32, mrcnn_class_probs [B,N,C] f32 or bf16, mrcnn_bbox [B,N,C,4] f32 or bf16 (independently; bf16
+ * under the head-output contract of od_proposal_forward: the argmax scan, its first-max and NaN rules, the score and
+ * the decode are those of the f32 call on the widened values),
  * window_norm [B,4] f32 (norm_boxes of the pixel window, utils.py:181-196);
  * detections [B,max_instances,6] f32 rows (y1,x1,y2,x2,class_id,score), zero padded. */
 int od_detection_forward(const DLTensor* proposals, const DLTensor* mrcnn_class_probs,

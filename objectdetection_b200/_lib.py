@@ -266,6 +266,20 @@ def as_cuda(x, dtype, device=None) -> torch.Tensor:
     return t.contiguous()
 
 
+def read_dtype(tensors, align: int, depth_multiple: int = 1) -> torch.dtype:
+    """The dtype the kernels read ``tensors`` in, for an argument they take in float32 or bfloat16.
+
+    bfloat16 when every tensor is a bfloat16 CUDA tensor whose data pointer is ``align``-byte aligned (the size of the
+    kernel's load) and whose last extent is a multiple of ``depth_multiple``: the tensors then go to the kernels as they
+    are, with no float32 copy. float32 for anything else (host arrays, float16, misaligned views, lists of mixed dtype),
+    which ``as_cuda`` converts as it always has. The kernels widen bfloat16 exactly, so either way the result is that of
+    the float32 path on ``t.float()``."""
+    if all(isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.bfloat16 and t.dim() > 0
+           and t.shape[-1] % depth_multiple == 0 and t.data_ptr() % align == 0 for t in tensors):
+        return torch.bfloat16
+    return torch.float32
+
+
 _const_cache = {}
 _CONST_CACHE_MAX = 4096
 

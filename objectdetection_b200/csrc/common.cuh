@@ -8,6 +8,7 @@
 //   * float -> int32 follows x86 cvttss2si (NaN / out of range -> INT_MIN);
 //   * ordering ties go to the lower index (composite 64-bit keys).
 #pragma once
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -90,6 +91,11 @@ inline int check_tensor(const DLTensor* t, const char* name, DType dt, std::init
 inline int check_opt_tensor(const DLTensor* t, const char* name, DType dt, std::initializer_list<int64_t> extents,
                             int align_bytes, DeviceScope& scope) {
   return t ? check_tensor(t, name, dt, extents, align_bytes, scope) : OD_OK;
+}
+// The dtype an argument that may be fp32 or bf16 is checked against: BF16 for a bfloat16 tensor, F32 for anything else,
+// which check_tensor then refuses unless it is fp32 (float16 included). NULL gives F32.
+inline DType f32_or_bf16(const DLTensor* t) {
+  return (t && t->dtype.code == kDLBfloat && t->dtype.bits == 16 && t->dtype.lanes == 1) ? BF16 : F32;
 }
 inline int64_t numel(const DLTensor* t) {
   int64_t n = 1;
@@ -248,6 +254,28 @@ __device__ __forceinline__ float tf_iou(const CBox& i, const CBox& j) {
 // 16-byte global accesses with cache hints.
 __device__ __forceinline__ float4 ldg_f4(const float4* p) { return __ldg(p); }
 __device__ __forceinline__ void stg_cs_f4(float4* p, float4 v) { __stcs(p, v); }   // streaming store (evict first)
+
+// Network-head outputs (RPN logits and deltas, classifier probabilities and boxes, the loss inputs) are read as fp32 or
+// bf16. A bf16 is the upper half of an fp32, so it is widened exactly with a shift: sign, NaN payload and subnormals
+// survive (the library is built without flush-to-zero), and everything after the load is the fp32 path on the widened
+// values. Element 0 of a packed pair sits in the low half. Loaded in one access each: one scalar, the i-th (x, y) pair
+// (8 B, or 4 B in bf16) or the i-th 4-value row (16 B, or 8 B in bf16) of p.
+__device__ __forceinline__ float widen_bf16(uint32_t bits) { return __uint_as_float(bits << 16); }
+__device__ __forceinline__ float2 widen_bf16x2(uint32_t u) { return make_float2(widen_bf16(u), __uint_as_float(u & 0xFFFF0000u)); }
+__device__ __forceinline__ float ld_head(const float* p) { return *p; }
+__device__ __forceinline__ float ld_head(const __nv_bfloat16* p) {
+  return widen_bf16(*reinterpret_cast<const unsigned short*>(p));
+}
+__device__ __forceinline__ float2 ldg_head2(const float* p, int64_t i) { return __ldg(reinterpret_cast<const float2*>(p) + i); }
+__device__ __forceinline__ float2 ldg_head2(const __nv_bfloat16* p, int64_t i) {
+  return widen_bf16x2(__ldg(reinterpret_cast<const unsigned int*>(p) + i));
+}
+__device__ __forceinline__ float4 ldg_head4(const float* p, int64_t i) { return __ldg(reinterpret_cast<const float4*>(p) + i); }
+__device__ __forceinline__ float4 ldg_head4(const __nv_bfloat16* p, int64_t i) {
+  const uint2 u = __ldg(reinterpret_cast<const uint2*>(p) + i);
+  const float2 lo = widen_bf16x2(u.x), hi = widen_bf16x2(u.y);
+  return make_float4(lo.x, lo.y, hi.x, hi.y);
+}
 
 constexpr int kNumSMsB200 = 148;
 

@@ -23,13 +23,15 @@ struct DetDebugPtrs {
   int32_t* keep_mask;
 };
 
-// One warp per ROI slot (slots >= N only clear their sort key).
-__global__ void __launch_bounds__(256)
-det_prepare_kernel(const float4* __restrict__ proposals, const float* __restrict__ probs,
-                   const float4* __restrict__ bbox, const float4* __restrict__ window, int N, int C, int n_pow2,
-                   float4 stddev, float min_conf, int32_t* __restrict__ cls_out, float* __restrict__ score_out,
-                   float4* __restrict__ clipped_out, unsigned long long* __restrict__ keys,
-                   int32_t* __restrict__ num_valid, DetDebugPtrs dbg) {
+// One warp per ROI slot (slots >= N only clear their sort key). TP, TB: the dtypes (float or bf16) of the probabilities
+// and of the box deltas; bf16 values are widened exactly, so the scan and the decode are the fp32 ones on those values.
+template <typename TP, typename TB>
+__device__ __forceinline__ void det_prepare_body(const float4* __restrict__ proposals, const TP* __restrict__ probs,
+                                                 const TB* __restrict__ bbox, const float4* __restrict__ window, int N,
+                                                 int C, int n_pow2, float4 stddev, float min_conf,
+                                                 int32_t* __restrict__ cls_out, float* __restrict__ score_out,
+                                                 float4* __restrict__ clipped_out, unsigned long long* __restrict__ keys,
+                                                 int32_t* __restrict__ num_valid, const DetDebugPtrs& dbg) {
   const int lane = threadIdx.x & 31;
   const int64_t slot = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int b = blockIdx.y;
@@ -41,21 +43,21 @@ det_prepare_kernel(const float4* __restrict__ proposals, const float* __restrict
   if (slot == 0 && lane == 0) num_valid[b] = 0;   // det_rank_gather_kernel raises it with atomicMax
   const int n = (int)slot;
   const int64_t r = (int64_t)b * N + n;
-  const float* p = probs + r * C;
+  const TP* p = probs + r * C;
   // argmax, first maximum (detection.py:115), as the sequential `best = p[0]; if (p[c] > best)` scan decides it: a NaN
   // in p[0] wins (nothing compares greater), a NaN anywhere else is never taken. A lane's own first value is the only
   // one it takes without a compare, so lanes other than 0 drop a NaN there.
   float best = -INFINITY;
   int arg = 0x7fffffff;
   if (lane < C) {
-    best = p[lane];
+    best = ld_head(p + lane);
     arg = lane;
     if (lane > 0 && best != best) {
       best = -INFINITY;
       arg = 0x7fffffff;
     }
     for (int c = lane + 32; c < C; c += 32) {
-      const float v = p[c];
+      const float v = ld_head(p + c);
       if (v > best) {
         best = v;
         arg = c;
@@ -73,8 +75,8 @@ det_prepare_kernel(const float4* __restrict__ proposals, const float* __restrict
   }
   if (lane != 0) return;
   if (arg == 0x7fffffff) arg = 0;
-  const float score = p[arg];                                                        // :129
-  const float4 raw = __ldg(&bbox[r * C + arg]);
+  const float score = ld_head(p + arg);                                              // :129
+  const float4 raw = ldg_head4(bbox, r * C + arg);
   const float4 d = make_float4(raw.x * stddev.x, raw.y * stddev.y, raw.z * stddev.z, raw.w * stddev.w);  // :117,:130
   const float4 ref = decode_box(proposals[r], d);                                    // :133
   const float4 cl = clip_box(ref, window[b]);                                        // :147
@@ -92,6 +94,26 @@ det_prepare_kernel(const float4* __restrict__ proposals, const float* __restrict
   if (dbg.refined) dbg.refined[r] = ref;
   if (dbg.clipped) dbg.clipped[r] = cl;
   if (dbg.keep_mask) dbg.keep_mask[r] = keep ? 1 : 0;
+}
+__global__ void __launch_bounds__(256)
+det_prepare_kernel(const float4* __restrict__ proposals, const float* __restrict__ probs,
+                   const float4* __restrict__ bbox, const float4* __restrict__ window, int N, int C, int n_pow2,
+                   float4 stddev, float min_conf, int32_t* __restrict__ cls_out, float* __restrict__ score_out,
+                   float4* __restrict__ clipped_out, unsigned long long* __restrict__ keys,
+                   int32_t* __restrict__ num_valid, DetDebugPtrs dbg) {
+  det_prepare_body<float, float>(proposals, probs, reinterpret_cast<const float*>(bbox), window, N, C, n_pow2, stddev,
+                                 min_conf, cls_out, score_out, clipped_out, keys, num_valid, dbg);
+}
+// bf16 probabilities and / or box deltas: the same body, an overload of the same name (the fp32 kernel above keeps its
+// name)
+template <typename TP, typename TB>
+__global__ void __launch_bounds__(256)
+det_prepare_kernel(const float4* __restrict__ proposals, const TP* __restrict__ probs, const TB* __restrict__ bbox,
+                   const float4* __restrict__ window, int N, int C, int n_pow2, float4 stddev, float min_conf,
+                   int32_t* __restrict__ cls_out, float* __restrict__ score_out, float4* __restrict__ clipped_out,
+                   unsigned long long* __restrict__ keys, int32_t* __restrict__ num_valid, DetDebugPtrs dbg) {
+  det_prepare_body<TP, TB>(proposals, probs, bbox, window, N, C, n_pow2, stddev, min_conf, cls_out, score_out,
+                           clipped_out, keys, num_valid, dbg);
 }
 
 // Rank sort of the N keys of one image fused with the gather: keys are unique, the sorted position of a key is the
@@ -376,10 +398,12 @@ int od_detection_forward(const DLTensor* proposals, const DLTensor* mrcnn_class_
   if (!params) OD_FAIL(OD_ERR_NULL, "params is NULL");
   DeviceScope scope;
   OD_CHECK(check_tensor(proposals, "proposals", F32, {kAny, kAny, 4}, 16, scope));
-  OD_CHECK(check_tensor(mrcnn_class_probs, "mrcnn_class_probs", F32, {proposals->shape[0], proposals->shape[1], kAny}, 4, scope));
+  const DType probs_dt = f32_or_bf16(mrcnn_class_probs), bbox_dt = f32_or_bf16(mrcnn_bbox);
+  OD_CHECK(check_tensor(mrcnn_class_probs, "mrcnn_class_probs", probs_dt, {proposals->shape[0], proposals->shape[1], kAny},
+                        probs_dt == BF16 ? 2 : 4, scope));
   const int64_t B = mrcnn_class_probs->shape[0], N = mrcnn_class_probs->shape[1], C = mrcnn_class_probs->shape[2];
   const int64_t M = params->max_instances;
-  OD_CHECK(check_tensor(mrcnn_bbox, "mrcnn_bbox", F32, {B, N, C, 4}, 16, scope));
+  OD_CHECK(check_tensor(mrcnn_bbox, "mrcnn_bbox", bbox_dt, {B, N, C, 4}, bbox_dt == BF16 ? 8 : 16, scope));
   OD_CHECK(check_tensor(window_norm, "window_norm", F32, {B, 4}, 16, scope));
   OD_CHECK(check_tensor(detections, "detections", F32, {B, M, 6}, 4, scope));
   if (N > 16384 || C > 65535 || C < 1) OD_FAIL(OD_ERR_PARAM, "DetectionLayer supports N <= 16384 ROIs and 1 <= C <= 65535 classes");
@@ -415,9 +439,24 @@ int od_detection_forward(const DLTensor* proposals, const DLTensor* mrcnn_class_
   dp.keep_mask = dptr<int32_t>(dbg.keep_mask);
   {
     const dim3 grid((unsigned)(((int64_t)n_pow2 * 32 + 255) / 256), (unsigned)B);
-    det_prepare_kernel<<<grid, 256, 0, st>>>(dptr<float4>(proposals), dptr<float>(mrcnn_class_probs),
-                                             dptr<float4>(mrcnn_bbox), dptr<float4>(window_norm), (int)N, (int)C, n_pow2,
-                                             sd, params->min_confidence, d.cls, d.score, d.clipped, d.keys, d.num_valid, dp);
+    using BF = __nv_bfloat16;
+    const float4* pr = dptr<float4>(proposals);
+    const float4* win = dptr<float4>(window_norm);
+    const float mc = params->min_confidence;
+    if (probs_dt == BF16 && bbox_dt == BF16)
+      det_prepare_kernel<BF, BF><<<grid, 256, 0, st>>>(pr, dptr<BF>(mrcnn_class_probs), dptr<BF>(mrcnn_bbox), win, (int)N,
+                                                       (int)C, n_pow2, sd, mc, d.cls, d.score, d.clipped, d.keys, d.num_valid, dp);
+    else if (probs_dt == BF16)
+      det_prepare_kernel<BF, float><<<grid, 256, 0, st>>>(pr, dptr<BF>(mrcnn_class_probs), dptr<float>(mrcnn_bbox), win,
+                                                          (int)N, (int)C, n_pow2, sd, mc, d.cls, d.score, d.clipped, d.keys,
+                                                          d.num_valid, dp);
+    else if (bbox_dt == BF16)
+      det_prepare_kernel<float, BF><<<grid, 256, 0, st>>>(pr, dptr<float>(mrcnn_class_probs), dptr<BF>(mrcnn_bbox), win,
+                                                          (int)N, (int)C, n_pow2, sd, mc, d.cls, d.score, d.clipped, d.keys,
+                                                          d.num_valid, dp);
+    else
+      det_prepare_kernel<<<grid, 256, 0, st>>>(pr, dptr<float>(mrcnn_class_probs), dptr<float4>(mrcnn_bbox), win, (int)N,
+                                               (int)C, n_pow2, sd, mc, d.cls, d.score, d.clipped, d.keys, d.num_valid, dp);
     OD_LAUNCH_CHECK("det_prepare_kernel");
   }
   const unsigned long long* sorted_keys = d.sorted_keys;

@@ -48,9 +48,11 @@ __device__ T cta_sum(T v, T* scratch) {
   return r;
 }
 
-// Pass 1: per 1024-anchor chunk, the cross-entropy sum and the counts of non-neutral / positive anchors.
-__global__ void __launch_bounds__(kLossThreads)
-rpn_loss_class_kernel(const int32_t* __restrict__ target, const float2* __restrict__ logits, int A, RpnLossPart* __restrict__ part) {
+// Pass 1: per 1024-anchor chunk, the cross-entropy sum and the counts of non-neutral / positive anchors. T: the dtype of
+// the logits (float or bf16, widened exactly).
+template <typename T>
+__device__ __forceinline__ void rpn_loss_class_body(const int32_t* __restrict__ target, const T* __restrict__ logits, int A,
+                                                    RpnLossPart* __restrict__ part) {
   __shared__ double sd[kLossWarps];
   __shared__ int si[kLossWarps];
   const int b = blockIdx.y, i0 = blockIdx.x * kLossChunk + 4 * threadIdx.x;
@@ -62,7 +64,7 @@ rpn_loss_class_kernel(const int32_t* __restrict__ target, const float2* __restri
     if (i >= A) break;
     const int t = target[(int64_t)b * A + i];
     if (t == 0) continue;
-    const float2 x = __ldg(&logits[(int64_t)b * A + i]);
+    const float2 x = ldg_head2(logits, (int64_t)b * A + i);
     const float m = f_max(x.x, x.y);
     const float s = f_exp(x.x - m) + f_exp(x.y - m);
     ce += (double)(f_log(s) - (((t == 1) ? x.y : x.x) - m));   // label 1 = foreground (:31)
@@ -83,12 +85,25 @@ rpn_loss_class_kernel(const int32_t* __restrict__ target, const float2* __restri
     part[(int64_t)b * gridDim.x + blockIdx.x] = p;
   }
 }
+__global__ void __launch_bounds__(kLossThreads)
+rpn_loss_class_kernel(const int32_t* __restrict__ target, const float2* __restrict__ logits, int A, RpnLossPart* __restrict__ part) {
+  rpn_loss_class_body<float>(target, reinterpret_cast<const float*>(logits), A, part);
+}
+// bf16 logits: the same body, an overload of the same name (the fp32 kernel above keeps its name)
+template <typename T>
+__global__ void __launch_bounds__(kLossThreads)
+rpn_loss_class_kernel(const int32_t* __restrict__ target, const T* __restrict__ logits, int A, RpnLossPart* __restrict__ part) {
+  rpn_loss_class_body<T>(target, logits, A, part);
+}
 
 // Pass 2: the r-th positive anchor of image b (ascending) pairs with rpn_target_bbox[b, r] (:66-74); positives past
-// the T target rows have no partner and are ignored. Optionally writes rpn_pred_box_pos (:64).
-__global__ void __launch_bounds__(kLossThreads)
-rpn_loss_box_kernel(const int32_t* __restrict__ target, const float4* __restrict__ pred, const float4* __restrict__ target_bbox,
-                    int A, int T, RpnLossPart* __restrict__ part, float4* __restrict__ pred_pos, int64_t pred_pos_rows) {
+// the T target rows have no partner and are ignored. Optionally writes rpn_pred_box_pos (:64), the widened values when
+// the predictions are bf16 (TP).
+template <typename TP>
+__device__ __forceinline__ void rpn_loss_box_body(const int32_t* __restrict__ target, const TP* __restrict__ pred,
+                                                  const float4* __restrict__ target_bbox, int A, int T,
+                                                  RpnLossPart* __restrict__ part, float4* __restrict__ pred_pos,
+                                                  int64_t pred_pos_rows) {
   __shared__ double sd[kLossWarps];
   __shared__ int si[kLossWarps];
   const int b = blockIdx.y, i0 = blockIdx.x * kLossChunk + 4 * threadIdx.x, nchunk = gridDim.x;
@@ -126,7 +141,7 @@ rpn_loss_box_kernel(const int32_t* __restrict__ target, const float4* __restrict
 #pragma unroll
   for (int u = 0; u < 4; ++u) {
     if (!(flags >> u & 1)) continue;
-    const float4 p = __ldg(&pred[(int64_t)b * A + i0 + u]);
+    const float4 p = ldg_head4(pred, (int64_t)b * A + i0 + u);
     if (pred_pos && (int64_t)earlier + r < pred_pos_rows) pred_pos[(int64_t)earlier + r] = p;
     if (r < T) {
       const float4 t = __ldg(&target_bbox[(int64_t)b * T + r]);
@@ -147,6 +162,18 @@ rpn_loss_box_kernel(const int32_t* __restrict__ target, const float4* __restrict
     part[(int64_t)b * nchunk + blockIdx.x].box_sum = sum_all;
     part[(int64_t)b * nchunk + blockIdx.x].used = used_all;
   }
+}
+__global__ void __launch_bounds__(kLossThreads)
+rpn_loss_box_kernel(const int32_t* __restrict__ target, const float4* __restrict__ pred, const float4* __restrict__ target_bbox,
+                    int A, int T, RpnLossPart* __restrict__ part, float4* __restrict__ pred_pos, int64_t pred_pos_rows) {
+  rpn_loss_box_body<float>(target, reinterpret_cast<const float*>(pred), target_bbox, A, T, part, pred_pos, pred_pos_rows);
+}
+// bf16 predictions: the same body, an overload of the same name
+template <typename TP>
+__global__ void __launch_bounds__(kLossThreads)
+rpn_loss_box_kernel(const int32_t* __restrict__ target, const TP* __restrict__ pred, const float4* __restrict__ target_bbox,
+                    int A, int T, RpnLossPart* __restrict__ part, float4* __restrict__ pred_pos, int64_t pred_pos_rows) {
+  rpn_loss_box_body<TP>(target, pred, target_bbox, A, T, part, pred_pos, pred_pos_rows);
 }
 
 __global__ void __launch_bounds__(kLossThreads)
@@ -175,11 +202,13 @@ rpn_loss_final_kernel(const RpnLossPart* __restrict__ part, int64_t n, float* __
   }
 }
 
-// Both mask-rcnn head losses, one CTA: thread-strided over the B*R ROIs, class loop sequential per ROI.
-__global__ void __launch_bounds__(1024)
-mrcnn_loss_kernel(const int32_t* __restrict__ target_ids, const float* __restrict__ logits, const float* __restrict__ active,
-                  const float4* __restrict__ target_box, const float4* __restrict__ pred_box, int64_t rows, int C,
-                  float* __restrict__ losses, float* __restrict__ pred_active_out) {
+// Both mask-rcnn head losses, one CTA: thread-strided over the B*R ROIs, class loop sequential per ROI. TL, TB: the
+// dtypes (float or bf16, widened exactly) of the logits and of the predicted boxes.
+template <typename TL, typename TB>
+__device__ __forceinline__ void mrcnn_loss_body(const int32_t* __restrict__ target_ids, const TL* __restrict__ logits,
+                                                const float* __restrict__ active, const float4* __restrict__ target_box,
+                                                const TB* __restrict__ pred_box, int64_t rows, int C,
+                                                float* __restrict__ losses, float* __restrict__ pred_active_out) {
   __shared__ double sd[32];
   __shared__ int si[32];
   double cls_sum = 0.0, act_sum = 0.0, box_sum = 0.0;
@@ -188,17 +217,17 @@ mrcnn_loss_kernel(const int32_t* __restrict__ target_ids, const float* __restric
   for (int64_t r = threadIdx.x; r < rows; r += blockDim.x) {
     const int label = target_ids[r];
     if (logits) {
-      const float* x = logits + r * C;
-      float m = x[0];
+      const TL* x = logits + r * C;
+      float m = ld_head(x);
       int arg = 0;
       for (int j = 1; j < C; ++j)
-        if (x[j] > m) {   // tf.argmax: first maximum (:113)
-          m = x[j];
+        if (ld_head(x + j) > m) {   // tf.argmax: first maximum (:113)
+          m = ld_head(x + j);
           arg = j;
         }
       float s = 0.0f;
-      for (int j = 0; j < C; ++j) s += f_exp(x[j] - m);
-      const float ce = (label >= 0 && label < C) ? f_log(s) - (x[label] - m) : __int_as_float(0x7fc00000);   // :139-142
+      for (int j = 0; j < C; ++j) s += f_exp(ld_head(x + j) - m);
+      const float ce = (label >= 0 && label < C) ? f_log(s) - (ld_head(x + label) - m) : __int_as_float(0x7fc00000);   // :139-142
       const float pa = active[arg];   // batch_active_class_ids[0] gathered at the predicted class (:115)
       if (pred_active_out) pred_active_out[r] = pa;
       cls_sum += (double)(ce * pa);   // :146
@@ -206,7 +235,7 @@ mrcnn_loss_kernel(const int32_t* __restrict__ target_ids, const float* __restric
     }
     if (pred_box && label > 0 && label < C) {   // positive ROI (:171): box predicted for its target class (:180-184)
       const float4 t = __ldg(&target_box[r]);
-      const float4 p = __ldg(&pred_box[r * C + label]);
+      const float4 p = ldg_head4(pred_box, r * C + label);
       const float tv[4] = {t.x, t.y, t.z, t.w}, pv[4] = {p.x, p.y, p.z, p.w};
 #pragma unroll
       for (int c = 0; c < 4; ++c) {
@@ -227,6 +256,21 @@ mrcnn_loss_kernel(const int32_t* __restrict__ target_ids, const float* __restric
     losses[0] = logits ? (float)(cls_sum / act_sum) : 0.0f;                      // :148 (0/0 = NaN like the reference)
     losses[1] = box_n > 0 ? (float)(box_sum / (4.0 * (double)box_n)) : 0.0f;     // :195-198
   }
+}
+__global__ void __launch_bounds__(1024)
+mrcnn_loss_kernel(const int32_t* __restrict__ target_ids, const float* __restrict__ logits, const float* __restrict__ active,
+                  const float4* __restrict__ target_box, const float4* __restrict__ pred_box, int64_t rows, int C,
+                  float* __restrict__ losses, float* __restrict__ pred_active_out) {
+  mrcnn_loss_body<float, float>(target_ids, logits, active, target_box, reinterpret_cast<const float*>(pred_box), rows, C,
+                                losses, pred_active_out);
+}
+// bf16 logits and / or predicted boxes: the same body, an overload of the same name (the fp32 kernel above keeps its name)
+template <typename TL, typename TB>
+__global__ void __launch_bounds__(1024)
+mrcnn_loss_kernel(const int32_t* __restrict__ target_ids, const TL* __restrict__ logits, const float* __restrict__ active,
+                  const float4* __restrict__ target_box, const TB* __restrict__ pred_box, int64_t rows, int C,
+                  float* __restrict__ losses, float* __restrict__ pred_active_out) {
+  mrcnn_loss_body<TL, TB>(target_ids, logits, active, target_box, pred_box, rows, C, losses, pred_active_out);
 }
 
 }  // namespace od
@@ -251,14 +295,15 @@ int od_rpn_loss_forward(const DLTensor* rpn_target_class, const DLTensor* rpn_cl
   else
     OD_CHECK(check_tensor(rpn_target_class, "rpn_target_class", I32, {kAny, kAny}, 4, scope));
   const int64_t B = rpn_target_class->shape[0], A = rpn_target_class->shape[1];
-  OD_CHECK(check_tensor(rpn_class_logits, "rpn_class_logits", F32, {B, A, 2}, 8, scope));
+  const DType logits_dt = f32_or_bf16(rpn_class_logits), pred_dt = f32_or_bf16(rpn_pred_box);
+  OD_CHECK(check_tensor(rpn_class_logits, "rpn_class_logits", logits_dt, {B, A, 2}, logits_dt == BF16 ? 4 : 8, scope));
   OD_CHECK(check_tensor(losses, "losses", F32, {2}, 4, scope));
   const bool with_box = rpn_target_bbox && rpn_pred_box;   // both NULL: class loss only (losses[1] = 0)
   if (!with_box && (rpn_target_bbox || rpn_pred_box || pred_box_pos)) OD_FAIL(OD_ERR_NULL, "rpn_target_bbox and rpn_pred_box go together");
   int64_t T = 0;
   if (with_box) {
     OD_CHECK(check_tensor(rpn_target_bbox, "rpn_target_bbox", F32, {B, kAny, 4}, 16, scope));
-    OD_CHECK(check_tensor(rpn_pred_box, "rpn_pred_box", F32, {B, A, 4}, 16, scope));
+    OD_CHECK(check_tensor(rpn_pred_box, "rpn_pred_box", pred_dt, {B, A, 4}, pred_dt == BF16 ? 8 : 16, scope));
     T = rpn_target_bbox->shape[1];
   }
   if (A >= (1ll << 31) || B > 65535) OD_FAIL(OD_ERR_PARAM, "supports A < 2^31, B <= 65535");
@@ -272,12 +317,18 @@ int od_rpn_loss_forward(const DLTensor* rpn_target_class, const DLTensor* rpn_cl
   if (!w.ok()) OD_FAIL(OD_ERR_WORKSPACE, "workspace %zu < %zu bytes", ws_bytes, w.off);
   if (B > 0 && A > 0) {
     const dim3 grid((unsigned)nchunk, (unsigned)B);
-    rpn_loss_class_kernel<<<grid, kLossThreads, 0, st>>>(dptr<int32_t>(rpn_target_class), dptr<float2>(rpn_class_logits), (int)A, part);
+    using BF = __nv_bfloat16;
+    const int32_t* tc = dptr<int32_t>(rpn_target_class);
+    if (logits_dt == BF16) rpn_loss_class_kernel<BF><<<grid, kLossThreads, 0, st>>>(tc, dptr<BF>(rpn_class_logits), (int)A, part);
+    else rpn_loss_class_kernel<<<grid, kLossThreads, 0, st>>>(tc, dptr<float2>(rpn_class_logits), (int)A, part);
     OD_LAUNCH_CHECK("rpn_loss_class_kernel");
     if (with_box) {
-      rpn_loss_box_kernel<<<grid, kLossThreads, 0, st>>>(dptr<int32_t>(rpn_target_class), dptr<float4>(rpn_pred_box),
-                                                         dptr<float4>(rpn_target_bbox), (int)A, (int)T, part,
-                                                         dptr<float4>(pred_box_pos), pos_rows);
+      if (pred_dt == BF16)
+        rpn_loss_box_kernel<BF><<<grid, kLossThreads, 0, st>>>(tc, dptr<BF>(rpn_pred_box), dptr<float4>(rpn_target_bbox), (int)A,
+                                                               (int)T, part, dptr<float4>(pred_box_pos), pos_rows);
+      else
+        rpn_loss_box_kernel<<<grid, kLossThreads, 0, st>>>(tc, dptr<float4>(rpn_pred_box), dptr<float4>(rpn_target_bbox), (int)A,
+                                                           (int)T, part, dptr<float4>(pred_box_pos), pos_rows);
       OD_LAUNCH_CHECK("rpn_loss_box_kernel");
     }
   }
@@ -298,22 +349,37 @@ int od_mrcnn_loss_forward(const DLTensor* target_class_ids, const DLTensor* pred
     OD_FAIL(OD_ERR_NULL, "pass (mrcnn_pred_logits, batch_active_class_ids) and / or (mrcnn_target_box, mrcnn_pred_box)");
   const int64_t B = target_class_ids->shape[0], R = target_class_ids->shape[1];
   int64_t C = 0;
+  const DType logits_dt = f32_or_bf16(pred_logits), box_dt = f32_or_bf16(pred_box);
   if (with_cls) {
-    OD_CHECK(check_tensor(pred_logits, "mrcnn_pred_logits", F32, {B, R, kAny}, 4, scope));
+    OD_CHECK(check_tensor(pred_logits, "mrcnn_pred_logits", logits_dt, {B, R, kAny}, logits_dt == BF16 ? 2 : 4, scope));
     C = pred_logits->shape[2];
     OD_CHECK(check_tensor(active_class_ids, "batch_active_class_ids", F32, {kAny, C}, 4, scope));
     if (active_class_ids->shape[0] < 1) OD_FAIL(OD_ERR_SHAPE, "batch_active_class_ids must be [B,C]");
   }
   if (with_box) {
     OD_CHECK(check_tensor(target_box, "mrcnn_target_box", F32, {B, R, 4}, 16, scope));
-    OD_CHECK(check_tensor(pred_box, "mrcnn_pred_box", F32, {B, R, with_cls ? C : kAny, 4}, 16, scope));
+    OD_CHECK(check_tensor(pred_box, "mrcnn_pred_box", box_dt, {B, R, with_cls ? C : kAny, 4}, box_dt == BF16 ? 8 : 16, scope));
     if (!with_cls) C = pred_box->shape[2];
   }
   if (C < 1 || C > (1 << 20)) OD_FAIL(OD_ERR_PARAM, "class count out of range");
   OD_CHECK(check_opt_tensor(pred_active, "pred_active", F32, {B, R}, 4, scope));
-  mrcnn_loss_kernel<<<1, 1024, 0, st>>>(dptr<int32_t>(target_class_ids), dptr<float>(pred_logits), dptr<float>(active_class_ids),
-                                        dptr<float4>(target_box), dptr<float4>(pred_box), B * R, (int)C, dptr<float>(losses),
-                                        dptr<float>(pred_active));
+  using BF = __nv_bfloat16;
+  const int32_t* ids = dptr<int32_t>(target_class_ids);
+  const float* act = dptr<float>(active_class_ids);
+  const float4* tb = dptr<float4>(target_box);
+  float* out = dptr<float>(losses);
+  float* pa = dptr<float>(pred_active);
+  // an omitted pair (NULL) counts as fp32
+  if (logits_dt == BF16 && box_dt == BF16)
+    mrcnn_loss_kernel<BF, BF><<<1, 1024, 0, st>>>(ids, dptr<BF>(pred_logits), act, tb, dptr<BF>(pred_box), B * R, (int)C, out, pa);
+  else if (logits_dt == BF16)
+    mrcnn_loss_kernel<BF, float><<<1, 1024, 0, st>>>(ids, dptr<BF>(pred_logits), act, tb, dptr<float>(pred_box), B * R, (int)C,
+                                                     out, pa);
+  else if (box_dt == BF16)
+    mrcnn_loss_kernel<float, BF><<<1, 1024, 0, st>>>(ids, dptr<float>(pred_logits), act, tb, dptr<BF>(pred_box), B * R, (int)C,
+                                                     out, pa);
+  else
+    mrcnn_loss_kernel<<<1, 1024, 0, st>>>(ids, dptr<float>(pred_logits), act, tb, dptr<float4>(pred_box), B * R, (int)C, out, pa);
   OD_LAUNCH_CHECK("mrcnn_loss_kernel");
   return OD_OK;
 }

@@ -16,32 +16,35 @@ struct ProposalDebugPtrs {
 };
 
 // RPN head outputs in their native layout: one [B, n_l, C] block per pyramid level (the reshape of the conv output
-// [B,H_l,W_l,a*C], rpn.py:54/66); the reference concatenates them along the anchor axis (training.py:163-166).
+// [B,H_l,W_l,a*C], rpn.py:54/66); the reference concatenates them along the anchor axis (training.py:163-166). Every
+// level of one table has one dtype, fp32 or bf16: the kernel reading it is instantiated for that dtype.
 struct LevelTable {
-  const float* base[OD_MAX_LEVELS];
+  const void* base[OD_MAX_LEVELS];
   int32_t off[OD_MAX_LEVELS + 1];   // first flat anchor index of each level
   int32_t num_levels;
 };
-template <int C>
-__device__ __forceinline__ const float* level_row(const LevelTable& t, int64_t b, int32_t i) {
+template <int C, typename T>
+__device__ __forceinline__ const T* level_row(const LevelTable& t, int64_t b, int32_t i) {
   int l = 0;
   while (l + 1 < t.num_levels && i >= t.off[l + 1]) ++l;
   const int64_t n_l = t.off[l + 1] - t.off[l];
-  return t.base[l] + (b * n_l + (i - t.off[l])) * C;
+  return static_cast<const T*>(t.base[l]) + (b * n_l + (i - t.off[l])) * C;
 }
 
-// One thread per selected anchor: 16 B delta + 16 B anchor (or fp64 regeneration) in, 16 B box out.
-template <bool LEVELS>
-__global__ void __launch_bounds__(256)
-proposal_decode_kernel(const float4* __restrict__ bbox, LevelTable lv, const float4* __restrict__ anchors, DevAnchorSpec spec,
-                       int use_spec, const int32_t* __restrict__ ix, int64_t total, int K, int A, float4 stddev,
-                       float4* __restrict__ clipped, ProposalDebugPtrs dbg) {
+// One thread per selected anchor: one delta row (16 B, or 8 B in bf16) + 16 B anchor (or fp64 regeneration) in, 16 B box
+// out. T: the dtype of the deltas, from the level table (LEVELS) or from bbox [B,A,4].
+template <typename T, bool LEVELS>
+__device__ __forceinline__ void proposal_decode_body(const T* __restrict__ bbox, const LevelTable& lv,
+                                                     const float4* __restrict__ anchors, const DevAnchorSpec& spec,
+                                                     int use_spec, const int32_t* __restrict__ ix, int64_t total, int K,
+                                                     int A, float4 stddev, float4* __restrict__ clipped,
+                                                     const ProposalDebugPtrs& dbg) {
   pdl_prologue();
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= total) return;
   const int64_t b = t / K;
   const int32_t i = ix[t];
-  const float4 raw = LEVELS ? __ldg(reinterpret_cast<const float4*>(level_row<4>(lv, b, i))) : __ldg(&bbox[b * A + i]);
+  const float4 raw = LEVELS ? ldg_head4(level_row<4, T>(lv, b, i), 0) : ldg_head4(bbox, b * A + i);
   const float4 d = make_float4(raw.x * stddev.x, raw.y * stddev.y, raw.z * stddev.z, raw.w * stddev.w);  // :157
   const float4 a = use_spec ? anchor_normalized(spec, i) : __ldg(&anchors[b * A + i]);
   const float4 dec = decode_box(a, d);                                            // :179
@@ -52,19 +55,46 @@ proposal_decode_kernel(const float4* __restrict__ bbox, LevelTable lv, const flo
   if (dbg.anchor_delta) dbg.anchor_delta[t] = dec;
   if (dbg.clipped_dbg) dbg.clipped_dbg[t] = c;
 }
+template <bool LEVELS>
+__global__ void __launch_bounds__(256)
+proposal_decode_kernel(const float4* __restrict__ bbox, LevelTable lv, const float4* __restrict__ anchors, DevAnchorSpec spec,
+                       int use_spec, const int32_t* __restrict__ ix, int64_t total, int K, int A, float4 stddev,
+                       float4* __restrict__ clipped, ProposalDebugPtrs dbg) {
+  proposal_decode_body<float, LEVELS>(reinterpret_cast<const float*>(bbox), lv, anchors, spec, use_spec, ix, total, K, A,
+                                      stddev, clipped, dbg);
+}
+// bf16 deltas: the same body, an overload of the same name (the fp32 kernel above keeps its name)
+template <typename T, bool LEVELS>
+__global__ void __launch_bounds__(256)
+proposal_decode_kernel(const T* __restrict__ bbox, LevelTable lv, const float4* __restrict__ anchors, DevAnchorSpec spec,
+                       int use_spec, const int32_t* __restrict__ ix, int64_t total, int K, int A, float4 stddev,
+                       float4* __restrict__ clipped, ProposalDebugPtrs dbg) {
+  proposal_decode_body<T, LEVELS>(bbox, lv, anchors, spec, use_spec, ix, total, K, A, stddev, clipped, dbg);
+}
 
 // Foreground probability of every anchor from the per-level class logits: softmax over the (bg, fg) pair
-// (rpn.py:58-59, tf.nn.softmax: exp(x - max) / sum) written as one contiguous [B,A] row per image for the top-k.
-__global__ void __launch_bounds__(256)
-rpn_level_scores_kernel(LevelTable lv, int A, int64_t total, float* __restrict__ scores) {
+// (rpn.py:58-59, tf.nn.softmax: exp(x - max) / sum) written as one contiguous [B,A] row per image for the top-k. T: the
+// dtype of the logits; the pair is one 8-byte (fp32) or 4-byte (bf16) load.
+template <typename T>
+__device__ __forceinline__ void rpn_level_scores_body(const LevelTable& lv, int A, int64_t total, float* __restrict__ scores) {
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= total) return;
   const int64_t b = t / A;
   const int32_t i = (int32_t)(t - b * A);
-  const float2 x = __ldg(reinterpret_cast<const float2*>(level_row<2>(lv, b, i)));
+  const float2 x = ldg_head2(level_row<2, T>(lv, b, i), 0);
   const float m = (x.x < x.y) ? x.y : x.x;
   const float e0 = f_exp(x.x - m), e1 = f_exp(x.y - m);
   scores[t] = e1 / (e0 + e1);
+}
+__global__ void __launch_bounds__(256)
+rpn_level_scores_kernel(LevelTable lv, int A, int64_t total, float* __restrict__ scores) {
+  rpn_level_scores_body<float>(lv, A, total, scores);
+}
+// bf16 logits: the same body, an overload of the same name
+template <typename T>
+__global__ void __launch_bounds__(256)
+rpn_level_scores_kernel(LevelTable lv, int A, int64_t total, float* __restrict__ scores) {
+  rpn_level_scores_body<T>(lv, A, total, scores);
 }
 
 // proposals[b,j] = clipped[b, keep_pos[b,j]] or zeros (tf.pad, :245-246).
@@ -249,11 +279,13 @@ namespace od {
 // Shared body of od_proposal_forward / od_proposal_forward_levels. `scores` addresses the fg score of anchor i of image b at
 // scores[b * score_sb + i * score_sa]; with `logits` (the per-level class logits), it is a workspace row that is first
 // filled from them. The deltas come from `rpn_bbox4` ([B,A,4]) or, when it is NULL, from `lv`. `p` is the carved
-// workspace. Shapes B, A are those of the caller's (virtual) [B,A,.] tensors.
-static int proposal_core(float* scores_src, int64_t score_sb, int64_t score_sa, const LevelTable* logits, const float4* rpn_bbox4,
-                         const LevelTable& lv, int64_t B, int64_t A, const DLTensor* anchors, const od_anchor_spec* spec,
-                         const od_proposal_params* params, DLTensor* proposals, const od_proposal_debug* debug, ProposalWs& p,
-                         DeviceScope& scope, cudaStream_t st) {
+// workspace. Shapes B, A are those of the caller's (virtual) [B,A,.] tensors. logits_dt and bbox_dt are the dtypes (F32
+// or BF16) of the logits and of the deltas.
+static int proposal_core(float* scores_src, int64_t score_sb, int64_t score_sa, const LevelTable* logits, DType logits_dt,
+                         const void* rpn_bbox4, const LevelTable& lv, DType bbox_dt, int64_t B, int64_t A,
+                         const DLTensor* anchors, const od_anchor_spec* spec, const od_proposal_params* params,
+                         DLTensor* proposals, const od_proposal_debug* debug, ProposalWs& p, DeviceScope& scope,
+                         cudaStream_t st) {
   const int64_t K = params->pre_nms_limit < A ? params->pre_nms_limit : A;
   const int64_t N = params->post_nms_count;
   OD_CHECK(check_tensor(proposals, "proposals", F32, {B, N, 4}, 16, scope));
@@ -281,7 +313,9 @@ static int proposal_core(float* scores_src, int64_t score_sb, int64_t score_sa, 
   OD_CHECK(check_opt_tensor(dbg.num_kept, "debug.num_kept", I32, {B}, 4, scope));
   if (B == 0 || N == 0) return OD_OK;
   if (logits && B * A > 0) {
-    rpn_level_scores_kernel<<<(unsigned)((B * A + 255) / 256), 256, 0, st>>>(*logits, (int)A, B * A, scores_src);
+    const unsigned grid = (unsigned)((B * A + 255) / 256);
+    if (logits_dt == BF16) rpn_level_scores_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(*logits, (int)A, B * A, scores_src);
+    else rpn_level_scores_kernel<<<grid, 256, 0, st>>>(*logits, (int)A, B * A, scores_src);
     OD_LAUNCH_CHECK("rpn_level_scores_kernel");
   }
   int32_t* ix = dbg.ix ? dptr<int32_t>(dbg.ix) : p.ix;
@@ -300,12 +334,21 @@ static int proposal_core(float* scores_src, int64_t score_sb, int64_t score_sa, 
     dp.clipped_dbg = dptr<float4>(dbg.anchor_delta_clipped);
     const int64_t total = B * K;
     const float4 sd = make_float4(params->bbox_stddev[0], params->bbox_stddev[1], params->bbox_stddev[2], params->bbox_stddev[3]);
-    if (rpn_bbox4)
-      OD_CUDA(launch_pdl(proposal_decode_kernel<false>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st,
-          rpn_bbox4, lv, dptr<float4>(anchors), dspec, use_spec, ix, total, (int)K, (int)A, sd, p.clipped, dp));
+    const dim3 grid((unsigned)((total + 255) / 256));
+    const float4* anc = dptr<float4>(anchors);
+    using BF = __nv_bfloat16;
+    if (rpn_bbox4 && bbox_dt == BF16)
+      OD_CUDA(launch_pdl(proposal_decode_kernel<BF, false>, grid, dim3(256), 0, st, static_cast<const BF*>(rpn_bbox4), lv, anc,
+                         dspec, use_spec, ix, total, (int)K, (int)A, sd, p.clipped, dp));
+    else if (rpn_bbox4)
+      OD_CUDA(launch_pdl(proposal_decode_kernel<false>, grid, dim3(256), 0, st, static_cast<const float4*>(rpn_bbox4), lv, anc,
+                         dspec, use_spec, ix, total, (int)K, (int)A, sd, p.clipped, dp));
+    else if (bbox_dt == BF16)
+      OD_CUDA(launch_pdl(proposal_decode_kernel<BF, true>, grid, dim3(256), 0, st, (const BF*)nullptr, lv, anc, dspec,
+                         use_spec, ix, total, (int)K, (int)A, sd, p.clipped, dp));
     else
-      OD_CUDA(launch_pdl(proposal_decode_kernel<true>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st,
-          (const float4*)nullptr, lv, dptr<float4>(anchors), dspec, use_spec, ix, total, (int)K, (int)A, sd, p.clipped, dp));
+      OD_CUDA(launch_pdl(proposal_decode_kernel<true>, grid, dim3(256), 0, st, (const float4*)nullptr, lv, anc, dspec,
+                         use_spec, ix, total, (int)K, (int)A, sd, p.clipped, dp));
     OD_LAUNCH_CHECK("proposal_decode_kernel");
   }
   // per-image NMS over boxes already in (score desc, index asc) order (:188-196, :234)
@@ -329,7 +372,8 @@ int od_proposal_forward(const DLTensor* rpn_class_probs, const DLTensor* rpn_bbo
   DeviceScope scope;
   OD_CHECK(check_tensor(rpn_class_probs, "rpn_class_probs", F32, {kAny, kAny, 2}, 4, scope));
   const int64_t B = rpn_class_probs->shape[0], A = rpn_class_probs->shape[1];
-  OD_CHECK(check_tensor(rpn_bbox, "rpn_bbox", F32, {B, A, 4}, 16, scope));
+  const DType bbox_dt = f32_or_bf16(rpn_bbox);
+  OD_CHECK(check_tensor(rpn_bbox, "rpn_bbox", bbox_dt, {B, A, 4}, bbox_dt == BF16 ? 8 : 16, scope));
   if (params->pre_nms_limit < 0 || params->post_nms_count < 0) OD_FAIL(OD_ERR_PARAM, "negative counts");
   const int64_t K = params->pre_nms_limit < A ? params->pre_nms_limit : A;
   const int64_t N = params->post_nms_count;
@@ -344,8 +388,8 @@ int od_proposal_forward(const DLTensor* rpn_class_probs, const DLTensor* rpn_bbo
   LevelTable lv;
   memset(&lv, 0, sizeof(lv));
   // scores = probs[:,:,1]  (:153)
-  return proposal_core(dptr<float>(rpn_class_probs) + 1, 2 * A, 2, nullptr, dptr<float4>(rpn_bbox), lv, B, A, anchors, spec,
-                       params, proposals, debug, p, scope, st);
+  return proposal_core(dptr<float>(rpn_class_probs) + 1, 2 * A, 2, nullptr, F32, dptr<void>(rpn_bbox), lv, bbox_dt, B, A,
+                       anchors, spec, params, proposals, debug, p, scope, st);
 }
 
 size_t od_proposal_levels_workspace_bytes(int64_t batch, int64_t num_anchors, const od_proposal_params* p) {
@@ -369,16 +413,24 @@ int od_proposal_forward_levels(const DLTensor* const* class_logits, const DLTens
   memset(&lb, 0, sizeof(lb));
   lc.num_levels = lb.num_levels = num_levels;
   int64_t B = kAny, A = 0;   // B: that of the first level
+  // every level must have the dtype of level 0, the logits and the deltas each on their own
+  const DType logits_dt = f32_or_bf16(class_logits[0]), bbox_dt = f32_or_bf16(bbox[0]);
   for (int l = 0; l < num_levels; ++l) {
     const DLTensor* c = class_logits[l];
     const DLTensor* d = bbox[l];
-    OD_CHECK(check_tensor(c, "class_logits[l]", F32, {B, kAny, kAny, kAny}, 8, scope));
+    if (c && f32_or_bf16(c) != logits_dt)
+      OD_FAIL(OD_ERR_DTYPE, "class_logits[l]: level %d is %s, level 0 is %s (one dtype for every level)", l,
+              logits_dt == BF16 ? "not bfloat16" : "bfloat16", logits_dt == BF16 ? "bfloat16" : "not");
+    OD_CHECK(check_tensor(c, "class_logits[l]", logits_dt, {B, kAny, kAny, kAny}, logits_dt == BF16 ? 4 : 8, scope));
     B = c->shape[0];
     if (c->shape[3] % 2) OD_FAIL(OD_ERR_SHAPE, "class_logits[l]: extent 3 is %lld, expected an even value (level %d)", (long long)c->shape[3], l);
-    OD_CHECK(check_tensor(d, "bbox[l]", F32, {B, c->shape[1], c->shape[2], 2 * c->shape[3]}, 16, scope));
+    if (d && f32_or_bf16(d) != bbox_dt)
+      OD_FAIL(OD_ERR_DTYPE, "bbox[l]: level %d is %s, level 0 is %s (one dtype for every level)", l,
+              bbox_dt == BF16 ? "not bfloat16" : "bfloat16", bbox_dt == BF16 ? "bfloat16" : "not");
+    OD_CHECK(check_tensor(d, "bbox[l]", bbox_dt, {B, c->shape[1], c->shape[2], 2 * c->shape[3]}, bbox_dt == BF16 ? 8 : 16, scope));
     const int64_t n_l = c->shape[1] * c->shape[2] * (c->shape[3] / 2);
-    lc.base[l] = dptr<float>(c);
-    lb.base[l] = dptr<float>(d);
+    lc.base[l] = dptr<void>(c);
+    lb.base[l] = dptr<void>(d);
     lc.off[l] = lb.off[l] = (int32_t)A;
     A += n_l;
     if (A >= (1ll << 31)) OD_FAIL(OD_ERR_PARAM, "too many anchors");
@@ -396,7 +448,8 @@ int od_proposal_forward_levels(const DLTensor* const* class_logits, const DLTens
     carve_proposal_ws(w, B, A, K, N, &p);
     if (!w.ok()) OD_FAIL(OD_ERR_WORKSPACE, "workspace %zu < %zu bytes", ws_bytes, w.off);
   }
-  return proposal_core(scores, A, 1, &lc, nullptr, lb, B, A, anchors, spec, params, proposals, debug, p, scope, st);
+  return proposal_core(scores, A, 1, &lc, logits_dt, nullptr, lb, bbox_dt, B, A, anchors, spec, params, proposals, debug, p,
+                       scope, st);
 }
 
 }  // extern "C"

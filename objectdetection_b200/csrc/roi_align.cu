@@ -1122,12 +1122,8 @@ static int launch_crop_bins(RoiSource src, int64_t n_rois, int32_t ph, int32_t p
   return OD_OK;
 }
 
-// The dtype a ROIAlign map or output tensor is checked against: BF16 for a bfloat16 tensor, F32 for anything else, which
-// check_tensor then refuses unless it is fp32 (float16 included).
-static DType map_or_out_dtype(const DLTensor* t) {
-  return (t && t->dtype.code == kDLBfloat && t->dtype.bits == 16 && t->dtype.lanes == 1) ? BF16 : F32;
-}
-// With a bf16 map or output a pixel must be whole 16-byte units of 8 channels.
+// A ROIAlign map or output tensor is checked against f32_or_bf16(t). With a bf16 map or output a pixel must be whole
+// 16-byte units of 8 channels.
 static int check_bf16_depth(DType map_dt, DType out_dt, int64_t D) {
   if ((map_dt == BF16 || out_dt == BF16) && D % 8)
     OD_FAIL(OD_ERR_SHAPE, "depth %lld must be a multiple of 8 with bfloat16 maps or output", (long long)D);
@@ -1195,7 +1191,7 @@ int od_pyramid_roi_align_forward_ordered(const DLTensor* const* fmaps, int32_t n
   const int64_t B = rois->shape[0], N = rois->shape[1];
   LevelTable lt;
   int64_t D = kAny;   // that of the first level
-  const DType map_dt = map_or_out_dtype(fmaps[0]);   // every level must have the first level's dtype
+  const DType map_dt = f32_or_bf16(fmaps[0]);   // every level must have the first level's dtype
   for (int l = 0; l < num_levels; ++l) {
     OD_CHECK(check_tensor(fmaps[l], "fmaps[l]", map_dt, {B, kAny, kAny, D}, 16, scope));
     D = fmaps[l]->shape[3];
@@ -1204,7 +1200,7 @@ int od_pyramid_roi_align_forward_ordered(const DLTensor* const* fmaps, int32_t n
     lt.W[l] = (int32_t)fmaps[l]->shape[2];
   }
   if (D % 4) OD_FAIL(OD_ERR_SHAPE, "depth %lld must be a multiple of 4", (long long)D);
-  const DType out_dt = map_or_out_dtype(pooled);
+  const DType out_dt = f32_or_bf16(pooled);
   if (pooled && pooled->ndim == 5) OD_CHECK(check_tensor(pooled, "pooled", out_dt, {1, B * N, pool_h, pool_w, D}, 16, scope));
   else OD_CHECK(check_tensor(pooled, "pooled", out_dt, {B * N, pool_h, pool_w, D}, 16, scope));
   OD_CHECK(check_bf16_depth(map_dt, out_dt, D));
@@ -1244,7 +1240,7 @@ int od_crop_and_resize(const DLTensor* image, const DLTensor* boxes, const DLTen
                        int32_t crop_w, float extrapolation_value, DLTensor* out, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   DeviceScope scope;
-  const DType map_dt = map_or_out_dtype(image), out_dt = map_or_out_dtype(out);
+  const DType map_dt = f32_or_bf16(image), out_dt = f32_or_bf16(out);
   OD_CHECK(check_tensor(image, "image", map_dt, {kAny, kAny, kAny, kAny}, 16, scope));
   OD_CHECK(check_tensor(boxes, "boxes", F32, {kAny, 4}, 16, scope));
   const int64_t n = boxes->shape[0], D = image->shape[3];

@@ -58,7 +58,11 @@ def unmold_detections_batch(original_image_shapes, image_shape, detections, imag
 
 class DetectionLayer():
     """Per-ROI argmax class -> class-specific delta decode -> clip to window -> bg/score filter -> per-class NMS
-    -> top-100 -> zero-padded [B,100,6] rows (y1,x1,y2,x2,class_id,score). Signature of detection.py:57."""
+    -> top-100 -> zero-padded [B,100,6] rows (y1,x1,y2,x2,class_id,score). Signature of detection.py:57.
+
+    ``mrcnn_class_probs`` and ``mrcnn_bbox`` may each be float32 or bfloat16: a bfloat16 CUDA tensor (2-byte aligned
+    probabilities, 8-byte aligned boxes) is read as it is, anything else is converted to float32. bfloat16 values are
+    widened exactly, so the detections and DEBUG tensors (float32) are bit for bit those of the call on ``t.float()``."""
 
     def __init__(self, conf, image_shape, num_batches, window, proposals, mrcnn_class_probs, mrcnn_bbox, DEBUG=False):
         self.image_shape = image_shape
@@ -81,8 +85,9 @@ class DetectionLayer():
         L = _lib.lib()
         props = _lib.as_cuda(proposals, torch.float32)
         dev = props.device
-        probs = _lib.as_cuda(mrcnn_class_probs, torch.float32, dev)
-        bbox = _lib.as_cuda(mrcnn_bbox, torch.float32, dev)
+        # bfloat16 head outputs are read as they are (see _lib.read_dtype), anything else as float32
+        probs = _lib.as_cuda(mrcnn_class_probs, _lib.read_dtype([mrcnn_class_probs], 2), dev)
+        bbox = _lib.as_cuda(mrcnn_bbox, _lib.read_dtype([mrcnn_bbox], 8), dev)
         if isinstance(window, torch.Tensor):
             win = _lib.as_cuda(window, torch.float32, dev).reshape(-1, 4)
         else:

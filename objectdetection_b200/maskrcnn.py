@@ -31,10 +31,7 @@ def _map_dtype(maps):
     """The dtype the kernels read ``maps`` in: bfloat16 (no copy) when they are all bfloat16 CUDA tensors that the
     bf16 kernels take as they are (D % 8 == 0, 16-byte aligned data); float32 for anything else, converted as for host
     arrays (fp32 CUDA maps pass through unchanged), so that every map the fp32 path accepted is still accepted."""
-    if all(isinstance(m, torch.Tensor) and m.is_cuda and m.dtype == torch.bfloat16 and m.dim() > 0
-           and m.shape[-1] % 8 == 0 and m.data_ptr() % 16 == 0 for m in maps):
-        return torch.bfloat16
-    return torch.float32
+    return _lib.read_dtype(maps, 16, depth_multiple=8)
 
 
 def pyramid_roi_align(feature_maps, proposals, image_shape, pool_shape, levels=(2, 3, 4, 5), out=None,

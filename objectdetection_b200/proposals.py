@@ -50,6 +50,12 @@ class Proposals():
     ``run_levels(class_logits, bbox)`` takes the RPN head's conv outputs per pyramid level instead
     (``[B,H_l,W_l,2a]`` 'rpn_class_raw' and ``[B,H_l,W_l,4a]`` 'rpn_bbox_pred', rpn.py:50-67): the reshape, the 2-way
     softmax and the concatenation over levels of training.py:146-166 happen inside the layer, nothing is concatenated.
+
+    Head outputs may be float32 or bfloat16 (what ``torch.autocast`` gives a conv): bfloat16 CUDA logits (every level
+    bfloat16, 4-byte aligned) and deltas (every level, or ``rpn_bbox``, bfloat16 and 8-byte aligned) are read as they
+    are, without a float32 copy; anything else is converted to float32. ``rpn_class_probs`` is float32. bfloat16 values
+    are widened exactly, so the proposals and DEBUG tensors (all float32) are bit for bit those of the float32 call on
+    ``t.float()``. ``get_proposal_graph()`` returns the inputs as the kernels read them.
     """
 
     def __init__(self, conf, batch_size, rpn_class_probs=None, rpn_bbox=None, inp_anchors=None,
@@ -85,17 +91,20 @@ class Proposals():
 
     def build(self, levels=None):
         L = _lib.lib()
+        # bfloat16 logits and deltas go to the kernels as they are (one 4-byte (bg, fg) pair, one 8-byte delta row per
+        # load); see _lib.read_dtype. The probabilities of run() are float32.
         if levels is None:
             probs = _lib.as_cuda(self.rpn_class_probs, torch.float32)
             dev = probs.device
-            bbox = _lib.as_cuda(self.rpn_bbox, torch.float32, dev)
+            bbox = _lib.as_cuda(self.rpn_bbox, _lib.read_dtype([self.rpn_bbox], 8), dev)
             if probs.dim() != 3:
                 raise ValueError("rpn_class_probs must be [batch, anchors, 2]")
             B, A = probs.shape[0], probs.shape[1]
         else:
-            logits = [_lib.as_cuda(t, torch.float32) for t in levels[0]]
+            logits_dt, deltas_dt = _lib.read_dtype(levels[0], 4), _lib.read_dtype(levels[1], 8)
+            logits = [_lib.as_cuda(t, logits_dt) for t in levels[0]]
             dev = logits[0].device
-            deltas = [_lib.as_cuda(t, torch.float32, dev) for t in levels[1]]
+            deltas = [_lib.as_cuda(t, deltas_dt, dev) for t in levels[1]]
             if any(t.dim() != 4 for t in logits + deltas):
                 raise ValueError("per-level RPN outputs must be [batch, H, W, channels]")
             B = logits[0].shape[0]

@@ -279,4 +279,12 @@ __device__ __forceinline__ float4 ldg_head4(const __nv_bfloat16* p, int64_t i) {
 
 constexpr int kNumSMsB200 = 148;
 
+// A launch gets 48 KiB of shared memory, static and dynamic together, unless its kernel was opted in to more dynamic shared
+// memory. The opt-in is needed as soon as the dynamic bytes plus the kernel's static shared memory pass 48 KiB, not only
+// when the dynamic bytes alone do. Call sites read the static size once: `static const size_t s = static_smem_bytes(k);`.
+inline size_t static_smem_bytes(const void* kernel) {
+  cudaFuncAttributes a;
+  return cudaFuncGetAttributes(&a, kernel) == cudaSuccess ? a.sharedSizeBytes : (size_t)48 * 1024;   // unknown: opt in
+}
+
 }  // namespace od

@@ -753,7 +753,8 @@ static int wide_scan_slice(int64_t B, int W, bool* prefetch) {
     if (pf) {
       if (S > kWidePrefetchMaxS) continue;
       const size_t smem = wide_scan_smem(S, wide_scan_blocks(S));
-      if (smem > 48 * 1024 &&
+      static const size_t wide_static = static_smem_bytes((const void*)nms_scan_wide_kernel<true>);
+      if (smem + wide_static > 48 * 1024 &&
           cudaFuncSetAttribute(nms_scan_wide_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
         continue;
       if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, nms_scan_wide_kernel<true>, kWideThreads, smem) != cudaSuccess || occ < 1)
@@ -790,7 +791,8 @@ static int scan_round_launch(const unsigned long long* mask, const unsigned long
   }
   if (nslots >= 2) {
     const size_t smem = plain + (size_t)nslots * per_slot;
-    if (smem > 48 * 1024)
+    static const size_t staged_static = static_smem_bytes((const void*)nms_scan_kernel<true>);
+    if (smem + staged_static > 48 * 1024)
       OD_CUDA(cudaFuncSetAttribute(nms_scan_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     OD_CUDA(launch_pdl(nms_scan_kernel<true>, dim3((unsigned)B), dim3(kScanThreads), smem, st, mask, diagT, num_valid, (int)K, W, Ws, nslots, (int)max_out,
                                                                    c_begin, c_end, final_round, scan_state, stride, keep_pos,
@@ -810,7 +812,8 @@ static int scan_round_launch(const unsigned long long* mask, const unsigned long
     return OD_OK;
   } else {
     const size_t smem = plain > 0 ? plain : 128;
-    if (smem > 48 * 1024)
+    static const size_t unstaged_static = static_smem_bytes((const void*)nms_scan_kernel<false>);
+    if (smem + unstaged_static > 48 * 1024)
       OD_CUDA(cudaFuncSetAttribute(nms_scan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     nms_scan_kernel<false><<<(unsigned)B, kScanThreads, smem, st>>>(mask, diagT, num_valid, (int)K, W, Ws, 0, (int)max_out, c_begin,
                                                                     c_end, final_round, scan_state, stride, keep_pos, num_kept,

@@ -582,7 +582,8 @@ int od_rpn_target_forward(const DLTensor* anchors, const DLTensor* gt_boxes, con
       OD_CUDA(launch_pdl(rpn_anchor_best_kernel<true>, grid, dim3(kRpnThreads), smem, st, an, (int)A, gt, gc, (int)G, r.iou_max, r.iou_arg, r.anchors_c,
                                                                      r.part_v, r.part_i));
     } else {
-      if (smem > 48 * 1024)
+      static const size_t best_static = static_smem_bytes((const void*)rpn_anchor_best_kernel<false>);
+      if (smem + best_static > 48 * 1024)
         OD_CUDA(cudaFuncSetAttribute(rpn_anchor_best_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       OD_CUDA(launch_pdl(rpn_anchor_best_kernel<false>, grid, dim3(kRpnThreads), smem, st, an, (int)A, gt, gc, (int)G, r.iou_max, r.iou_arg, r.anchors_c,
                                                                       nullptr, nullptr));

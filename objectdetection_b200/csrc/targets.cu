@@ -401,7 +401,8 @@ int od_detection_target_forward(const DLTensor* proposals, const DLTensor* gt_cl
   dp.gt_assignment = dptr<int32_t>(dbg.gt_assignment);
   const float4 sd = make_float4(params->bbox_stddev[0], params->bbox_stddev[1], params->bbox_stddev[2], params->bbox_stddev[3]);
   const size_t smem_iou = (size_t)(G > 0 ? G : 1) * sizeof(float4);      // <= 128 KiB at the G <= 8192 cap
-  if (smem_iou > 48 * 1024)
+  static const size_t iou_static = static_smem_bytes((const void*)detection_iou_kernel);
+  if (smem_iou + iou_static > 48 * 1024)
     OD_CUDA(cudaFuncSetAttribute(detection_iou_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_iou));
   if (N > 0) {
     const dim3 grid((unsigned)((N + kIouRows - 1) / kIouRows), (unsigned)B);

@@ -507,7 +507,8 @@ int topk_launch(const float* scores, int64_t rows, int64_t cols, int64_t row_str
     OD_CUDA(launch_pdl(topk_tile_sort_kernel, dim3((unsigned)ntiles, (unsigned)rows), dim3(kTileSortThreads), 0, st, buf, n_pow2, (int)k));
     OD_LAUNCH_CHECK("topk_tile_sort_kernel");
     const size_t smem = (size_t)k * sizeof(unsigned long long);
-    if (smem > 48 * 1024)
+    static const size_t merge_static = static_smem_bytes((const void*)topk_merge_emit_kernel);
+    if (smem + merge_static > 48 * 1024)
       OD_CUDA(cudaFuncSetAttribute(topk_merge_emit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     OD_CUDA(launch_pdl(topk_merge_emit_kernel, dim3((unsigned)((k + kMergeThreads - 1) / kMergeThreads), (unsigned)rows), dim3(kMergeThreads), smem, st, 
         buf, n_pow2, (int)k, ib, scores, row_stride, col_stride, idx_out, val_out));

@@ -37,6 +37,7 @@ from test_gpu_parity import assert_bits, cu, host  # noqa: E402
 
 torch = pytest.importorskip("torch")
 f32 = np.float32
+F32, BF16 = torch.float32, torch.bfloat16
 CSRC = os.path.join(os.path.dirname(HERE), "objectdetection_b200", "csrc")
 
 F_SENT, I_SENT = 0x7FBADBAD, 0x7EADBEEF
@@ -293,10 +294,10 @@ def _flat(s):
     return re.sub(r"\s+", "", s)
 
 
-def parse_constants(csrc=CSRC):
-    """Values of the CONST names as the sources define them (simple constexpr expressions over earlier constants)."""
+def parse_constants(consts=CONST, csrc=CSRC):
+    """Values of the `consts` names as the sources define them (simple constexpr expressions over earlier constants)."""
     got = {}
-    for name, (fname, _) in CONST.items():
+    for name, (fname, _) in consts.items():
         src = open(os.path.join(csrc, fname)).read()
         m = re.search(rf"constexpr\s+[\w:]+\s+{name}\s*=\s*([^;]+);", src)
         assert m, f"{name} is not defined in {fname}"
@@ -311,16 +312,18 @@ def parse_constants(csrc=CSRC):
     return got
 
 
-def check_sources(csrc=CSRC):
-    parsed = parse_constants(csrc)
-    wrong = {n: (parsed[n], v) for n, (_, v) in CONST.items() if parsed[n] != v}
-    assert not wrong, f"constants changed in the sources (now, table): {wrong}; update CONST and the formulas"
-    missing = [(f, s) for f, s in LITERALS if _flat(s) not in _flat(open(os.path.join(csrc, f)).read())]
+def check_sources(consts, literals, csrc=CSRC):
+    """Every (file, value) of `consts` is what the sources define, and every (file, text) of `literals` is still in its
+    file (whitespace-insensitive): a table built on them restates the planning code as it stands."""
+    parsed = parse_constants(consts, csrc)
+    wrong = {n: (parsed[n], v) for n, (_, v) in consts.items() if parsed[n] != v}
+    assert not wrong, f"constants changed in the sources (now, table): {wrong}; update the constants and the formulas"
+    missing = [(f, s) for f, s in literals if _flat(s) not in _flat(open(os.path.join(csrc, f)).read())]
     assert not missing, f"thresholds the table restates are no longer in the sources: {missing}"
 
 
 def test_boundary_constants_match_sources():
-    check_sources()
+    check_sources(CONST, LITERALS)
 
 
 def test_boundary_table_values():
@@ -368,6 +371,18 @@ def assert_written(a, what, untouched=None):
     bad = np.argwhere(hit & ~untouched.reshape(-1, 1))
     assert bad.size == 0, f"{what}: {bad.shape[0]} words still hold the sentinel, first at {bad[:3].tolist()}"
     assert hit[untouched].all(), f"{what}: rows that must stay untouched were written"
+
+
+def bf16_round(a):
+    """The bf16 value nearest to each element (round to nearest even, as torch converts), as fp32."""
+    return torch.from_numpy(np.ascontiguousarray(a, f32)).to(BF16).float().numpy()
+
+
+def head_inputs(arrays, dts, vals):
+    """Head-output arrays for a call on dtypes `dts`: each array whose entry in `vals` is BF16 holds bf16 values (so that
+    the fp32 reference sees the widened inputs); returns (host arrays, CUDA tensors of dtypes dts)."""
+    arrays = [bf16_round(a) if v == BF16 else a for a, v in zip(arrays, vals)]
+    return arrays, [cu(a).to(dt) for a, dt in zip(arrays, dts)]
 
 
 def poison(nbytes, dev):
@@ -632,15 +647,17 @@ def _det_inputs(rs, B, N, C, kept=None):
     return props, probs, bbox
 
 
-def run_detection(trace, N, kept=None, C=5):
+def run_detection(trace, N, kept=None, C=5, dts=(F32, F32)):
+    """dts: the dtypes of mrcnn_class_probs and mrcnn_bbox (bf16 inputs hold bf16 values; the oracle sees them widened)."""
     _lib, L, dl = _L()
     conf = Conf()
     rs = np.random.RandomState(N * 11 + (kept or 0))
     B, M = 2, conf.DETECTION_POST_NMS_INSTANCES
     props, probs, bbox = _det_inputs(rs, B, N, C, kept)
+    (probs, bbox), (tpr, tbb) = head_inputs((probs, bbox), dts, dts)
     win_px = np.array([[131, 0, 893, 1024], [0, 0, 1024, 1024]], np.int32)
     win = oracle.norm_boxes(win_px, [1024, 1024]).astype(f32)
-    tp, tpr, tbb, tw = cu(props), cu(probs), cu(bbox), cu(win)
+    tp, tw = cu(props), cu(win)
     det = sent_f32((B, M, 6))
     d = dict(class_ids=sent_i32((B, N)), class_scores=sent_f32((B, N)), refined_proposals=sent_f32((B, N, 4)),
              clipped_proposals=sent_f32((B, N, 4)), keep_mask=sent_i32((B, N)), nms_keep_mask=sent_i32((B, N)))
@@ -676,7 +693,9 @@ def run_detection(trace, N, kept=None, C=5):
     return names, got
 
 
-def run_rpn_loss(trace, A):
+def run_rpn_loss(trace, A, dts=(F32, F32), vals=None):
+    """dts: the dtypes of rpn_class_logits and rpn_pred_box; vals (default dts): the inputs that hold bf16 values.
+    Returns the kernel names and the outputs (losses, pred_box_pos, num_pos)."""
     _lib, L, dl = _L()
     rs = np.random.RandomState(A)
     B, T = 2, 256
@@ -685,7 +704,8 @@ def run_rpn_loss(trace, A):
     lg = rs.normal(0, 2, (B, A, 2)).astype(f32)
     tb = rs.normal(0, 1, (B, T, 4)).astype(f32)
     pb = rs.normal(0, 1, (B, A, 4)).astype(f32)
-    t = [cu(x) for x in (tc, lg, tb, pb)]
+    (lg, pb), (tlg, tpb) = head_inputs((lg, pb), dts, vals or dts)
+    t = [cu(tc), tlg, cu(tb), tpb]
     P = int((tc == 1).sum())
     out, pos, num = sent_f32((2,)), sent_f32((P, 4)), sent_i32((1,))
 
@@ -701,10 +721,12 @@ def run_rpn_loss(trace, A):
     assert_written(out, "losses")
     assert_written(pos, "pred_box_pos")
     assert_written(num, "num_pos")
-    return names
+    return names, (out, pos, num)
 
 
-def run_mrcnn_loss(trace, BR):
+def run_mrcnn_loss(trace, BR, dts=(F32, F32), vals=None):
+    """dts: the dtypes of mrcnn_pred_logits and mrcnn_pred_box; vals (default dts): the inputs that hold bf16 values.
+    Returns the kernel names and the outputs (losses, pred_active)."""
     _lib, L, dl = _L()
     rs = np.random.RandomState(BR)
     B, R, C = 1, BR, 7
@@ -716,7 +738,8 @@ def run_mrcnn_loss(trace, BR):
     act[0, 3] = 0
     tb = rs.random_sample((B, R, 4)).astype(f32)
     pb = rs.random_sample((B, R, C, 4)).astype(f32)
-    t = [cu(x) for x in (ids, lg, act, tb, pb)]
+    (lg, pb), (tlg, tpb) = head_inputs((lg, pb), dts, vals or dts)
+    t = [cu(ids), tlg, cu(act), cu(tb), tpb]
     out, pa = sent_f32((2,)), sent_f32((B, R))
 
     def call():
@@ -729,7 +752,7 @@ def run_mrcnn_loss(trace, BR):
     assert np.isclose(out[0], w_c, rtol=1e-6) and np.isclose(out[1], w_b, rtol=1e-6), (out, w_c, w_b)
     assert_written(out, "losses")
     assert_written(pa, "pred_active")
-    return names
+    return names, (out, pa)
 
 
 def run_rpn_targets(trace, A, G):
@@ -844,9 +867,9 @@ def test_boundary(_cuda, kernel_trace, name, value):
     elif name == "det_finalize_kept":
         names, got = run_detection(kernel_trace, 2048, kept=v)
     elif name == "rpn_loss_chunk":
-        names = run_rpn_loss(kernel_trace, v)
+        names, _ = run_rpn_loss(kernel_trace, v)
     elif name == "mrcnn_loss_cta":
-        names = run_mrcnn_loss(kernel_trace, v)
+        names, _ = run_mrcnn_loss(kernel_trace, v)
     elif name == "rpn_target_chunk":
         names = run_rpn_targets(kernel_trace, v, 12)
     elif name == "rpn_target_fused_gt":

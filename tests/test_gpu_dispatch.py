@@ -29,6 +29,7 @@ f32 = np.float32
 CSRC = os.path.join(os.path.dirname(HERE), "objectdetection_b200", "csrc")
 
 P, D_ = "test_gpu_parity.py::", "test_gpu_dispatch.py::"
+FRONT = "test_gpu_boundaries_front.py::test_front_boundary"          # the bf16 overloads' rows and Faster R-CNN's scan
 KERNEL_PATHS = {
     # topk.cu
     "topk_collect_kernel": P + "test_topk",
@@ -65,12 +66,23 @@ KERNEL_PATHS = {
     "roi_order_kernel": P + "test_roi_pooling_processing_order",
     "crop_rows_kernel": D_ + "test_roi_align_d256_crop_rows_serves_bounds",
     "crop_pool_bins_kernel": D_ + "test_roi_pool_non_power_of_two_depth",
+    "crop_rows_kernel<__nv_bfloat16, float>": FRONT,
+    "crop_rows_kernel<float, __nv_bfloat16>": FRONT,
+    "crop_rows_kernel<__nv_bfloat16, __nv_bfloat16>": FRONT,
+    "crop_bins_kernel<__nv_bfloat16, float, 32, 2, true, false>": FRONT,
+    "crop_bins_kernel<float, __nv_bfloat16, 32, 2, true, false>": FRONT,
+    "crop_bins_kernel<__nv_bfloat16, __nv_bfloat16, 32, 2, true, false>": FRONT,
+    "crop_bins_kernel<__nv_bfloat16, float, 512, 2, true, false>": FRONT,
+    "crop_bins_kernel<float, __nv_bfloat16, 512, 2, true, false>": FRONT,
+    "crop_bins_kernel<__nv_bfloat16, __nv_bfloat16, 512, 2, true, false>": FRONT,
     # nms.cu
     "nms_mask_kernel<true>": D_ + "test_nms_thresholds_zero_one_and_padded_rows",
     "nms_mask_kernel<false>": D_ + "test_nms_negative_threshold",
     "nms_scan_kernel<true>": P + "test_nms",
-    # reached in the second round of a two-round NMS; single-round it needs hundreds of images at K > 12600 (GBs of mask)
+    # od_nms reaches it in the second round of a two-round NMS; Faster R-CNN runs it in one round past the staged ring
+    # (pre_nms_top_n >= 12545: the frcnn_staged_limit row)
     "nms_scan_kernel<false>": P + "test_nms_two_rounds_on_clustered_boxes",
+    "nms_scan_kernel<false> (single round)": FRONT,
     "nms_scan_wide_kernel<true>": D_ + "test_detection_16384_rois_wide_nms_and_finalize_carry",
     "nms_scan_wide_kernel<false>": D_ + "test_nms_wide_scan_without_prefetch",
     "nms_build_keys_kernel": P + "test_nms",
@@ -84,6 +96,9 @@ KERNEL_PATHS = {
     "proposal_decode_kernel": P + "test_proposals_coco_shape",
     "rpn_level_scores_kernel": P + "test_proposals_from_rpn_level_outputs",
     "proposal_gather_kernel": P + "test_proposals_coco_shape",
+    "proposal_decode_kernel<__nv_bfloat16, false>": FRONT,
+    "proposal_decode_kernel<__nv_bfloat16, true>": FRONT,
+    "rpn_level_scores_kernel<__nv_bfloat16>": FRONT,
     "apply_box_deltas_kernel": P + "test_apply_box_deltas_and_clip",
     "clip_boxes_kernel": P + "test_apply_box_deltas_and_clip",
     "gen_anchors_norm_kernel": P + "test_gen_anchors_bit_exact",
@@ -94,8 +109,16 @@ KERNEL_PATHS = {
     "rpn_loss_box_kernel": P + "test_head_losses",
     "rpn_loss_final_kernel": P + "test_head_losses",
     "mrcnn_loss_kernel": P + "test_head_losses",
+    "rpn_loss_class_kernel<__nv_bfloat16>": FRONT,
+    "rpn_loss_box_kernel<__nv_bfloat16>": FRONT,
+    "mrcnn_loss_kernel<__nv_bfloat16, float>": FRONT,
+    "mrcnn_loss_kernel<float, __nv_bfloat16>": FRONT,
+    "mrcnn_loss_kernel<__nv_bfloat16, __nv_bfloat16>": FRONT,
     # detection.cu
     "det_prepare_kernel": P + "test_detection_coco_shape",
+    "det_prepare_kernel<__nv_bfloat16, float>": FRONT,
+    "det_prepare_kernel<float, __nv_bfloat16>": FRONT,
+    "det_prepare_kernel<__nv_bfloat16, __nv_bfloat16>": FRONT,
     "det_rank_gather_kernel": D_ + "test_detection_rank_gather_multi_tile",
     "det_gather_kernel": D_ + "test_detection_bitonic_sort_and_gather",
     "det_finalize_kernel": D_ + "test_detection_16384_rois_wide_nms_and_finalize_carry",

@@ -56,7 +56,9 @@ typedef enum {
   kDLCUDAManaged = 13
 } DLDeviceType;
 typedef struct { DLDeviceType device_type; int32_t device_id; } DLDevice;
-typedef enum { kDLInt = 0U, kDLUInt = 1U, kDLFloat = 2U, kDLOpaqueHandle = 3U, kDLBfloat = 4U } DLDataTypeCode;
+typedef enum {
+  kDLInt = 0U, kDLUInt = 1U, kDLFloat = 2U, kDLOpaqueHandle = 3U, kDLBfloat = 4U, kDLBool = 6U
+} DLDataTypeCode;
 typedef struct { uint8_t code; uint8_t bits; uint16_t lanes; } DLDataType;
 typedef struct {
   void* data;
@@ -279,10 +281,14 @@ size_t od_detection_target_workspace_bytes(int64_t batch, int64_t num_proposals,
  * (data_processor.py:587,:597): the j-th entry of the shuffled list is
  * list[q_j] where q = (p for p in perm if p < len(list)), in perm order.
  * rois [B,R,4] f32, roi_gt_class_ids [B,R] i32, roi_gt_box_deltas [B,R,4] f32.
- * gt_masks [B,G,Mh,Mw] (or [B,Mh,Mw,G], see mask_layout_hwg) f32 and mask_targets [B,R,mask_h,mask_w] f32 are optional
+ * gt_masks [B,G,Mh,Mw] (or [B,Mh,Mw,G], see mask_layout_hwg) and mask_targets [B,R,mask_h,mask_w] f32 are optional
  * (both NULL or both set): target[r] = round(crop_and_resize(gt_mask[assigned GT of r], box_r, [mask_h,mask_w])) for
  * the sampled positives, zero rows elsewhere (north-star extension: the reference prepares the masks but its mask
- * head is commented out; semantics of the model it re-writes). */
+ * head is commented out; semantics of the model it re-writes).
+ * gt_masks is f32, u8 (kDLUInt, 8 bits) or bool (kDLBool, 8 bits), the dtypes mask datasets store masks in; every other
+ * dtype (float16, bf16, int8, float64, ...) is refused with OD_ERR_DTYPE. A byte mask needs no alignment (f32: 4 bytes).
+ * Each byte is widened to fp32 exactly (bool 0 / 1, u8 0..255) and everything after the load is the f32 path, so the
+ * targets equal those of the f32 call on the widened masks bit for bit. mask_targets is always f32. */
 int od_detection_target_forward(const DLTensor* proposals, const DLTensor* gt_class_ids,
                                 const DLTensor* gt_boxes, const DLTensor* perm_pos, const DLTensor* perm_neg,
                                 const od_target_params* params,

@@ -72,7 +72,8 @@ struct DeviceScope {
 };
 
 // ----------------------------------------------------------------------------- DLPack checks
-enum DType { F32, F64, I32, BF16 };   // BF16: kDLBfloat, 16 bits (float16 is kDLFloat, 16 bits, and matches none)
+// BF16: kDLBfloat, 16 bits (float16 is kDLFloat, 16 bits, and matches none); U8: kDLUInt, 8 bits; BOOL: kDLBool, 8 bits
+enum DType { F32, F64, I32, BF16, U8, BOOL };
 // An extent check_tensor accepts at any value. A caller's int64 parameter is checked for a negative value before it is
 // used as an extent, so that it cannot pass as kAny.
 constexpr int64_t kAny = INT64_MIN;
@@ -96,6 +97,12 @@ inline int check_opt_tensor(const DLTensor* t, const char* name, DType dt, std::
 // which check_tensor then refuses unless it is fp32 (float16 included). NULL gives F32.
 inline DType f32_or_bf16(const DLTensor* t) {
   return (t && t->dtype.code == kDLBfloat && t->dtype.bits == 16 && t->dtype.lanes == 1) ? BF16 : F32;
+}
+// The same for an argument that may be fp32 or a byte mask (uint8 or bool): U8 or BOOL for an 8-bit kDLUInt or kDLBool
+// tensor, F32 for anything else (int8 is kDLInt and is refused). NULL gives F32.
+inline DType f32_or_byte(const DLTensor* t) {
+  if (!t || t->dtype.bits != 8 || t->dtype.lanes != 1) return F32;
+  return t->dtype.code == kDLUInt ? U8 : t->dtype.code == kDLBool ? BOOL : F32;
 }
 inline int64_t numel(const DLTensor* t) {
   int64_t n = 1;

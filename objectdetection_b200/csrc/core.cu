@@ -39,8 +39,9 @@ int check_tensor(const DLTensor* t, const char* name, DType dt, const int64_t* e
   } else if (scope.device != t->device.device_id) {
     OD_FAIL(OD_ERR_DEVICE, "%s is on cuda:%d, expected cuda:%d", name, t->device.device_id, scope.device);
   }
-  const uint8_t code = (dt == I32) ? (uint8_t)kDLInt : (dt == BF16) ? (uint8_t)kDLBfloat : (uint8_t)kDLFloat;
-  const uint8_t bits = (dt == F64) ? 64 : (dt == BF16) ? 16 : 32;
+  const uint8_t code = (dt == I32) ? (uint8_t)kDLInt : (dt == BF16) ? (uint8_t)kDLBfloat : (dt == U8) ? (uint8_t)kDLUInt
+                       : (dt == BOOL) ? (uint8_t)kDLBool : (uint8_t)kDLFloat;
+  const uint8_t bits = (dt == F64) ? 64 : (dt == BF16) ? 16 : (dt == U8 || dt == BOOL) ? 8 : 32;
   if (t->dtype.code != code || t->dtype.bits != bits || t->dtype.lanes != 1)
     OD_FAIL(OD_ERR_DTYPE, "%s: dtype (code %d, bits %d) != expected (code %d, bits %d)", name, t->dtype.code,
             t->dtype.bits, code, bits);

@@ -274,11 +274,17 @@ detection_target_kernel(const float4* __restrict__ proposals, const int32_t* __r
 //   box = roi                                   (full-size masks), or
 //   box = (roi - gt_box.y1x1y1x1) / (gt_h, gt_w, gt_h, gt_w)        (mini masks: ROI in the GT box's frame)
 //   target = round(crop_and_resize(gt_mask[assigned GT], box, [mask_h, mask_w]))   round = half to even
-// rows of non-positive ROIs are zero. One CTA per (roi slot, image); D = 1 channel, so plain 4-byte taps.
-__global__ void __launch_bounds__(256)
-mask_target_kernel(const float4* __restrict__ rois, const float4* __restrict__ gt_boxes, const int32_t* __restrict__ mask_src,
-                   const float* __restrict__ gt_masks, int R, int G, int Mh, int Mw, int hwg_layout, int use_mini_mask,
-                   int mh, int mw, float* __restrict__ targets) {
+// rows of non-positive ROIs are zero. One CTA per (roi slot, image); D = 1 channel, so plain scalar taps: 4 bytes for
+// fp32 masks, 1 byte for uint8 and bool masks. A byte widens to fp32 exactly (bool 0 / 1, uint8 0..255), and everything
+// after the load is the fp32 path, so a byte mask gives the fp32 call's targets on the widened mask bit for bit.
+__device__ __forceinline__ float ldg_mask(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ldg_mask(const uint8_t* p) { return (float)__ldg(p); }
+
+template <typename TMask>
+__device__ __forceinline__ void mask_target_body(const float4* __restrict__ rois, const float4* __restrict__ gt_boxes,
+                                                 const int32_t* __restrict__ mask_src, const TMask* __restrict__ gt_masks,
+                                                 int R, int G, int Mh, int Mw, int hwg_layout, int use_mini_mask, int mh,
+                                                 int mw, float* __restrict__ targets) {
   const int r = blockIdx.x, b = blockIdx.y;
   float* o = targets + ((int64_t)b * R + r) * mh * mw;
   const int g = mask_src[(int64_t)b * R + r];
@@ -294,7 +300,7 @@ mask_target_kernel(const float4* __restrict__ rois, const float4* __restrict__ g
     box = make_float4((box.x - gt.x) / gt_h, (box.y - gt.y) / gt_w, (box.z - gt.x) / gt_h, (box.w - gt.y) / gt_w);
   }
   // element (y, x) of GT mask g: [B,G,Mh,Mw] or the reference's [B,Mh,Mw,G]
-  const float* img = gt_masks + (int64_t)b * G * Mh * Mw + (hwg_layout ? (int64_t)g : (int64_t)g * Mh * Mw);
+  const TMask* img = gt_masks + (int64_t)b * G * Mh * Mw + (hwg_layout ? (int64_t)g : (int64_t)g * Mh * Mw);
   const int64_t sy = hwg_layout ? (int64_t)Mw * G : Mw, sx = hwg_layout ? G : 1;
   const float Hm1 = (float)(Mh - 1), Wm1 = (float)(Mw - 1);
   const float hs = (mh > 1) ? (box.z - box.x) * Hm1 / (float)(mh - 1) : 0.0f;
@@ -308,14 +314,29 @@ mask_target_kernel(const float4* __restrict__ rois, const float4* __restrict__ g
       const float fy = floorf(in_y), fx = floorf(in_x);
       const int64_t top = (int64_t)fy, bot = (int64_t)ceilf(in_y), left = (int64_t)fx, right = (int64_t)ceilf(in_x);
       const float yl = in_y - fy, xl = in_x - fx;
-      const float tl = __ldg(img + top * sy + left * sx), tr = __ldg(img + top * sy + right * sx);
-      const float bl = __ldg(img + bot * sy + left * sx), br = __ldg(img + bot * sy + right * sx);
+      const float tl = ldg_mask(img + top * sy + left * sx), tr = ldg_mask(img + top * sy + right * sx);
+      const float bl = ldg_mask(img + bot * sy + left * sx), br = ldg_mask(img + bot * sy + right * sx);
       const float t = tl + (tr - tl) * xl;
       const float bt = bl + (br - bl) * xl;
       v = t + (bt - t) * yl;
     }
     o[e] = rintf(v);
   }
+}
+
+__global__ void __launch_bounds__(256)
+mask_target_kernel(const float4* __restrict__ rois, const float4* __restrict__ gt_boxes, const int32_t* __restrict__ mask_src,
+                   const float* __restrict__ gt_masks, int R, int G, int Mh, int Mw, int hwg_layout, int use_mini_mask,
+                   int mh, int mw, float* __restrict__ targets) {
+  mask_target_body<float>(rois, gt_boxes, mask_src, gt_masks, R, G, Mh, Mw, hwg_layout, use_mini_mask, mh, mw, targets);
+}
+// uint8 and bool masks (TMask = uint8_t): the same body, an overload of the same name (the fp32 kernel above keeps its name)
+template <typename TMask>
+__global__ void __launch_bounds__(256)
+mask_target_kernel(const float4* __restrict__ rois, const float4* __restrict__ gt_boxes, const int32_t* __restrict__ mask_src,
+                   const TMask* __restrict__ gt_masks, int R, int G, int Mh, int Mw, int hwg_layout, int use_mini_mask,
+                   int mh, int mw, float* __restrict__ targets) {
+  mask_target_body<TMask>(rois, gt_boxes, mask_src, gt_masks, R, G, Mh, Mw, hwg_layout, use_mini_mask, mh, mw, targets);
 }
 
 }  // namespace od
@@ -353,9 +374,11 @@ int od_detection_target_forward(const DLTensor* proposals, const DLTensor* gt_cl
   OD_CHECK(check_tensor(roi_gt_box_deltas, "roi_gt_box_deltas", F32, {B, R, 4}, 16, scope));
   if ((gt_masks == nullptr) != (mask_targets == nullptr)) OD_FAIL(OD_ERR_NULL, "gt_masks and mask_targets go together");
   int64_t Mh = 0, Mw = 0;
+  const DType mask_dt = f32_or_byte(gt_masks);            // f32, u8 or bool; a byte mask is read one byte per element
   if (gt_masks) {
-    if (params->mask_layout_hwg) OD_CHECK(check_tensor(gt_masks, "gt_masks", F32, {B, kAny, kAny, G}, 4, scope));
-    else OD_CHECK(check_tensor(gt_masks, "gt_masks", F32, {B, G, kAny, kAny}, 4, scope));
+    const int mask_align = (mask_dt == F32) ? 4 : 1;
+    if (params->mask_layout_hwg) OD_CHECK(check_tensor(gt_masks, "gt_masks", mask_dt, {B, kAny, kAny, G}, mask_align, scope));
+    else OD_CHECK(check_tensor(gt_masks, "gt_masks", mask_dt, {B, G, kAny, kAny}, mask_align, scope));
     Mh = gt_masks->shape[params->mask_layout_hwg ? 1 : 2];
     Mw = gt_masks->shape[params->mask_layout_hwg ? 2 : 3];
     if (params->mask_h < 1 || params->mask_w < 1 || Mh < 1 || Mw < 1) OD_FAIL(OD_ERR_PARAM, "mask sizes must be positive");
@@ -418,7 +441,14 @@ int od_detection_target_forward(const DLTensor* proposals, const DLTensor* gt_cl
       dptr<int32_t>(perm_neg), (int)N, (int)G, (int)R, sd, dptr<float4>(rois), dptr<int32_t>(roi_gt_class_ids),
       dptr<float4>(roi_gt_box_deltas), ws_i32, ws_f32, (const int32_t*)n_prop, gt_masks ? mask_src : nullptr, dp));
   OD_LAUNCH_CHECK("detection_target_kernel");
-  if (gt_masks) {
+  if (gt_masks && mask_dt != F32) {
+    const dim3 grid((unsigned)R, (unsigned)B);
+    mask_target_kernel<uint8_t><<<grid, 256, 0, st>>>(dptr<float4>(rois), dptr<float4>(gt_boxes), mask_src, dptr<uint8_t>(gt_masks),
+                                                      (int)R, (int)G, (int)Mh, (int)Mw, params->mask_layout_hwg ? 1 : 0,
+                                                      params->use_mini_mask ? 1 : 0, params->mask_h, params->mask_w,
+                                                      dptr<float>(mask_targets));
+    OD_LAUNCH_CHECK("mask_target_kernel<uint8_t>");
+  } else if (gt_masks) {
     const dim3 grid((unsigned)R, (unsigned)B);
     mask_target_kernel<<<grid, 256, 0, st>>>(dptr<float4>(rois), dptr<float4>(gt_boxes), mask_src, dptr<float>(gt_masks), (int)R,
                                              (int)G, (int)Mh, (int)Mw, params->mask_layout_hwg ? 1 : 0,

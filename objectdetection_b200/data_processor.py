@@ -10,6 +10,19 @@ from . import _lib
 from .proposals import _stddev4
 
 
+def _mask_dtype(gt_masks) -> torch.dtype:
+    """The dtype od_detection_target_forward reads ``gt_masks`` in: bool or uint8 for a bool or uint8 tensor or numpy
+    array, float32 for anything else."""
+    import numpy as np
+    if isinstance(gt_masks, torch.Tensor):
+        dt = gt_masks.dtype
+    elif isinstance(gt_masks, np.ndarray):
+        dt = {np.dtype(np.bool_): torch.bool, np.dtype(np.uint8): torch.uint8}.get(gt_masks.dtype)
+    else:
+        dt = None
+    return dt if dt in (torch.bool, torch.uint8) else torch.float32
+
+
 class BuildDetectionTargets():
     """Proposal <-> GT IoU, positive/negative sampling, GT assignment, box-delta targets, zero padding.
 
@@ -58,10 +71,12 @@ class BuildDetectionTargets():
         rcls = torch.empty((B, R), dtype=torch.int32, device=dev)
         deltas = torch.empty((B, R, 4), dtype=torch.float32, device=dev)
         # optional mask targets: gt_masks in the reference's batch layout [B,Mh,Mw,G] ([Mh,Mw,G] per image,
-        # data_processor.py:386,399); MINI_MASK_SHAPE masks cropped to their GT box when conf.USE_MINI_MASK
+        # data_processor.py:386,399); MINI_MASK_SHAPE masks cropped to their GT box when conf.USE_MINI_MASK.
+        # bool and uint8 masks (what mask datasets store) stay one byte per element, on the host-to-device copy too:
+        # the kernel widens each byte exactly, so the targets are those of gt_masks.float(). Other dtypes go as float32.
         masks = mtargets = None
         if gt_masks is not None:
-            masks = _lib.as_cuda(gt_masks, torch.float32, dev)
+            masks = _lib.as_cuda(gt_masks, _mask_dtype(gt_masks), dev)
             if single:
                 masks = masks[None]
             if masks.dim() != 4 or masks.shape[0] != B or masks.shape[3] != G:
